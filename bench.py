@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the LFM hot path (BASELINE.json metric: NLML+grad evaluations / second, fp64).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload at every N: BASELINE config 2, synthetic LFM 50 genes x 80 time points (N = 4000), one
 "step" = one NLML + gradient evaluation at the reference's initial hyper-parameters.  A single
@@ -101,6 +101,14 @@ def clocks_parse(path, dev_index):
             "samples": len(sm)}
 
 
+def dump_outputs(path, nlml_grad, info):
+    """--dump-outputs: what the last timed step returned, as float64 .npy files.  The inputs are seeded, so two builds
+    (or a build and --impl reference) can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "nlml_grad.npy"), np.asarray(nlml_grad, dtype=np.float64).reshape(-1))
+    np.save(os.path.join(path, "info.npy"), np.asarray(info, dtype=np.float64).reshape(-1))
+
+
 def run_reference(args):
     """CPU arm: the oracle restatement of the reference path on the host cores (rank 0 only)."""
     rank = int(os.environ.get("RANK", "0"))
@@ -117,24 +125,22 @@ def run_reference(args):
         blas_threads = max([m.get("num_threads", 0) for m in threadpoolctl.threadpool_info()] or [0])
     except Exception:
         pass
-    budget = 150.0
-    t0 = time.perf_counter(); o.nlml_and_grad(p, X, y, threads=cores); t1 = time.perf_counter() - t0
-    warm_done = 1
-    while warm_done < args.warmup and (warm_done + 1) * t1 < 0.25 * budget:
-        o.nlml_and_grad(p, X, y, threads=cores); warm_done += 1
-    steps_exec = int(max(1, min(args.steps, (budget - warm_done * t1) // max(t1, 1e-3))))
-    t0 = time.perf_counter()
-    for _ in range(steps_exec):
+    for _ in range(args.warmup):
         o.nlml_and_grad(p, X, y, threads=cores)
+    t0 = time.perf_counter()
+    for _ in range(args.steps):
+        v, g = o.nlml_and_grad(p, X, y, threads=cores)
     dt = time.perf_counter() - t0
-    val = steps_exec / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.concatenate([[v], g]), 0)   # the oracle raises where the device reports info > 0
+    val = args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus,
-            "steps": args.steps, "steps_executed": steps_exec, "warmup": args.warmup,
-            "ms_per_step": 1e3 * dt / steps_exec, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+            "steps": args.steps, "steps_executed": args.steps, "warmup": args.warmup,
+            "ms_per_step": 1e3 * dt / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f64", "data": "synthetic",
             "config": CONFIG,
             "cpu_baseline": {"value": val, "unit": UNIT, "cores": cores, "blas_threads": blas_threads, "kind": "port",
-                             "sample": f"{steps_exec} full NLML+grad evaluations at N=4000 (oracle/lfm_oracle.py, "
+                             "sample": f"{args.steps} full NLML+grad evaluations at N=4000 (oracle/lfm_oracle.py, "
                                        "numpy+scipy+LAPACK, row chunks over all host threads)"},
             "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
@@ -149,7 +155,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-secondary", action="store_true", help="skip the batched / N=32768 secondary measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (rank 0) as float64 .npy files to DIR: "
+                         "nlml_grad.npy (NLML, then the gradient) and info.npy (factorisation status, 0 = success)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -250,6 +263,8 @@ def main():
     dev_s = sum(e0.elapsed_time(e1) for e0, e1 in evs) * 1e-3
     dev_s = max_over_ranks(dev_s)
     value = world * args.steps / dev_s
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out.cpu().numpy(), info.cpu().numpy())
 
     # ---- e2e: the host-buffer C-ABI call (H2D of X, y, theta and D2H of NLML+grad inside the timed region) ----
     import ctypes as C

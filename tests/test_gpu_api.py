@@ -251,6 +251,43 @@ def test_examples_main_runs_the_reference_script(cuda, tmp_path):
     assert len(cmp_rows) == 5 and float(cmp_rows[3]["S_learned"]) == 1.0 and float(cmp_rows[3]["D_learned"]) == 0.8
 
 
+def test_bench_dump_outputs_are_the_last_timed_step(cuda, tmp_path):
+    """bench.py --dump-outputs: after the timed steps, the NLML+gradient and status the evaluation plan returned in the
+    last one are written as float64 .npy files; two runs with the same arguments write the same bits (seeded inputs), and
+    --impl reference writes the oracle's numbers for the same inputs, which they match to 1e-9.  Both arms run exactly
+    --steps timed steps: the device arm's launch count is that many replays of the N = 4000 evaluation plan."""
+    import subprocess
+    import sys
+    from dis_project_b200 import _lib, ops
+    lib = _lib.lib()
+    plan = ops.NlmlGradPlan(o.make_inputs(50, 80), np.zeros(4000), 50, 1e-4)   # bench.py's config-2 shape
+    th = o.Params.reference_init(50).pack()
+    plan(th)
+    l0 = lib.lfm_debug_launch_count()
+    plan(th)
+    launches_per_step = lib.lfm_debug_launch_count() - l0
+    plan.close()
+    assert launches_per_step > 0
+    bench = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
+    dumps = []
+    for run, extra in (("a", []), ("b", []), ("ref", ["--impl", "reference"])):
+        d = tmp_path / run
+        r = subprocess.run([sys.executable, bench, "--steps", "2", "--warmup", "1", "--no-secondary", "--no-cpu",
+                            "--dump-outputs", str(d)] + extra, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        if extra:
+            assert line["steps_executed"] == 2
+        else:
+            assert line["gpu_launches"] == 2 * launches_per_step, (line["gpu_launches"], launches_per_step)
+        assert sorted(os.listdir(d)) == ["info.npy", "nlml_grad.npy"]
+        dumps.append((np.load(d / "nlml_grad.npy"), np.load(d / "info.npy")))
+    (out, info), (out2, info2), (ref, _) = dumps
+    assert out.dtype == np.float64 and out.shape == (3 * 50 + 3,) and info.tolist() == [0.0]
+    assert np.array_equal(out, out2) and np.array_equal(info, info2)
+    assert abs(out[0] - ref[0]) <= RTOL * abs(ref[0]) and relerr(out[1:], ref[1:]) < RTOL
+
+
 def test_batched_team_size_follows_the_batch(cuda):
     """lfm_batched_team_size: a shard that leaves SMs idle gets four warps per LFM, a full GPU one warp per LFM,
     shapes outside the warp / team kernels report 0 (CTA-per-LFM kernel)."""
@@ -553,11 +590,10 @@ def test_warp_specialised_gemm_is_bit_identical(cuda, tmp_path, ws):
     assert np.array_equal(other, got)
 
 
-@pytest.mark.skipif(os.environ.get("LFM_FULLSIZE") != "1", reason="minutes of host time: set LFM_FULLSIZE=1 (tools/fullsize_parity.py)")
 def test_configs_3_and_5_full_size_oracle_parity(cuda, tmp_path):
     """BASELINE configs 3 and 5 against the oracle at FULL size (N = 32768; 102 400 test times, the oracle on a sample of
-    256 of them): 1e-9 relative, north_star's tolerance.  Opt-in (about 3 minutes on 16 host cores); the record of the
-    last run is profiles/fullsize_parity_r2.json, checked by tests/test_host.py."""
+    256 of them): 1e-9 relative, north_star's tolerance.  The oracle takes minutes of host time (about 2.5 on 16 cores,
+    profiles/fullsize_parity_r2.json, whose record tests/test_host.py checks)."""
     import subprocess
     import sys
     out = tmp_path / "fullsize.json"
