@@ -86,6 +86,11 @@ SIGNATURES = {
     "lfm_batched_queue_bytes": (_sz, [_i64, _int, _int]),
     "lfm_batched_fit_queue": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
                                      _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _ptr, _int, _ptr, _sz]),
+    "lfm_batched_nlml_grad_unc_het": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _dbl, _int, _int,
+                                             _ptr, _ptr, _ptr]),
+    "lfm_batched_fit_het": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl,
+                                   _dbl, _int, _int, _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _ptr,
+                                   _int, _ptr, _sz]),
     "lfm_batched_structure_bytes": (_sz, [_i64, _int, _int, _int]),
     "lfm_batched_team_size": (_int, [_i64, _i64, _int, _int, _int]),
     "lfm_batched_best": (_int, [_ptr, _i64, _int, _ptr, _i64, _i64, _ptr, _dbl, _ptr]),
@@ -104,6 +109,8 @@ SIGNATURES = {
                                          _ptr, _ptr]),
     "lfm_batched_fit_host": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
                                     _int, _int, _int, _ptr, _ptr, _ptr]),
+    "lfm_batched_fit_het_host": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
+                                        _int, _int, _int, _ptr, _ptr, _ptr]),
     "lfm_debug_leaf_profile": (_int, [_ptr, _ptr, _ptr, _ptr, _ptr]),
     "lfm_debug_launch_count": (C.c_ulonglong, []),
     "lfm_debug_batched_stamps": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _int, _int, _int, _ptr, _ptr,

@@ -146,7 +146,9 @@ class _MsfPlan:
     copies into the staging buffer and five stream-ordered calls -- the fit kernel is in flight ~30 us after
     `multi_start_fit` is entered instead of ~200 us (`tools/msf_timeline.py`: the device used to wait for the host)."""
 
-    def __init__(self, device, N, G, Bl, per_lfm_y, num_iters, chunk, trace, world):
+    def __init__(self, device, N, G, Bl, per_lfm_y, num_iters, chunk, trace, world, var_rows=0):
+        """`var_rows`: 0 without measurement variances, 1 with one vector shared by the shard, Bl with one row per LFM:
+        they ride in the same staging buffer and copy, [X | y | variances | start points]."""
         import torch
 
         from . import ops
@@ -154,14 +156,18 @@ class _MsfPlan:
         P = 3 * G + 2
         ev = lambda n: (int(n) + 1) & ~1
         ny = Bl * N if per_lfm_y else N
+        nv = var_rows * N
         self.N, self.G, self.P, self.Bl, self.ny, self.num_iters, self.chunk, self.trace = N, G, P, Bl, ny, num_iters, chunk, trace
-        self.oy, self.oth = ev(3 * N), ev(3 * N) + ev(ny)
+        self.oy, self.ov = ev(3 * N), ev(3 * N) + ev(ny)
+        self.nv, self.oth = nv, self.ov + ev(nv)
         total = self.oth + ev(Bl * P)
         self.pin_in = torch.empty(total, dtype=torch.float64, pin_memory=True)
         self.h_in = self.pin_in.numpy()
         self.d_in = torch.empty(total, dtype=torch.float64, device=device)
         self.Xd = self.d_in[:3 * N].view(N, 3)
         self.yd = self.d_in[self.oy:self.oy + ny]
+        self.vd = self.d_in[self.ov:self.ov + nv] if nv else None
+        self.var_stride = N if var_rows > 1 else 0
         self.th0 = self.d_in[self.oth:self.oth + Bl * P].view(Bl, P)
         self.y_stride = N if per_lfm_y else 0
         self.nchunks = max((num_iters + chunk - 1) // chunk, 1)
@@ -217,7 +223,7 @@ class _MsfPlan:
 
 
 def _msf_planned(Xh, yh, theta0_all, lo, hi, per_lfm_y, jitter, num_iters, lr, fix_params, num_steps_per_epoch, chunk,
-                 b1, b2, eps, trace, comm, queue_chunk, dist, rank, world, device, timing):
+                 b1, b2, eps, trace, comm, queue_chunk, dist, rank, world, device, timing, vh=None, per_lfm_var=False):
     """The host-buffer path of `multi_start_fit` over a cached `_MsfPlan` (same results, same collectives)."""
     import time
 
@@ -236,19 +242,22 @@ def _msf_planned(Xh, yh, theta0_all, lo, hi, per_lfm_y, jitter, num_iters, lr, f
             torch.cuda.synchronize()
             tmarks.append(time.perf_counter())
 
+    var_rows = 0 if vh is None else (Bl if per_lfm_var else 1)
     key = (device.index if device.index is not None else torch.cuda.current_device(), N, G, Bl, per_lfm_y, num_iters, chunk,
-           trace, world)
+           trace, world, vh is not None, per_lfm_var)
     plan = _PLANS.get(key)
     if plan is None:
         if len(_PLANS) > 8:
             _PLANS.clear()
-        plan = _PLANS[key] = _MsfPlan(device, N, G, Bl, per_lfm_y, num_iters, chunk, trace, world)
+        plan = _PLANS[key] = _MsfPlan(device, N, G, Bl, per_lfm_y, num_iters, chunk, trace, world, var_rows)
     lib = ops._lib.lib()
     check = ops._lib.check
     st = plan.st
     plan.stage_X(Xh)
     h = plan.h_in
     h[plan.oy:plan.oy + plan.ny] = (yh[lo:hi] if per_lfm_y else yh).reshape(-1)
+    if vh is not None:
+        h[plan.ov:plan.ov + plan.nv] = (vh[lo:hi] if per_lfm_var else vh).reshape(-1)
     h[plan.oth:plan.oth + Bl * P] = theta0_all[lo:hi].reshape(-1)
     main = torch.cuda.current_stream()
     s = main.cuda_stream
@@ -269,7 +278,12 @@ def _msf_planned(Xh, yh, theta0_all, lo, hi, per_lfm_y, jitter, num_iters, lr, f
         best_key = None if trace else keys_ptr + 8 * c
         step_keys = keys_ptr if trace else None
         qb = plan.queue(queue_chunk) if (trace and chunk >= num_iters and queue_chunk > 0 and done == 0) else 0
-        if qb > 0:
+        if plan.vd is not None:   # one entry point for the chunked and the queue launches
+            check(lib.lfm_batched_fit_het(s, *common[:6], plan.vd.data_ptr(), plan.var_stride, *common[6:], done, steps,
+                                          num_iters, *tail, best_key, step_keys, plan.struct.data_ptr(),
+                                          int(queue_chunk) if qb > 0 else 0, plan.queue_ws.data_ptr() if qb > 0 else None,
+                                          qb), "lfm_batched_fit_het")
+        elif qb > 0:
             check(lib.lfm_batched_fit_queue(s, *common, num_iters, *tail, best_key, step_keys, plan.struct.data_ptr(),
                                             int(queue_chunk), plan.queue_ws.data_ptr(), qb), "lfm_batched_fit_queue")
         else:
@@ -341,7 +355,7 @@ def _msf_planned(Xh, yh, theta0_all, lo, hi, per_lfm_y, jitter, num_iters, lr, f
 def multi_start_fit(X, y, theta0_all, jitter: float, *, num_iters: int = 150, lr: float = 0.01,
                     fix_params: bool = True, num_steps_per_epoch: int = 1000, chunk: Optional[int] = 1,
                     b1: float = 0.9, b2: float = 0.999, eps: float = 1e-8, trace: bool = False,
-                    comm=None, queue_chunk: int = 10) -> MultiStartResult:
+                    comm=None, queue_chunk: int = 10, variances=None) -> MultiStartResult:
     """Fit all restarts of this rank's shard on the current CUDA device.
 
     `theta0_all` is the (B, P) array of constrained start points of the WHOLE job (every rank passes
@@ -363,6 +377,9 @@ def multi_start_fit(X, y, theta0_all, jitter: float, *, num_iters: int = 150, lr
     one-CTA-per-LFM assignment would leave SMs unevenly loaded (e.g. 512 LFMs per GPU), ignored elsewhere; 0 = never.
     `comm`: a ``dis_project_b200.comm.LfmComm`` -- the collectives then run through the C-ABI's own NCCL communicator
     (``lfm_comm_*``) and rank / world come from it; default: ``torch.distributed``.
+    `variances`: None, or the measurement variances of the heteroscedastic objective, Sigma = K + diag(variances) +
+    (jitter + sigma^2) I (the third output of ``dataset_3d``): (N,) / (N, 1) shared by every LFM, or (B, N) with one row
+    per LFM, sliced per shard like `y` (``lfm_batched_fit_het``, include/lfm_b200.h).
     """
     import torch
     import torch.distributed as dist
@@ -395,7 +412,11 @@ def multi_start_fit(X, y, theta0_all, jitter: float, *, num_iters: int = 150, lr
     device = X.device if isinstance(X, torch.Tensor) and X.is_cuda else torch.device("cuda", torch.cuda.current_device())
     yh = y if isinstance(y, torch.Tensor) else np.asarray(y, dtype=np.float64)
     per_lfm_y = yh.ndim == 2 and yh.shape[0] == B and yh.shape[1] == (X.shape[0]) and B != 1
-    host_inputs = not isinstance(X, torch.Tensor) and not isinstance(yh, torch.Tensor)
+    vh, per_lfm_var = None, False
+    if variances is not None:
+        vh = variances if isinstance(variances, torch.Tensor) else np.asarray(variances, dtype=np.float64)
+        per_lfm_var = ops._variance_layout(vh.shape, B, X.shape[0])
+    host_inputs = not isinstance(X, torch.Tensor) and not isinstance(yh, torch.Tensor) and not isinstance(vh, torch.Tensor)
     hint = tg = None
     if host_inputs and hi > lo and os.environ.get("LFM_MSF_PLAN", "1") != "0":
         Xh = np.ascontiguousarray(np.asarray(X, dtype=np.float64))
@@ -403,7 +424,7 @@ def multi_start_fit(X, y, theta0_all, jitter: float, *, num_iters: int = 150, lr
             raise ValueError(f"x must have shape (n, 3) = [time, gene_index, flag] (dataset.py:391), got {Xh.shape}")
         return _msf_planned(Xh, yh, theta0_all, lo, hi, per_lfm_y, jitter, num_iters, lr, fix_params, num_steps_per_epoch,
                             chunk, b1, b2, eps, trace, comm, queue_chunk, dist if distributed and comm is None else None,
-                            rank, world, device, timing)
+                            rank, world, device, timing, vh, per_lfm_var)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     if host_inputs:
@@ -412,12 +433,17 @@ def multi_start_fit(X, y, theta0_all, jitter: float, *, num_iters: int = 150, lr
         ops._check_training_flags(Xh)
         hint, tg = ops.unique_rows(Xh), ops.distinct_times(Xh)  # from the host copy: no device->host round trip
         ysel = np.ascontiguousarray(yh[lo:hi]) if per_lfm_y else yh.reshape(-1)
-        Xd, yd, th0 = _stage_to_device(device, [Xh, ysel, np.ascontiguousarray(theta0_all[lo:hi])])
+        staged = [Xh, ysel, np.ascontiguousarray(theta0_all[lo:hi])]
+        if vh is not None:
+            staged.append(np.ascontiguousarray(vh[lo:hi]) if per_lfm_var else vh.reshape(-1))
+        Xd, yd, th0, *vd = _stage_to_device(device, staged)
+        vd = vd[0] if vd else None
         Xd = ops._rows3(Xd, "x")
     else:
         Xd = ops._rows3(X, "x")
         yd = ops._dev(yh[lo:hi]) if per_lfm_y else ops._dev(yh).reshape(-1)
         th0 = theta0_all[lo:hi]
+        vd = None if vh is None else (ops._dev(vh[lo:hi]) if per_lfm_var else ops._dev(vh).reshape(-1))
     nchunks = max((num_iters + chunk - 1) // chunk, 1)
     nkeys = max(num_iters, 1) if trace else nchunks
     # behind the state of the shard, in the same allocation: what this rank contributes to the final all-gather --
@@ -447,7 +473,7 @@ def multi_start_fit(X, y, theta0_all, jitter: float, *, num_iters: int = 150, lr
             ops.batched_fit_steps(st, Xd, yd, jitter, steps, lr=lr, b1=b1, b2=b2, eps=eps, fix_params=fix_params,
                                   steps_per_epoch=num_steps_per_epoch, best_key=None if trace else keys[c:c + 1],
                                   step_keys=keys if trace else None,
-                                  queue_chunk=queue_chunk if trace and chunk >= num_iters else 0)
+                                  queue_chunk=queue_chunk if trace and chunk >= num_iters else 0, variances=vd)
         done += steps
         if side is not None:
             ev = torch.cuda.Event()

@@ -50,13 +50,16 @@ __device__ __forceinline__ void pair_decode(int p, int& r, int& c) {
 }
 
 // BT = 128 when the unique rows fit 64 (two threads per row in the Cholesky), else 256.
-template <int BT>
+// HET: heteroscedastic objective (a.var != NULL), noise c_i = v_i + c per point; M = diag(cbar) + R K_u (header of
+// include/lfm_b200.h, lfm_batched_nlml_grad_unc_het).
+template <int BT, bool HET>
 __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(BatchedArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int N = a.N, G = a.G, P = 3 * G + 2;
   const int tid = threadIdx.x;
   const int64_t bidx = blockIdx.x;
   const double* yb = a.y + bidx * a.y_stride;   // this LFM's observations (y_stride = 0: shared)
+  const double* vb = HET ? a.var + bidx * a.var_stride : nullptr;   // ... and their variances
   // ---- carve shared memory (matrix sized for the worst case U = N) ---------------------------------
   const int MU = a.max_unique;
   double* S = reinterpret_cast<double*>(smem_raw);
@@ -74,7 +77,9 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
   double* av = am + P;                  // P adam v
   double* mu = av + P;                  // G positional means B/D
   double* red = mu + G;                 // 16
-  LfmPoint* pts = reinterpret_cast<LfmPoint*>(red + 16);
+  double* cbar = red + 16;              // HET: R / sum_{i in u} 1/c_i     (U)
+  double* tw = cbar + (HET ? N : 0);    // HET: weight of M^-1_uu in tr Sigma^-1 (U)
+  LfmPoint* pts = reinterpret_cast<LfmPoint*>(red + 16 + (HET ? 2 * N : 0));
   int* umap = reinterpret_cast<int*>(pts + N);  // row -> unique index      (N)
   int* urow = umap + N;                         // unique index -> first row (N)
   __shared__ double piv;
@@ -157,6 +162,8 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
     if (tid < G) mu[tid] = th[2 * G + tid] / th[tid];
     if (tid < U) pts[tid] = lfm_make_point(a.X + 3 * urow[tid], G, th, th + G, l, true);
     __syncthreads();
+    double zz, lsum = 0.0, tr0 = 0.0;   // HET: zz = sum z_i^2 / c_i, lsum = sum log c_i - sum log cbar_u, tr0
+    if constexpr (!HET) {
     double zz_part = 0.0;
     if (tid < N) {
       int m = tid / blk;
@@ -164,7 +171,7 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
       const double zi = yb[tid] - mu[m] * (double)((int)a.X[3 * tid + 2]);
       zz_part = zi * zi;
     }
-    const double zz = block_sum<BT>(zz_part, red);
+    zz = block_sum<BT>(zz_part, red);
     if (tid < U) {
       double acc = 0.0;
       for (int i = 0; i < N; ++i) {
@@ -176,12 +183,30 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
       }
       q[tid] = acc;
     }
+    } else {
+    double zp = 0.0, lp = 0.0, tp = 0.0;
+    if (tid < U) {
+      double om = 0.0, om2 = 0.0, s = 0.0;
+      for (int i = 0; i < N; ++i) {
+        if (umap[i] == tid) {
+          int m = i / blk;
+          if (m > G - 1) m = G - 1;
+          lfm_het_point(yb[i] - mu[m] * (double)((int)a.X[3 * i + 2]), vb[i], c, om, om2, s, zp, lp);
+        }
+      }
+      lfm_het_row(dR, om, om2, s, cbar[tid], q[tid], tw[tid], lp, tp);
+    }
+    zz = block_sum<BT>(zp, red);
+    lsum = block_sum<BT>(lp, red);
+    tr0 = block_sum<BT>(tp, red);
+    if (tid == 0 && !(lsum == lsum) && fail == 0) fail = 1;   // some c_i <= 0: Sigma is not a covariance
+    }
     // ---- C. M = c I + R K_u (lower + diagonal) -------------------------------------------------------
     for (int p = tid; p < npairs; p += BT) {
       int r, cc;
       pair_decode(p, r, cc);
       double k = dR * lfm_kxx(pts[r], pts[cc], l, inv_l);
-      if (r == cc) k += c;
+      if (r == cc) k += HET ? cbar[r] : c;
       S[r * ld + cc] = k;
     }
     __syncthreads();
@@ -258,15 +283,15 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
       const double* uj = S + tid * ld;
       for (int i = tid + 1; i < U; ++i) acc += uj[i] * w[i];
       beta[tid] = acc;
-      const double kbv = (q[tid] - c * acc) / dR;
+      const double kbv = (q[tid] - (HET ? cbar[tid] : c) * acc) / dR;
       kb[tid] = kbv;
-      qkb_part = q[tid] * kbv;
+      qkb_part = (HET ? q[tid] / cbar[tid] : q[tid]) * kbv;
       kbkb_part = kbv * kbv;
     }
     const double qkb = block_sum<BT>(qkb_part, red);
     const double kbkb = block_sum<BT>(kbkb_part, red);
-    const double quad = (zz - qkb) / c;
-    const double nlml = 0.5 * ((double)N * LFM_LOG_2PI + (double)(N - U) * log(c) + logdetM + quad);
+    const double quad = HET ? zz - qkb : (zz - qkb) / c;
+    const double nlml = 0.5 * ((double)N * LFM_LOG_2PI + (HET ? lsum : (double)(N - U) * log(c)) + logdetM + quad);
     // ---- G. M^-1 = W^T W into the lower triangle (+ sdiag), every entry independent --------------------
     for (int p = tid; p < npairs; p += BT) {
       int r, cc;
@@ -317,23 +342,41 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
       for (int i = 0; i < U; ++i) {
         if (pts[i].gene == m) {
           gd += dsum[i];
-          gs += 1.0 - c * sdiag[i] - beta[i] * kb[i];
+          gs += 1.0 - (HET ? cbar[i] : c) * sdiag[i] - beta[i] * kb[i];
         }
       }
-      // asum_m = sum_{i in positional block m} alpha_i,  alpha_i = (z_i - (K_u beta)_{u(i)}) / c
-      for (int i = m * blk; i < (m + 1) * blk; ++i)
-        asum += yb[i] - mu[m] * (double)((int)a.X[3 * i + 2]) - kb[umap[i]];
-      asum /= c;
+      // asum_m = sum_{i in positional block m} alpha_i,  alpha_i = (z_i - (K_u beta)_{u(i)}) / c_i
+      if constexpr (HET) {
+        for (int i = m * blk; i < (m + 1) * blk; ++i)
+          asum += (yb[i] - mu[m] * (double)((int)a.X[3 * i + 2]) - kb[umap[i]]) / (vb[i] + c);
+      } else {
+        for (int i = m * blk; i < (m + 1) * blk; ++i)
+          asum += yb[i] - mu[m] * (double)((int)a.X[3 * i + 2]) - kb[umap[i]];
+        asum /= c;
+      }
       const double D = th[m], Sm = th[G + m], Bm = th[2 * G + m];
       gr[m] = gd + asum * Bm / (D * D);
       gr[G + m] = gs / Sm;
       gr[2 * G + m] = -asum / D;
     }
     if (tid == G) {
-      double tr = 0.0;
-      for (int i = 0; i < U; ++i) tr += sdiag[i];
-      const double trSinv = ((double)(N - U) + c * tr) / c;
-      const double aa = (zz - 2.0 * qkb + dR * kbkb) / (c * c);
+      double tr = 0.0, trSinv, aa;
+      if constexpr (HET) {
+        // tr Sigma^-1 = tr0 + sum_u tw_u M^-1_uu,  alpha^T alpha = sum_i alpha_i^2
+        for (int i = 0; i < U; ++i) tr += tw[i] * sdiag[i];
+        trSinv = tr0 + tr;
+        aa = 0.0;
+        for (int i = 0; i < N; ++i) {
+          int m = i / blk;
+          if (m > G - 1) m = G - 1;
+          const double al = (yb[i] - mu[m] * (double)((int)a.X[3 * i + 2]) - kb[umap[i]]) / (vb[i] + c);
+          aa += al * al;
+        }
+      } else {
+        for (int i = 0; i < U; ++i) tr += sdiag[i];
+        trSinv = ((double)(N - U) + c * tr) / c;
+        aa = (zz - 2.0 * qkb + dR * kbkb) / (c * c);
+      }
       gr[3 * G] = gl;
       gr[3 * G + 1] = sigma * (trSinv - aa);
     }
@@ -394,10 +437,10 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
   }
 }
 
-static size_t batched_smem_bytes(int N, int G, int MU) {
+static size_t batched_smem_bytes(int N, int G, int MU, bool het) {
   const size_t P = 3 * (size_t)G + 2;
   const size_t ld = (size_t)(MU | 1);
-  size_t d = (size_t)MU * ld + 7 * (size_t)N + 5 * P + (size_t)G + 16;
+  size_t d = (size_t)MU * ld + (het ? 9 : 7) * (size_t)N + 5 * P + (size_t)G + 16;
   return d * 8 + (size_t)N * sizeof(LfmPoint) + 2 * (size_t)N * sizeof(int);
 }
 
@@ -405,6 +448,7 @@ static int batched_launch(cudaStream_t st, const BatchedArgs& a, int time_grid) 
   if (a.B <= 0 || a.N <= 0 || a.G <= 0 || !a.X || !a.y || !a.u_io) return LFM_ERR_INVALID;
   if (a.N % a.G) return LFM_ERR_INVALID;
   if (a.y_stride != 0 && a.y_stride < a.N) return LFM_ERR_INVALID;
+  if (a.var && a.var_stride != 0 && a.var_stride < a.N) return LFM_ERR_INVALID;
   if (a.N > 128 || a.B > 0x7fffffff) return LFM_ERR_UNSUPPORTED;
   BatchedArgs b = a;
   if (b.max_unique <= 0 || b.max_unique > b.N) b.max_unique = b.N;
@@ -413,27 +457,37 @@ static int batched_launch(cudaStream_t st, const BatchedArgs& a, int time_grid) 
     if (st2 != LFM_ERR_UNSUPPORTED) return st2;
   }
   b.queue = nullptr;   // the CTA-per-LFM kernel has no queue mode: plain launch over all the steps it was given
-  const size_t smem = batched_smem_bytes(b.N, b.G, b.max_unique);
+  const bool het = b.var != nullptr;
+  const size_t smem = batched_smem_bytes(b.N, b.G, b.max_unique, het);
   if (smem > 227 * 1024) return LFM_ERR_UNSUPPORTED;
   const bool small = b.max_unique <= 64 && b.N <= 128 && 3 * b.G + 2 <= 128;
   if (!small && 3 * b.G + 2 > 256) return LFM_ERR_UNSUPPORTED;
-  static LfmSmemConfig conf128, conf256;
-  if (small) {
-    LFM_CUDA_OK(lfm_ensure_smem(lfm_batched_kernel<128>, conf128, smem));
-    lfm_batched_kernel<128><<<(unsigned)b.B, 128, smem, st>>>(b);
+  static LfmSmemConfig conf128, conf256, conf128h, conf256h;
+  if (het) {
+    if (small) {
+      LFM_CUDA_OK(lfm_ensure_smem(lfm_batched_kernel<128, true>, conf128h, smem));
+      lfm_batched_kernel<128, true><<<(unsigned)b.B, 128, smem, st>>>(b);
+    } else {
+      LFM_CUDA_OK(lfm_ensure_smem(lfm_batched_kernel<256, true>, conf256h, smem));
+      lfm_batched_kernel<256, true><<<(unsigned)b.B, 256, smem, st>>>(b);
+    }
+  } else if (small) {
+    LFM_CUDA_OK(lfm_ensure_smem(lfm_batched_kernel<128, false>, conf128, smem));
+    lfm_batched_kernel<128, false><<<(unsigned)b.B, 128, smem, st>>>(b);
   } else {
-    LFM_CUDA_OK(lfm_ensure_smem(lfm_batched_kernel<256>, conf256, smem));
-    lfm_batched_kernel<256><<<(unsigned)b.B, 256, smem, st>>>(b);
+    LFM_CUDA_OK(lfm_ensure_smem(lfm_batched_kernel<256, false>, conf256, smem));
+    lfm_batched_kernel<256, false><<<(unsigned)b.B, 256, smem, st>>>(b);
   }
   LFM_LAUNCHED(1);
   LFM_CUDA_OK(cudaGetLastError());
   return LFM_OK;
 }
 
-extern "C" int lfm_batched_nlml_grad_unc_multi(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
-                                               const double* y, int64_t y_stride, const double* theta_unc, double jitter,
-                                               int unique_rows_hint, int time_grid_hint, double* out_val,
-                                               double* out_grad, int* info) {
+extern "C" int lfm_batched_nlml_grad_unc_het(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
+                                             const double* y, int64_t y_stride, const double* variances,
+                                             int64_t var_stride, const double* theta_unc, double jitter,
+                                             int unique_rows_hint, int time_grid_hint, double* out_val,
+                                             double* out_grad, int* info) {
   if (!out_val || !out_grad) return LFM_ERR_INVALID;
   BatchedArgs a;
   memset(&a, 0, sizeof(a));
@@ -441,8 +495,16 @@ extern "C" int lfm_batched_nlml_grad_unc_multi(lfm_stream_t stream, int64_t B, i
   a.u_io = const_cast<double*>(theta_unc);  // read-only in eval mode
   a.jitter = jitter; a.steps = 1; a.total_steps = 1; a.steps_per_epoch = 1;
   a.eval_val = out_val; a.eval_grad = out_grad; a.info = info; a.max_unique = unique_rows_hint;
+  a.var = variances; a.var_stride = variances ? var_stride : 0;
   if (N > 128) return LFM_ERR_UNSUPPORTED;
   return batched_launch((cudaStream_t)stream, a, time_grid_hint);
+}
+extern "C" int lfm_batched_nlml_grad_unc_multi(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
+                                               const double* y, int64_t y_stride, const double* theta_unc, double jitter,
+                                               int unique_rows_hint, int time_grid_hint, double* out_val,
+                                               double* out_grad, int* info) {
+  return lfm_batched_nlml_grad_unc_het(stream, B, N, G, X, y, y_stride, nullptr, 0, theta_unc, jitter, unique_rows_hint,
+                                       time_grid_hint, out_val, out_grad, info);
 }
 extern "C" int lfm_batched_nlml_grad_unc_tg(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
                                             const double* y, const double* theta_unc, double jitter,
@@ -485,14 +547,17 @@ extern "C" size_t lfm_batched_queue_bytes(int64_t B, int total_steps, int chunk_
   if (B * nchunks > 0x7fffffff) return 0;
   return (size_t)(4 + B + B * nchunks) * sizeof(int);
 }
-extern "C" int lfm_batched_fit_queue(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                                     int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter,
-                                     double lr, double b1, double b2, double eps, int total_steps, int fix_params,
-                                     int steps_per_epoch, int unique_rows_hint, int time_grid_hint, double* out_hist,
-                                     int64_t ld_hist, double* out_theta, int* info, long long* best_key,
-                                     long long* step_keys, void* structure_cache, int chunk_steps, void* queue_ws,
-                                     size_t queue_bytes) {
-  if (total_steps < 0 || steps_per_epoch <= 0) return LFM_ERR_INVALID;
+// One body for the chunked (queue_ws NULL) and the persistent-queue fits, with or without variances (see the header).
+extern "C" int lfm_batched_fit_het(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
+                                   int64_t y_stride, const double* variances, int64_t var_stride, double* theta_unc_io,
+                                   double* adam_state, double jitter, double lr, double b1, double b2, double eps,
+                                   int first_step, int steps, int total_steps, int fix_params, int steps_per_epoch,
+                                   int unique_rows_hint, int time_grid_hint, double* out_hist, int64_t ld_hist,
+                                   double* out_theta, int* info, long long* best_key, long long* step_keys,
+                                   void* structure_cache, int chunk_steps, void* queue_ws, size_t queue_bytes) {
+  if (steps < 0 || first_step < 0 || steps_per_epoch <= 0) return LFM_ERR_INVALID;
+  if (first_step > 0 && !adam_state) return LFM_ERR_INVALID;
+  if (queue_ws && (first_step != 0 || steps != total_steps)) return LFM_ERR_INVALID;   // the queue runs the whole fit
   if (N > 128) return LFM_ERR_UNSUPPORTED;
   if (queue_ws && (chunk_steps <= 0 || queue_bytes < lfm_batched_queue_bytes(B, total_steps, chunk_steps) ||
                    lfm_batched_queue_bytes(B, total_steps, chunk_steps) == 0 || !adam_state))
@@ -501,12 +566,26 @@ extern "C" int lfm_batched_fit_queue(lfm_stream_t stream, int64_t B, int64_t N, 
   memset(&a, 0, sizeof(a));
   a.B = B; a.N = (int)N; a.G = G; a.X = X; a.y = y; a.y_stride = y_stride; a.u_io = theta_unc_io; a.adam = adam_state;
   a.jitter = jitter; a.lr = lr; a.b1 = b1; a.b2 = b2; a.eps = eps;
-  a.first_step = 0; a.steps = total_steps; a.total_steps = total_steps; a.fix_params = fix_params;
+  a.first_step = first_step; a.steps = steps; a.total_steps = total_steps; a.fix_params = fix_params;
   a.steps_per_epoch = steps_per_epoch; a.hist = out_hist; a.ld_hist = ld_hist; a.theta_out = out_theta;
   a.info = info; a.max_unique = unique_rows_hint; a.best_key = best_key; a.step_keys = step_keys;
   a.struct_cache = structure_cache;
-  a.queue = (int*)queue_ws; a.queue_chunk = chunk_steps;
+  if (queue_ws) { a.queue = (int*)queue_ws; a.queue_chunk = chunk_steps; }
+  a.var = variances; a.var_stride = variances ? var_stride : 0;
   return batched_launch((cudaStream_t)stream, a, time_grid_hint);
+}
+extern "C" int lfm_batched_fit_queue(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
+                                     int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter,
+                                     double lr, double b1, double b2, double eps, int total_steps, int fix_params,
+                                     int steps_per_epoch, int unique_rows_hint, int time_grid_hint, double* out_hist,
+                                     int64_t ld_hist, double* out_theta, int* info, long long* best_key,
+                                     long long* step_keys, void* structure_cache, int chunk_steps, void* queue_ws,
+                                     size_t queue_bytes) {
+  if (total_steps < 0) return LFM_ERR_INVALID;
+  return lfm_batched_fit_het(stream, B, N, G, X, y, y_stride, nullptr, 0, theta_unc_io, adam_state, jitter, lr, b1, b2,
+                             eps, 0, total_steps, total_steps, fix_params, steps_per_epoch, unique_rows_hint,
+                             time_grid_hint, out_hist, ld_hist, out_theta, info, best_key, step_keys, structure_cache,
+                             chunk_steps, queue_ws, queue_bytes);
 }
 extern "C" int lfm_batched_fit_trace(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
                                      int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter,
@@ -514,18 +593,10 @@ extern "C" int lfm_batched_fit_trace(lfm_stream_t stream, int64_t B, int64_t N, 
                                      int total_steps, int fix_params, int steps_per_epoch, int unique_rows_hint,
                                      int time_grid_hint, double* out_hist, int64_t ld_hist, double* out_theta,
                                      int* info, long long* best_key, long long* step_keys, void* structure_cache) {
-  if (steps < 0 || first_step < 0 || steps_per_epoch <= 0) return LFM_ERR_INVALID;
-  if (first_step > 0 && !adam_state) return LFM_ERR_INVALID;
-  if (N > 128) return LFM_ERR_UNSUPPORTED;
-  BatchedArgs a;
-  memset(&a, 0, sizeof(a));
-  a.B = B; a.N = (int)N; a.G = G; a.X = X; a.y = y; a.y_stride = y_stride; a.u_io = theta_unc_io; a.adam = adam_state;
-  a.jitter = jitter; a.lr = lr; a.b1 = b1; a.b2 = b2; a.eps = eps;
-  a.first_step = first_step; a.steps = steps; a.total_steps = total_steps; a.fix_params = fix_params;
-  a.steps_per_epoch = steps_per_epoch; a.hist = out_hist; a.ld_hist = ld_hist; a.theta_out = out_theta;
-  a.info = info; a.max_unique = unique_rows_hint; a.best_key = best_key; a.step_keys = step_keys;
-  a.struct_cache = structure_cache;
-  return batched_launch((cudaStream_t)stream, a, time_grid_hint);
+  return lfm_batched_fit_het(stream, B, N, G, X, y, y_stride, nullptr, 0, theta_unc_io, adam_state, jitter, lr, b1, b2,
+                             eps, first_step, steps, total_steps, fix_params, steps_per_epoch, unique_rows_hint,
+                             time_grid_hint, out_hist, ld_hist, out_theta, info, best_key, step_keys, structure_cache, 0,
+                             nullptr, 0);
 }
 // Debug: one launch of `steps` >= 2 steps with clock64 stamps at the phase boundaries of the SECOND step of LFM 0
 // (warp-per-LFM kernel only): A B C D E[load] E[routine] E[W^T W] E[Schur] E[store] F I J K end.

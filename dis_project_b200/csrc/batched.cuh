@@ -25,6 +25,11 @@ struct BatchedArgs {
   int queue_chunk;      // steps per task in queue mode
   long long* step_keys; // NULL or total_steps device words: word s receives atomicMin of lfm_loss_key(loss at step s) over the batch
   long long* best_key; // NULL or one device word: atomicMin of lfm_loss_key(loss after the launch's last step) over the batch     // shared-memory matrix is sized for this many unique rows (N when unknown)
+  // Heteroscedastic objective (the HET instantiations; appended so that the parameter offsets of the others stay put):
+  // NULL, or the measurement variances v, Sigma = K + diag(v) + (jitter + sigma^2) I.  var_stride 0: one vector of N
+  // shared by every LFM; N or more: LFM b reads var + b * var_stride (as y / y_stride).
+  const double* var;
+  int64_t var_stride;
 };
 
 // Order-preserving map double -> signed 64-bit integer (finite values and infinities; NaN never enters): the
@@ -49,6 +54,31 @@ struct LfmQueue {
 };
 __host__ __device__ inline LfmQueue lfm_queue_view(int* base, int64_t B) {
   LfmQueue q; q.head = base; q.tail = base + 1; q.done = base + 4; q.ring = base + 4 + B; q.B = B; return q;
+}
+
+// Per-row noise of the heteroscedastic objective, c_i = v_i + jitter + sigma^2, folded into one unique row u (rows i in
+// u): accumulates omega = sum 1/c_i, omega2 = sum 1/c_i^2, s = sum z_i / c_i, zz = sum z_i^2 / c_i and lc = sum log c_i.
+// A non-positive (or NaN) c_i makes lc NaN: the kernels report it as a failed factorisation.
+__device__ __forceinline__ void lfm_het_point(double z, double v, double c, double& om, double& om2, double& s,
+                                              double& zz, double& lc) {
+  const double ci = v + c;
+  const double inv = 1.0 / ci;
+  om += inv;
+  om2 += inv * inv;
+  s += z * inv;
+  zz += z * z * inv;
+  lc += ci > 0.0 ? log(ci) : __longlong_as_double(0x7ff8000000000000LL);
+}
+// ... and closes the row: cbar = R / omega (the diagonal of M = diag(cbar) + R K_u), q = cbar s, the weight
+// tw = R omega2 / omega^2 of M^-1_uu in tr Sigma^-1; lc -= log cbar, tr0 += omega - omega2 / omega.
+__device__ __forceinline__ void lfm_het_row(double R, double om, double om2, double s, double& cbar, double& q,
+                                            double& tw, double& lc, double& tr0) {
+  const double cb = R / om;
+  cbar = cb;
+  q = cb * s;
+  tw = R * om2 / (om * om);
+  lc -= log(cb);
+  tr0 += om - om2 / om;
 }
 
 // batched_warp.cu: launches the warp-per-LFM kernel when the problem fits its limits, else LFM_ERR_UNSUPPORTED

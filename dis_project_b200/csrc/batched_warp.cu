@@ -62,7 +62,9 @@ template <int NW> __device__ __forceinline__ double tsum(double v, double* red, 
   for (int w = 1; w < NW; ++w) s += r[w];
   return s;
 }
-template <int NW> __device__ __forceinline__ int tsum_int(int v) {
+// (HET: one static red_i per kernel instantiation -- an array shared by two kernels is not demoted into either and
+// would move the static shared layout of the homoscedastic ones)
+template <int NW, bool HET> __device__ __forceinline__ int tsum_int(int v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   if constexpr (NW == 1) {
     return v;
@@ -184,13 +186,14 @@ __device__ __forceinline__ unsigned stage1_class_decode(int cls, int i, int G, i
 struct WarpLayout {
   int ld;
   size_t S, tA1R1, tA1, tG1, g2, inv, utime, e2, c2, q, beta, kb, sdiag, dsum, th, u, gr, am, av, mu, ys, ring, red, side, Msm, Xs, gterm, Em, Ep, e3, g3t, Gt, Gd, er1, dval;
+  size_t vs, cbar, tw;  // heteroscedastic objective only: variances (N), cbar and the trace weights (MU)
   size_t pts;       // byte offset
   size_t ints;      // byte offset: umap[N], urow[MU], rows_of[N], mflag[N]
   size_t itab;      // byte offset (inside the integer region, so that it travels with the structure cache)
   size_t bytes;
 };
 #define ITAB 512          // stage-1 items of a step whose decoding is tabulated once per fit (team kernels)
-__host__ __device__ inline WarpLayout warp_layout(int N, int G, int MU, int MT, bool team) {
+__host__ __device__ inline WarpLayout warp_layout(int N, int G, int MU, int MT, bool team, bool het) {
   WarpLayout L;
   const int P = 3 * G + 2;
   L.ld = MU | 1;
@@ -214,6 +217,8 @@ __host__ __device__ inline WarpLayout warp_layout(int N, int G, int MU, int MT, 
   L.side = take((size_t)P + 4 + 2 * (size_t)G);   // team kernels: Jacobians of the bijectors + scalars + 1/D, 1/S prepared by the spare warp
   L.gterm = take(4 * (size_t)G);
   L.dval = take((size_t)MT * MT);
+  L.vs = L.cbar = L.tw = 0;
+  if (het) { L.vs = take(N); L.cbar = take(MU); L.tw = take(MU); }
   {  // aliases inside S
     size_t so = L.S;
     auto sub = [&](size_t n) { size_t r = so; so += (n + 1) & ~(size_t)1; return r; };
@@ -237,7 +242,9 @@ __host__ __device__ inline WarpLayout warp_layout(int N, int G, int MU, int MT, 
   return L;
 }
 
-template <int NW>
+// HET: heteroscedastic objective (a.var != NULL): noise c_i = v_i + c per point, M = diag(cbar) + R K_u; the per-step
+// quantities cbar, q and the trace weights come out of phase B, alpha_i = (z_i - (K_u beta)_u(i)) / c_i out of phase J.
+template <int NW, bool HET>
 __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_batched_warp_kernel(BatchedArgs a, int MT) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int NT = 32 * NW;
@@ -249,7 +256,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
   // until the fit is done; bidx / first_step / task_steps are then per task (see the task loop below)
   int64_t bidx = a.queue ? (int64_t)(blockIdx.x % a.B) : (int64_t)blockIdx.x;
   const int MU = a.max_unique;
-  const WarpLayout L = warp_layout(N, G, MU, MT, NW > 1);
+  const WarpLayout L = warp_layout(N, G, MU, MT, NW > 1, HET);
   double* base = reinterpret_cast<double*>(smem_raw);
   double* S = base + L.S;
   double* tA1R1 = base + L.tA1R1; double* tA1 = base + L.tA1; double* tG1 = base + L.tG1;
@@ -264,6 +271,8 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
   (void)side;
   double* Msm = base + L.Msm; double* Xs = base + L.Xs;
   double* gterm = base + L.gterm;
+  double* vs = base + L.vs; double* cbar = base + L.cbar; double* tw = base + L.tw;
+  (void)vs; (void)cbar; (void)tw;
   double* Em = base + L.Em; double* Ep = base + L.Ep; double* e3 = base + L.e3;
   double* Gt = base + L.Gt; double* Gd = base + L.Gd; double* er1 = base + L.er1; double* dval = base + L.dval;
   LfmPoint* pts = reinterpret_cast<LfmPoint*>(smem_raw + L.pts);
@@ -297,6 +306,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
     for (int i = tid; i < MT; i += NT) utime[i] = srcd[i];
     for (int i = tid; i < MT * MT; i += NT) dval[i] = srcd[MT + i];
     for (int i = tid; i < N; i += NT) ys[i] = a.y[bidx * a.y_stride + i];
+    if constexpr (HET) for (int i = tid; i < N; i += NT) vs[i] = a.var[bidx * a.var_stride + i];
     ld = U | 1;
     npairs = U * (U + 1) / 2;
     tsync<NW>();
@@ -312,6 +322,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       if (Xsm[3 * j] == t0 && Xsm[3 * j + 1] == g0 && Xsm[3 * j + 2] == f0) { rep = j; break; }
     umap[i] = rep;
     ys[i] = a.y[bidx * a.y_stride + i];
+    if constexpr (HET) vs[i] = a.var[bidx * a.var_stride + i];
     int m = i / blk;
     if (m > G - 1) m = G - 1;
     mflag[i] = 2 * m + (((int)f0) != 0 ? 1 : 0);
@@ -328,7 +339,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       rows_of[i] = cnt;  // temporarily the multiplicity of row i's class
     }
     tsync<NW>();
-    nrep = tsum_int<NW>(nrep);
+    nrep = tsum_int<NW, HET>(nrep);
     const int cnt0 = rows_of[0];
     int bad = 0;
     for (int i = tid; i < N; i += NT) bad |= (rows_of[i] != cnt0);
@@ -372,7 +383,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       pts[r].flag = first;  // temporary marker
     }
     tsync<NW>();
-    Tu = tsum_int<NW>(nfirst);
+    Tu = tsum_int<NW, HET>(nfirst);
     if (Tu > MT) { fail = -2; }  // caller's time-grid bound was wrong: refuse (info = -2)
     else {
       for (int r = tid; r < U; r += NT) {
@@ -417,7 +428,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
     tsync<NW>();
     int cnt = 0;
     for (int p = tid; p < TTp; p += NT) cnt += (didx[p] == p);
-    nD = tsum_int<NW>(cnt);
+    nD = tsum_int<NW, HET>(cnt);
     tsync<NW>();
     for (int p = tid; p < TTp; p += NT) didx[p] = (unsigned short)(int)Gd[p];
   }
@@ -498,6 +509,8 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
     task_steps = min(a.queue_chunk, a.total_steps - first_step);
     if (a.y_stride != 0)
       for (int i = tid; i < N; i += NT) ys[i] = __ldcg(a.y + bidx * a.y_stride + i);
+    if (HET && a.var_stride != 0)
+      for (int i = tid; i < N; i += NT) vs[i] = __ldcg(a.var + bidx * a.var_stride + i);
     fail = fail_struct;
   }
   for (int p = tid; p < P; p += NT) {
@@ -548,6 +561,8 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
     // Stage 1: every item is ONE transcendental of (theta, l, times) alone; stage 2: the products.
     int slow = 0;
     double zz = 0.0;
+    double lsum = 0.0, tr0 = 0.0;   // HET: zz = sum z_i^2 / c_i, lsum = sum log c_i - sum log cbar_u, tr0 (lfm_het_row)
+    (void)lsum; (void)tr0;
     if constexpr (NW == 1) {
     double* g3t = base + L.g3t;
     for (int m = lane; m < G; m += 32) {
@@ -607,6 +622,18 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       pgene[r] = p.gene;
     }
     __syncwarp();
+    if constexpr (HET) {
+      for (int r = lane; r < U; r += 32) {
+        double om = 0.0, om2 = 0.0, sz = 0.0;
+        for (int k = 0; k < R; ++k) {
+          const int i = rows_of[r * R + k];
+          lfm_het_point(ys[i] - mu[mflag[i] >> 1] * (double)(mflag[i] & 1), vs[i], c, om, om2, sz, zz, lsum);
+        }
+        lfm_het_row(dR, om, om2, sz, cbar[r], q[r], tw[r], lsum, tr0);
+      }
+      zz = wsum(zz); lsum = wsum(lsum); tr0 = wsum(tr0);
+      __syncwarp();
+    } else {
     for (int i = lane; i < N; i += 32) {
       const double zi = ys[i] - mu[mflag[i] >> 1] * (double)(mflag[i] & 1);
       zz += zi * zi;
@@ -619,6 +646,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
         acc += ys[i] - mu[mflag[i] >> 1] * (double)(mflag[i] & 1);
       }
       q[r] = acc;
+    }
     }
     } else {
     {
@@ -710,6 +738,16 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       ibase += U;
       TEAM_ITEMS(e, G * G, ibase) inv[e] = 1.0 / (th[e / G] + th[e % G]);
       ibase += G * G;
+      if constexpr (HET) {
+        TEAM_ITEMS(r, U, ibase) {
+          double om = 0.0, om2 = 0.0, sz = 0.0;
+          for (int k = 0; k < R; ++k) {
+            const int i = rows_of[r * R + k];
+            lfm_het_point(ys[i] - mu[mflag[i] >> 1] * (double)(mflag[i] & 1), vs[i], c, om, om2, sz, zz, lsum);
+          }
+          lfm_het_row(dR, om, om2, sz, cbar[r], q[r], tw[r], lsum, tr0);
+        }
+      } else {
       TEAM_ITEMS(r, U, ibase) {
         double acc = 0.0;
         for (int k = 0; k < R; ++k) {
@@ -718,15 +756,22 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
         }
         q[r] = acc;
       }
+      }
     }
     WSTAMPX(2);
+    if constexpr (HET) {
+      tsum2<NW>(zz, lsum, red, flip);
+      tr0 = tsum<NW>(tr0, red, flip);
+    } else {
     for (int i = tid; i < N; i += NT) {
       const double zi = ys[i] - mu[mflag[i] >> 1] * (double)(mflag[i] & 1);
       zz += zi * zi;
     }
     zz = tsum<NW>(zz, red, flip);
+    }
     tsync<NW>();
     }
+    if (HET && !(lsum == lsum) && fail == 0) fail = 1;   // some c_i <= 0: Sigma is not a covariance
     WSTAMP();
     // ---- C. time-grid tables: per (b, ia, ib) products of the factors above (tG1 holds A1 * g1) -----------------
     for (int e = tid; e < G * TT; e += NT) {
@@ -779,7 +824,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       w_h_core<false>(pj, pi, l, inv_l, pair_terms(pj, pi), H1, u0, u1, u2);
       w_h_core<false>(pi, pj, l, inv_l, pair_terms(pi, pj), H2, u0, u1, u2);
       double k = dR * (pi.s * pj.s * (LFM_SQRT_PI * 0.5 * l) * (H1 + H2));
-      if (r == cc) k += c;
+      if (r == cc) k += HET ? cbar[r] : c;
       return k;
     };
     for (int p = tid; p < npairs; p += 2 * NT) {
@@ -1105,7 +1150,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       __syncthreads();
       fail = fail_sh;
       {   // log det M and tr M^-1 in one team sum (sdiag was stored before the barrier above)
-        double ldp = (tid < U) ? log(mypiv) : 0.0, trp = (tid < U) ? sdiag[tid] : 0.0;
+        double ldp = (tid < U) ? log(mypiv) : 0.0, trp = (tid < U) ? (HET ? tw[tid] * sdiag[tid] : sdiag[tid]) : 0.0;
         tsum2<NW>(ldp, trp, red, flip);
         logdetM = ldp;
         tr_team = trp;
@@ -1135,16 +1180,18 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
         acc = (acc + acc1) + (acc2 + acc3);
       }
       beta[r] = acc;
-      const double kbv = (NW == 1) ? (q[r] - c * acc) / dR : (q[r] - c * acc) * inv_R;
+      const double cr = HET ? cbar[r] : c;
+      const double kbv = (NW == 1) ? (q[r] - cr * acc) / dR : (q[r] - cr * acc) * inv_R;
       kb[r] = kbv;
-      qkb += q[r] * kbv;
+      qkb += (HET ? q[r] / cr : q[r]) * kbv;
       kbkb += kbv * kbv;
     }
     WSTAMPX(5);
     tsum2<NW>(qkb, kbkb, red, flip);
     const double inv_c = (NW == 1) ? 1.0 / c : side[0];
-    const double quad = (NW == 1) ? (zz - qkb) / c : (zz - qkb) * inv_c;
-    const double nlml = 0.5 * ((double)N * LFM_LOG_2PI + (double)(N - U) * ((NW == 1) ? log(c) : side[1]) + logdetM + quad);
+    const double quad = HET ? zz - qkb : ((NW == 1) ? (zz - qkb) / c : (zz - qkb) * inv_c);
+    const double logc = HET ? lsum : (double)(N - U) * ((NW == 1) ? log(c) : side[1]);
+    const double nlml = 0.5 * ((double)N * LFM_LOG_2PI + logc + logdetM + quad);
     tsync<NW>();
     WSTAMP();
     // ---- I. fused derivative contraction over the lower triangle of the unique pairs --------------------
@@ -1205,6 +1252,16 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       dsum[r] = s0 + s1;
     }
     tsync<NW>();
+    double aa_het = 0.0;   // HET: alpha^T alpha; alpha_i into S[i] (free from here to the next step)
+    if constexpr (HET) {
+      for (int i = tid; i < N; i += NT) {
+        const double al = (ys[i] - mu[mflag[i] >> 1] * (double)(mflag[i] & 1) - kb[umap[i]]) / (vs[i] + c);
+        S[i] = al;
+        aa_het += al * al;
+      }
+      aa_het = tsum<NW>(aa_het, red, flip);
+      if constexpr (NW == 1) __syncwarp();
+    }
     WSTAMP();
     // ---- J. fold by gene; mean-function terms; sigma ---------------------------------------------
     if constexpr (NW == 1) {
@@ -1213,13 +1270,17 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       for (int i = 0; i < U; ++i) {
         if (pgene[i] == m) {
           gd += dsum[i];
-          gs += 1.0 - c * sdiag[i] - beta[i] * kb[i];
+          gs += 1.0 - (HET ? cbar[i] : c) * sdiag[i] - beta[i] * kb[i];
         }
       }
       // asum_m = sum_{i in positional block m} alpha_i,  alpha_i = (z_i - (K_u beta)_{u(i)}) / c
-      for (int i = m * blk; i < (m + 1) * blk; ++i)
-        asum += ys[i] - mu[m] * (double)(mflag[i] & 1) - kb[umap[i]];
-      asum /= c;
+      if constexpr (HET) {
+        for (int i = m * blk; i < (m + 1) * blk; ++i) asum += S[i];
+      } else {
+        for (int i = m * blk; i < (m + 1) * blk; ++i)
+          asum += ys[i] - mu[m] * (double)(mflag[i] & 1) - kb[umap[i]];
+        asum /= c;
+      }
       const double D = th[m], Sm = th[G + m], Bm = th[2 * G + m];
       gr[m] = gd + asum * Bm / (D * D);
       gr[G + m] = gs / Sm;
@@ -1234,11 +1295,11 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
         for (int i = hl; i < U; i += 16) {
           if (pgene[i] == m) {
             gd += dsum[i];
-            gs += 1.0 - c * sdiag[i] - beta[i] * kb[i];
+            gs += 1.0 - (HET ? cbar[i] : c) * sdiag[i] - beta[i] * kb[i];
           }
         }
         for (int i = m * blk + hl; i < (m + 1) * blk; i += 16)
-          asum += ys[i] - mu[m] * (double)(mflag[i] & 1) - kb[umap[i]];
+          asum += HET ? S[i] : ys[i] - mu[m] * (double)(mflag[i] & 1) - kb[umap[i]];
 #pragma unroll
         for (int o = 8; o > 0; o >>= 1) {
           gd += __shfl_xor_sync(hmask, gd, o);
@@ -1246,7 +1307,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
           asum += __shfl_xor_sync(hmask, asum, o);
         }
         if (hl == 0) {
-          asum *= inv_c;
+          if (!HET) asum *= inv_c;
           const double Bm = th[2 * G + m];
           const double rD = side[4 + P + m];
           gr[m] = gd + asum * Bm * rD * rD;
@@ -1259,14 +1320,15 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
     {
       double tr = 0.0;
       if constexpr (NW == 1) {
-        for (int i = tid; i < U; i += NT) tr += sdiag[i];
+        for (int i = tid; i < U; i += NT) tr += HET ? tw[i] * sdiag[i] : sdiag[i];
         tr = tsum<NW>(tr, red, flip);
       } else {
         tr = tr_team;
       }
       if (tid == 0) {
-        const double trSinv = (NW == 1) ? ((double)(N - U) + c * tr) / c : ((double)(N - U) + c * tr) * inv_c;
-        const double aa = (NW == 1) ? (zz - 2.0 * qkb + dR * kbkb) / (c * c) : (zz - 2.0 * qkb + dR * kbkb) * (inv_c * inv_c);
+        // HET: tr Sigma^-1 = tr0 + sum_u tw_u M^-1_uu (tr is that weighted sum)
+        const double trSinv = HET ? tr0 + tr : ((NW == 1) ? ((double)(N - U) + c * tr) / c : ((double)(N - U) + c * tr) * inv_c);
+        const double aa = HET ? aa_het : ((NW == 1) ? (zz - 2.0 * qkb + dR * kbkb) / (c * c) : (zz - 2.0 * qkb + dR * kbkb) * (inv_c * inv_c));
         gr[3 * G] = gl;
         gr[3 * G + 1] = sigma * (trSinv - aa);
       }
@@ -1356,18 +1418,18 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
 
 size_t lfm_batched_warp_structure_bytes(int N, int G, int MU, int MT) {
   if (MU <= 0 || MT <= 0) return 0;
-  const WarpLayout L = warp_layout(N, G, MU, MT, true);
+  const WarpLayout L = warp_layout(N, G, MU, MT, true, false);   // (the integer region does not depend on HET)
   return ((32 + (L.bytes - L.ints) + 8 * ((size_t)MT + (size_t)MT * MT)) + 15) & ~(size_t)15;
 }
 
 // Opt-in dynamic shared memory of one instantiation: only ever raised (the occupancy query and the launches of
 // differently sized problems share it).
-template <int NW>
+template <int NW, bool HET>
 static cudaError_t team_smem(size_t bytes) {
   static LfmSmemConfig conf;
-  return lfm_ensure_smem(lfm_batched_warp_kernel<NW>, conf, bytes);
+  return lfm_ensure_smem(lfm_batched_warp_kernel<NW, HET>, conf, bytes);
 }
-template <int NW> static int team_slots(size_t bytes);
+template <int NW, bool HET> static int team_slots(size_t bytes);
 __global__ void lfm_queue_init_kernel(int* base, int64_t B, int total) {
   const LfmQueue q = lfm_queue_view(base, B);
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -1375,9 +1437,9 @@ __global__ void lfm_queue_init_kernel(int* base, int64_t B, int total) {
   if (i < B) q.done[i] = 0;
   if (i < total) q.ring[i] = i < B ? (int)i : -1;
 }
-template <int NW>
+template <int NW, bool HET>
 static int team_launch(cudaStream_t st, const BatchedArgs& a, int time_grid, size_t bytes) {
-  LFM_CUDA_OK(team_smem<NW>(bytes));
+  LFM_CUDA_OK((team_smem<NW, HET>(bytes)));
   BatchedArgs b = a;
   unsigned grid = (unsigned)a.B;
   if (a.queue) {
@@ -1385,7 +1447,7 @@ static int team_launch(cudaStream_t st, const BatchedArgs& a, int time_grid, siz
     // than resident CTA slots, and not a whole number per SM (512 LFMs on 148 SMs: 68 SMs would carry 4 teams for the
     // whole fit and 80 SMs 3; with the queue an LFM moves to a free slot after every chunk and the loads average out).
     int dev = 0, sms = 0;
-    const int slots = team_slots<NW>(bytes);
+    const int slots = team_slots<NW, HET>(bytes);
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) sms = 0;
     const char* env = getenv("LFM_BATCHED_QUEUE");   // 0: never, 1: whenever a workspace is given (measurements)
     const int forced = env ? atoi(env) : -1;
@@ -1405,18 +1467,18 @@ static int team_launch(cudaStream_t st, const BatchedArgs& a, int time_grid, siz
       b.queue = nullptr;
     }
   }
-  lfm_batched_warp_kernel<NW><<<grid, 32 * NW, bytes, st>>>(b, time_grid);
+  lfm_batched_warp_kernel<NW, HET><<<grid, 32 * NW, bytes, st>>>(b, time_grid);
   LFM_LAUNCHED(1);
   LFM_CUDA_OK(cudaGetLastError());
   return LFM_OK;
 }
-template <int NW>
+template <int NW, bool HET>
 static int team_slots(size_t bytes) {   // LFMs of team size NW resident on the device at a time
   int dev = 0, sms = 0, per_sm = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
   if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-  if (team_smem<NW>(bytes) != cudaSuccess) return 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lfm_batched_warp_kernel<NW>, 32 * NW, bytes) != cudaSuccess) return 0;
+  if (team_smem<NW, HET>(bytes) != cudaSuccess) return 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lfm_batched_warp_kernel<NW, HET>, 32 * NW, bytes) != cudaSuccess) return 0;
   return sms * per_sm;
 }
 
@@ -1427,6 +1489,7 @@ static int team_slots(size_t bytes) {   // LFMs of team size NW resident on the 
 // A full GPU keeps the warp-per-LFM kernel (most LFMs resident per wave); a shard that leaves lanes idle -- the
 // multi-GPU case -- spends them on a shorter dependent chain per optimiser step.  Team 8 never wins (2 CTAs per SM)
 // and is only reachable through LFM_BATCHED_TEAM = 1 | 4 | 8, which overrides the choice (debug / measurements).
+template <bool HET>
 static int team_choice(int64_t B, size_t bytes, size_t bytes_team) {
   const char* env = getenv("LFM_BATCHED_TEAM");
   const int forced = env ? atoi(env) : 0;
@@ -1438,7 +1501,7 @@ static int team_choice(int64_t B, size_t bytes, size_t bytes_team) {
   const int dev_now = lfm_current_device();
   if (bytes != cached_bytes || bytes_team != cached_team || dev_now != cached_dev) {
     int dev = 0;
-    s1 = team_slots<1>(bytes); s4 = team_slots<4>(bytes_team);
+    s1 = team_slots<1, HET>(bytes); s4 = team_slots<4, HET>(bytes_team);
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) sms = 0;
     cached_bytes = bytes; cached_team = bytes_team; cached_dev = dev_now;
   }
@@ -1457,12 +1520,20 @@ int lfm_batched_warp_launch(cudaStream_t st, const BatchedArgs& a, int time_grid
   const int MU = a.max_unique;
   if (time_grid <= 0 || MU <= 0 || MU > 32 + WEX || a.N > 128 || P > 64) return LFM_ERR_UNSUPPORTED;
   if ((long long)a.G * time_grid * time_grid > 2048 || a.G > 127) return LFM_ERR_UNSUPPORTED;
-  const WarpLayout L = warp_layout(a.N, a.G, MU, time_grid, false), Lt = warp_layout(a.N, a.G, MU, time_grid, true);
+  const bool het = a.var != nullptr;
+  const WarpLayout L = warp_layout(a.N, a.G, MU, time_grid, false, het), Lt = warp_layout(a.N, a.G, MU, time_grid, true, het);
   if (Lt.bytes > 100 * 1024) return LFM_ERR_UNSUPPORTED;
-  switch (team_choice(a.B, L.bytes, Lt.bytes)) {
-    case 8: return team_launch<8>(st, a, time_grid, Lt.bytes);
-    case 4: return team_launch<4>(st, a, time_grid, Lt.bytes);
-    default: return team_launch<1>(st, a, time_grid, L.bytes);
+  if (het) {
+    switch (team_choice<true>(a.B, L.bytes, Lt.bytes)) {
+      case 8: return team_launch<8, true>(st, a, time_grid, Lt.bytes);
+      case 4: return team_launch<4, true>(st, a, time_grid, Lt.bytes);
+      default: return team_launch<1, true>(st, a, time_grid, L.bytes);
+    }
+  }
+  switch (team_choice<false>(a.B, L.bytes, Lt.bytes)) {
+    case 8: return team_launch<8, false>(st, a, time_grid, Lt.bytes);
+    case 4: return team_launch<4, false>(st, a, time_grid, Lt.bytes);
+    default: return team_launch<1, false>(st, a, time_grid, L.bytes);
   }
 }
 
@@ -1472,7 +1543,7 @@ int lfm_batched_warp_team(int64_t B, int N, int G, int MU, int time_grid) {
   const int P = 3 * G + 2;
   if (time_grid <= 0 || MU <= 0 || MU > 32 + WEX || N > 128 || P > 64) return 0;
   if ((long long)G * time_grid * time_grid > 2048 || G > 127) return 0;
-  const WarpLayout L = warp_layout(N, G, MU, time_grid, false), Lt = warp_layout(N, G, MU, time_grid, true);
+  const WarpLayout L = warp_layout(N, G, MU, time_grid, false, false), Lt = warp_layout(N, G, MU, time_grid, true, false);
   if (Lt.bytes > 100 * 1024) return 0;
-  return team_choice(B, L.bytes, Lt.bytes);
+  return team_choice<false>(B, L.bytes, Lt.bytes);
 }

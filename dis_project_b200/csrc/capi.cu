@@ -296,13 +296,15 @@ extern "C" int lfm_latent_posterior_host(lfm_handle* h, int64_t N, int G, const 
   return LFM_OK;
 }
 
-extern "C" int lfm_batched_fit_host(lfm_handle* h, int64_t B, int64_t N, int G, const double* X, const double* y,
-                                    const double* theta0, double jitter, double lr, double b1, double b2,
-                                    double eps, int steps, int fix_params, int steps_per_epoch, double* out_theta,
-                                    double* out_hist, int* info) {
+extern "C" int lfm_batched_fit_het_host(lfm_handle* h, int64_t B, int64_t N, int G, const double* X, const double* y,
+                                        const double* variances, const double* theta0, double jitter, double lr,
+                                        double b1, double b2, double eps, int steps, int fix_params,
+                                        int steps_per_epoch, double* out_theta, double* out_hist, int* info) {
   if (!h || B <= 0 || N <= 0 || G <= 0 || steps < 0 || !X || !y || !theta0 || !out_theta) return LFM_ERR_INVALID;
   const size_t P = 3 * (size_t)G + 2;
-  const size_t oX = 0, oy = oX + r2(3 * (size_t)N), oth = oy + r2((size_t)N), nin = oth + r2((size_t)B * P);
+  // [X | y | variances (when given) | theta0]: one host->device copy
+  const size_t nv = variances ? r2((size_t)N) : 0;
+  const size_t oX = 0, oy = oX + r2(3 * (size_t)N), ov = oy + r2((size_t)N), oth = ov + nv, nin = oth + r2((size_t)B * P);
   const size_t ou = nin, oadam = ou + r2((size_t)B * P), ohist = oadam + r2(2 * (size_t)B * P),
                ntot = ohist + r2((size_t)B * (size_t)(steps > 0 ? steps : 1));
   LFM_TRY(ensure((void**)&h->dbuf, &h->dbuf_bytes, ntot * 8, false));
@@ -318,14 +320,16 @@ extern "C" int lfm_batched_fit_host(lfm_handle* h, int64_t B, int64_t N, int G, 
   if (h->x_tg < 0) h->x_tg = lfm_count_distinct_times(N, X);
   if (B > 4096) { LFM_CUDA_OK(cudaMalloc((void**)&dinfo, (size_t)B * sizeof(int))); } else dinfo = h->dinfo;
   memcpy(hp + oy, y, (size_t)N * 8);
+  if (variances) memcpy(hp + ov, variances, (size_t)N * 8);
   memcpy(hp + oth, theta0, (size_t)B * P * 8);
   double* d = h->dbuf;
   int st = cudaMemcpyAsync(h->dbuf, hp, nin * 8, cudaMemcpyHostToDevice, h->stream) == cudaSuccess ? LFM_OK : LFM_ERR_CUDA;
   if (st == LFM_OK) st = lfm_unconstrain(h->stream, B, G, d + oth, d + ou);
   if (st == LFM_OK)
-    st = lfm_batched_fit_tg(h->stream, B, N, G, d + oX, d + oy, d + ou, d + oadam, jitter, lr, b1, b2, eps, 0, steps,
-                            steps, fix_params, steps_per_epoch, lfm_count_unique_rows(N, X),
-                            (int)h->x_tg, d + ohist, steps, d + oth, dinfo, nullptr, nullptr);
+    st = lfm_batched_fit_het(h->stream, B, N, G, d + oX, d + oy, 0, variances ? d + ov : nullptr, 0, d + ou, d + oadam,
+                             jitter, lr, b1, b2, eps, 0, steps, steps, fix_params, steps_per_epoch,
+                             lfm_count_unique_rows(N, X), (int)h->x_tg, d + ohist, steps, d + oth, dinfo, nullptr,
+                             nullptr, nullptr, 0, nullptr, 0);
   // d + oth (the start points, dead after lfm_unconstrain) receives the constrained result
   if (st == LFM_OK) {
     cudaMemcpyAsync(hp + ou, d + oth, (size_t)B * P * 8, cudaMemcpyDeviceToHost, h->stream);
@@ -339,4 +343,11 @@ extern "C" int lfm_batched_fit_host(lfm_handle* h, int64_t B, int64_t N, int G, 
   }
   if (B > 4096) cudaFree(dinfo);
   return st;
+}
+extern "C" int lfm_batched_fit_host(lfm_handle* h, int64_t B, int64_t N, int G, const double* X, const double* y,
+                                    const double* theta0, double jitter, double lr, double b1, double b2,
+                                    double eps, int steps, int fix_params, int steps_per_epoch, double* out_theta,
+                                    double* out_hist, int* info) {
+  return lfm_batched_fit_het_host(h, B, N, G, X, y, nullptr, theta0, jitter, lr, b1, b2, eps, steps, fix_params,
+                                  steps_per_epoch, out_theta, out_hist, info);
 }

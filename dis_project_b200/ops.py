@@ -356,10 +356,30 @@ def _batched_y(y, B: int, N: int) -> Tuple[torch.Tensor, int]:
     return y, 0
 
 
-def batched_nlml_grad_unc(X, y, theta_unc, jitter: float, G: int, time_grid: Optional[int] = None):
+def _variance_layout(shape, B: int, N: int) -> bool:
+    """Shape of the measurement variances of the batched heteroscedastic objective: (B, N) -> True, one row per LFM
+    (mirrors `_batched_y`); (N,) or (N, 1) -> False, shared by every LFM.  Anything else raises ValueError."""
+    shape = tuple(int(n) for n in shape)
+    if shape == (B, N) and B != 1:
+        return True
+    if shape in ((N,), (N, 1)) or (B == 1 and shape == (1, N)):
+        return False
+    raise ValueError(f"variances must be (N,), (N, 1) with N={N} (shared) or (B, N)=({B}, {N}) (one row per LFM), "
+                     f"got {shape}")
+
+
+def _batched_variances(variances, B: int, N: int) -> Tuple[torch.Tensor, int]:
+    """variances -> (device tensor, var_stride): 0 when shared, N when one row per LFM."""
+    v = _dev(variances)
+    return (v, N) if _variance_layout(v.shape, B, N) else (v.reshape(-1), 0)
+
+
+def batched_nlml_grad_unc(X, y, theta_unc, jitter: float, G: int, time_grid: Optional[int] = None, variances=None):
     """B independent value_and_grad evaluations.  theta_unc (B, P) -> (val[B], grad[B,P], info[B]).
     y is (N,) -- every LFM sees the same observations -- or (B, N): LFM b sees y[b] (replicas / candidate TFs).
-    `time_grid`: bound on the distinct times of X (None: counted from X; 0: one CTA per LFM, no tables)."""
+    `time_grid`: bound on the distinct times of X (None: counted from X; 0: one CTA per LFM, no tables).
+    `variances`: None, or the measurement variances of the heteroscedastic objective (Sigma += diag(variances),
+    include/lfm_b200.h, lfm_batched_nlml_grad_unc_het): (N,) / (N, 1) shared, or (B, N) one row per LFM."""
     hint = unique_rows(X)
     tg = distinct_times(X) if time_grid is None else int(time_grid)
     _check_training_flags(X)
@@ -370,10 +390,17 @@ def batched_nlml_grad_unc(X, y, theta_unc, jitter: float, G: int, time_grid: Opt
         raise ValueError(f"theta_unc must be (B, {P})")
     B, N = u.shape[0], X.shape[0]
     y, y_stride = _batched_y(y, B, N)
+    v, v_stride = _batched_variances(variances, B, N) if variances is not None else (None, 0)
     val = torch.empty(B, dtype=F64, device=X.device)
     grad = torch.empty((B, P), dtype=F64, device=X.device)
     info = torch.zeros(B, dtype=torch.int32, device=X.device)
     if B == 0:
+        return val, grad, info
+    if v is not None:
+        _lib.check(_lib.lib().lfm_batched_nlml_grad_unc_het(_stream(), B, N, G, X.data_ptr(), y.data_ptr(), y_stride,
+                                                            v.data_ptr(), v_stride, u.data_ptr(), float(jitter), hint, tg,
+                                                            val.data_ptr(), grad.data_ptr(), info.data_ptr()),
+                   "lfm_batched_nlml_grad_unc_het")
         return val, grad, info
     _lib.check(_lib.lib().lfm_batched_nlml_grad_unc_multi(_stream(), B, N, G, X.data_ptr(), y.data_ptr(), y_stride,
                                                           u.data_ptr(), float(jitter), hint, tg, val.data_ptr(),
@@ -488,9 +515,11 @@ def loss_key_to_float(keys):
 def batched_fit_steps(state: BatchedFitState, X, y, jitter: float, steps: int, *, lr: float = 0.01,
                       b1: float = 0.9, b2: float = 0.999, eps: float = 1e-8, fix_params: bool = True,
                       steps_per_epoch: int = 1000, best_key: Optional[torch.Tensor] = None,
-                      step_keys: Optional[torch.Tensor] = None, queue_chunk: int = 0) -> None:
+                      step_keys: Optional[torch.Tensor] = None, queue_chunk: int = 0, variances=None) -> None:
     """Advance every fit in `state` by `steps` optimiser steps (reference src/trainer.py:201-216).
     y is (N,) (multi-start: one data set, B start points) or (B, N) (one row of observations per LFM).
+    `variances`: None, or the measurement variances of the heteroscedastic objective, (N,) / (N, 1) shared or (B, N)
+    one row per LFM (lfm_batched_fit_het, include/lfm_b200.h).
     `best_key`: one int64 device word, atomicMin of the loss keys after the last step of this call; `step_keys`:
     total_steps int64 device words, word s = atomicMin of the loss keys at step s (include/lfm_b200.h).
     `queue_chunk` > 0 with the whole fit in this one call: lfm_batched_fit_queue (persistent workers, tasks of
@@ -502,6 +531,7 @@ def batched_fit_steps(state: BatchedFitState, X, y, jitter: float, steps: int, *
         state.time_grid = distinct_times(X)
     X = _rows3(X, "x")
     y, y_stride = _batched_y(y, state.B, X.shape[0])
+    v, v_stride = _batched_variances(variances, state.B, X.shape[0]) if variances is not None else (None, 0)
     if state.B == 0 or steps <= 0:
         return
     steps = min(steps, state.total_steps - state.step)
@@ -510,6 +540,10 @@ def batched_fit_steps(state: BatchedFitState, X, y, jitter: float, steps: int, *
         state.struct_cache = torch.empty(max(nb, 16), dtype=torch.uint8, device=X.device)  # written by the first launch
     if step_keys is not None and step_keys.numel() < state.total_steps:
         raise ValueError("step_keys must hold one int64 word per step of the fit")
+    if v is not None:
+        _batched_fit_het(state, X, y, y_stride, v, v_stride, jitter, steps, lr, b1, b2, eps, fix_params, steps_per_epoch,
+                         best_key, step_keys, queue_chunk)
+        return
     if queue_chunk > 0 and state.step == 0 and steps == state.total_steps:
         # the whole fit in one launch: persistent workers + task queue where a static assignment would be unbalanced
         # (lfm_batched_fit_queue, include/lfm_b200.h); the library ignores the queue where it does not pay
@@ -539,6 +573,28 @@ def batched_fit_steps(state: BatchedFitState, X, y, jitter: float, steps: int, *
                                                 step_keys.data_ptr() if step_keys is not None else None,
                                                 state.struct_cache.data_ptr()),
                "lfm_batched_fit_trace")
+    state.step += steps
+
+
+def _batched_fit_het(state, X, y, y_stride, v, v_stride, jitter, steps, lr, b1, b2, eps, fix_params, steps_per_epoch,
+                     best_key, step_keys, queue_chunk) -> None:
+    """batched_fit_steps with variances: one entry point (lfm_batched_fit_het) for the chunked and the queue launches."""
+    l = _lib.lib()
+    qb = 0
+    if queue_chunk > 0 and state.step == 0 and steps == state.total_steps:
+        qb = int(l.lfm_batched_queue_bytes(state.B, state.total_steps, int(queue_chunk)))
+        if qb > 0 and (state.queue_ws is None or state.queue_ws.numel() < qb):
+            state.queue_ws = torch.empty(qb, dtype=torch.uint8, device=X.device)
+    _lib.check(l.lfm_batched_fit_het(_stream(), state.B, X.shape[0], state.G, X.data_ptr(), y.data_ptr(), y_stride,
+                                     v.data_ptr(), v_stride, state.u.data_ptr(), state.adam.data_ptr(), float(jitter), lr,
+                                     b1, b2, eps, state.step, steps, state.total_steps, int(bool(fix_params)),
+                                     int(steps_per_epoch), state.unique_hint, int(state.time_grid), state.hist.data_ptr(),
+                                     state.hist.shape[1], state.theta.data_ptr(), state.info.data_ptr(),
+                                     best_key.data_ptr() if best_key is not None else None,
+                                     step_keys.data_ptr() if step_keys is not None else None,
+                                     state.struct_cache.data_ptr(), int(queue_chunk) if qb > 0 else 0,
+                                     state.queue_ws.data_ptr() if qb > 0 else None, qb),
+               "lfm_batched_fit_het")
     state.step += steps
 
 

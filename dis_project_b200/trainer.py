@@ -63,7 +63,9 @@ class JaxTrainer:
         n = self.training_data.n
         return (isinstance(self.objective, CustomConjMLL) and self.objective.negative
                 and isinstance(self.optim, GradientTransformation) and self.optim.name == "adam"
-                and getattr(self.objective, "variances", None) is None  # the batched kernels have no variance term
+                # with variances the fit stays the host loop of dense evaluations (the batched kernels have the
+                # heteroscedastic objective too, lfm_batched_fit_het, but this path is not routed to them)
+                and getattr(self.objective, "variances", None) is None
                 and n <= 128 and n % self.model.num_genes == 0 and not self.track_parameters)
 
     def fit(self, fix_params: Optional[bool] = True, num_steps_per_epoch: Optional[int] = 1000) -> tuple:

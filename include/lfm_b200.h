@@ -253,6 +253,34 @@ int lfm_batched_fit_queue(lfm_stream_t stream, int64_t B, int64_t N, int G, cons
  * chunked fit.  The call with first_step == 0 stores the structure of X (duplicate rows, distinct times and time
  * differences, pair table) there; calls with first_step > 0 load it instead of repeating the O(N^2) scans. */
 size_t lfm_batched_structure_bytes(int64_t N, int G, int unique_rows_hint, int time_grid_hint);
+/* ---- batched fits with measurement variances: the heteroscedastic objective of lfm_nlml_grad_unc_het_tg ------------
+ * Sigma = K + diag(v) + (jitter + sigma^2) I, i.e. noise c_i = v_i + jitter + sigma^2 per point.  `variances` is N
+ * device doubles shared by every LFM (var_stride 0) or one row per LFM at variances + b * var_stride (var_stride >= N),
+ * as y / y_stride; NULL means exactly lfm_batched_nlml_grad_unc_multi / lfm_batched_fit_trace / _fit_queue.
+ * The duplicate-row compression stays exact with a noise per point (same rule for U and R as above): per unique row u
+ *   omega_u = sum_{i in u} 1/c_i, omega2_u = sum_{i in u} 1/c_i^2, cbar_u = R / omega_u, q_u = cbar_u sum_{i in u} z_i/c_i,
+ *   M = diag(cbar) + R K_u,  beta = M^-1 q = P^T alpha,  K_u beta = (q - cbar o beta) / R,
+ *   log det Sigma = sum_i log c_i - sum_u log cbar_u + log det M,
+ *   z^T Sigma^-1 z = sum_i z_i^2/c_i - sum_u (q_u/cbar_u) (K_u beta)_u,
+ *   P^T Kbar P = 1/2 (R M^-1 - beta beta^T) (the kernel-parameter weights: unchanged),
+ *   diag(P^T Kbar P K_u)_u = 1/2 (1 - cbar_u M^-1_uu - beta_u (K_u beta)_u),   alpha_i = (z_i - (K_u beta)_u(i)) / c_i,
+ *   tr Sigma^-1 = sum_i 1/c_i - sum_u omega2_u/omega_u + R sum_u omega2_u M^-1_uu / omega_u^2,
+ *   dNLML/dsigma = sigma (tr Sigma^-1 - alpha^T alpha);
+ * with v = 0 every line is the homoscedastic one.  Every c_i must be > 0: otherwise (or with NaN variances) info = 1 and
+ * the loss / gradient are NaN, as for a failed factorisation. */
+int lfm_batched_nlml_grad_unc_het(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
+                                  int64_t y_stride, const double* variances, int64_t var_stride,
+                                  const double* theta_unc, double jitter, int unique_rows_hint, int time_grid_hint,
+                                  double* out_val, double* out_grad, int* info);
+/* lfm_batched_fit_trace with variances; with `queue_ws` non-NULL it is lfm_batched_fit_queue instead (then first_step must
+ * be 0 and steps == total_steps: the queue runs the whole fit). */
+int lfm_batched_fit_het(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
+                        int64_t y_stride, const double* variances, int64_t var_stride, double* theta_unc_io,
+                        double* adam_state, double jitter, double lr, double b1, double b2, double eps, int first_step,
+                        int steps, int total_steps, int fix_params, int steps_per_epoch, int unique_rows_hint,
+                        int time_grid_hint, double* out_hist, int64_t ld_hist, double* out_theta, int* info,
+                        long long* best_key, long long* step_keys, void* structure_cache, int chunk_steps,
+                        void* queue_ws, size_t queue_bytes);
 /* best_key (may be NULL): one device word that receives atomicMin over the batch of the order-preserving integer
  * image of each LFM's loss after the last step of this call (finite losses only; initialise it to INT64_MAX).
  * key(v) = bits(v) for v >= 0, bits(v) ^ 0x7fff...f otherwise -- monotone in v, so the global best objective of a
@@ -262,7 +290,9 @@ size_t lfm_batched_structure_bytes(int64_t N, int G, int unique_rows_hint, int t
 /* Warps per LFM the batched entry points use for a batch of B LFMs of this shape on the current device: 1 (one warp per
  * LFM, register-resident Cholesky; a full GPU), 4 (a team of four warps per LFM, symmetric sweep in register tiles;
  * shards that leave SMs idle, e.g. 4096 restarts over 8 GPUs), or 0 when the shape runs the CTA-per-LFM kernel.
- * LFM_BATCHED_TEAM = 1 | 4 | 8 in the environment overrides the choice (measurements). */
+ * LFM_BATCHED_TEAM = 1 | 4 | 8 in the environment overrides the choice (measurements).  The answer is for the entry
+ * points without variances: the _het ones keep N + 2U more doubles per LFM in shared memory and choose from their own
+ * occupancy. */
 int lfm_batched_team_size(int64_t B, int64_t N, int G, int unique_rows_hint, int time_grid_hint);
 
 /* Winner of a shard after a fit: out_packed (P + 2 doubles) = [loss, id, theta(P)] of the LFM with the smallest FINITE
@@ -326,6 +356,12 @@ int lfm_batched_fit_host(lfm_handle* h, int64_t B, int64_t N, int G, const doubl
                          const double* theta0, double jitter, double lr, double b1, double b2,
                          double eps, int steps, int fix_params, int steps_per_epoch, double* out_theta,
                          double* out_hist, int* info);
+/* lfm_batched_fit_host with measurement variances (N host doubles, staged in the same single host->device copy as X, y
+ * and theta0; the objective of lfm_batched_fit_het) or NULL (= lfm_batched_fit_host). */
+int lfm_batched_fit_het_host(lfm_handle* h, int64_t B, int64_t N, int G, const double* X, const double* y,
+                             const double* variances, const double* theta0, double jitter, double lr, double b1,
+                             double b2, double eps, int steps, int fix_params, int steps_per_epoch, double* out_theta,
+                             double* out_hist, int* info);
 
 /* ---- diagnostics used by bench.py for the roofline denominators ------------------------------ */
 
