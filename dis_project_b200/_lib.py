@@ -91,6 +91,11 @@ SIGNATURES = {
     "lfm_batched_fit_het": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl,
                                    _dbl, _int, _int, _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _ptr,
                                    _int, _ptr, _sz]),
+    "lfm_batched_posterior_workspace_bytes": (_sz, [_i64, _i64, _int, _i64, _int, _int]),
+    "lfm_batched_latent_posterior": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _dbl, _i64, _ptr,
+                                            _int, _ptr, _sz, _ptr, _ptr, _ptr]),
+    "lfm_batched_gene_posterior": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _dbl, _i64, _ptr,
+                                          _int, _ptr, _sz, _ptr, _ptr, _ptr, _ptr]),
     "lfm_batched_structure_bytes": (_sz, [_i64, _int, _int, _int]),
     "lfm_batched_team_size": (_int, [_i64, _i64, _int, _int, _int]),
     "lfm_batched_best": (_int, [_ptr, _i64, _int, _ptr, _i64, _i64, _ptr, _dbl, _ptr]),

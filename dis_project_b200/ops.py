@@ -409,6 +409,67 @@ def batched_nlml_grad_unc(X, y, theta_unc, jitter: float, G: int, time_grid: Opt
     return val, grad, info
 
 
+def _batched_posterior(fn_name: str, gene: bool, X, y, variances, theta, jitter: float, Xstar, G: int,
+                       full_cov: bool):
+    """Shared body of batched_latent_posterior / batched_gene_posterior (lfm_batched_*_posterior, include/lfm_b200.h)."""
+    import numpy as np
+
+    if variances is None:
+        raise ValueError("variances are required (the posteriors' training covariance is K + diag(variances) + ...)")
+    _check_training_flags(X)
+    shape = lambda a: tuple(a.shape) if hasattr(a, "shape") else np.shape(a)   # checked before any device copy
+    P = 3 * G + 2
+    for name, s in (("x", shape(X)), ("test_inputs", shape(Xstar))):
+        if len(s) != 2 or s[1] != 3:
+            raise ValueError(f"{name} must have shape (n, 3) = [time, gene_index, flag] (dataset.py:391), got {s}")
+    if len(shape(theta)) != 2 or shape(theta)[1] != P:
+        raise ValueError(f"theta must be (B, {P}) constrained [d,s,b,l,sigma] rows, got {shape(theta)}")
+    B, N, T = shape(theta)[0], shape(X)[0], shape(Xstar)[0]
+    if shape(y) != (B, N) and int(np.prod(shape(y))) != N:
+        raise ValueError(f"y must hold N={N} observations (shared) or be (B, N)=({B}, {N}) (one row per LFM), "
+                         f"got {shape(y)}")
+    _variance_layout(shape(variances), B, N)
+    if N % G or (gene and T % G):
+        raise ValueError("mean_function: rows must be divisible by num_genes (model.py:145-149)")
+    hint = unique_rows(X)
+    X, Xs, th = _rows3(X, "x"), _rows3(Xstar, "test_inputs"), _dev(theta)
+    y, y_stride = _batched_y(y, B, N)
+    v, v_stride = _batched_variances(variances, B, N)
+    dev = X.device
+    mean = torch.empty((B, T), dtype=F64, device=dev)
+    var = torch.empty((B, T), dtype=F64, device=dev)
+    cov = torch.empty((B, T, T), dtype=F64, device=dev) if full_cov else None
+    info = torch.zeros(B, dtype=torch.int32, device=dev)
+    if B == 0 or (T == 0 and not gene):
+        return mean, cov, var, info
+    l = _lib.lib()
+    ws = _workspace(max(int(l.lfm_batched_posterior_workspace_bytes(B, N, G, T, hint, int(bool(full_cov)))), 16), dev,
+                    "bpost")
+    args = [_stream(), B, N, G, X.data_ptr(), y.data_ptr(), y_stride, v.data_ptr(), v_stride, th.data_ptr(),
+            float(jitter), T, Xs.data_ptr(), hint, ws.data_ptr(), ws.numel(), mean.data_ptr()]
+    if gene:
+        args.append(cov.data_ptr() if full_cov else None)
+    args += [var.data_ptr(), info.data_ptr()]
+    _lib.check(getattr(l, fn_name)(*args), fn_name)
+    return mean, cov, var, info
+
+
+def batched_latent_posterior(X, y, variances, theta, jitter: float, Xstar, G: int):
+    """ExactLFM.latent_predict (reference src/model.py:420-463) of B LFMs in one launch: theta (B, P) constrained (e.g.
+    MultiStartResult.theta), y (N,) or (B, N), variances (N,), (N, 1) or (B, N).  Returns (mean (B, T*), var (B, T*),
+    info (B,)); info as lfm_batched_latent_posterior (include/lfm_b200.h), a failed LFM has NaN outputs."""
+    mean, _, var, info = _batched_posterior("lfm_batched_latent_posterior", False, X, y, variances, theta, jitter, Xstar,
+                                            G, False)
+    return mean, var, info
+
+
+def batched_gene_posterior(X, y, variances, theta, jitter: float, Xstar, G: int, full_cov: bool = False):
+    """ExactLFM.multi_gene_predict (reference src/model.py:465-514) of B LFMs in one launch; arguments as
+    batched_latent_posterior.  Returns (mean (B, T*), cov (B, T*, T*) or None, var (B, T*), info (B,))."""
+    return _batched_posterior("lfm_batched_gene_posterior", True, X, y, variances, theta, jitter, Xstar, G,
+                              bool(full_cov))
+
+
 class BatchedFitState:
     """Device-resident state of B independent fits (iterates, Adam moments, loss history).
 

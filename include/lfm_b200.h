@@ -281,6 +281,35 @@ int lfm_batched_fit_het(lfm_stream_t stream, int64_t B, int64_t N, int G, const 
                         int time_grid_hint, double* out_hist, int64_t ld_hist, double* out_theta, int* info,
                         long long* best_key, long long* step_keys, void* structure_cache, int chunk_steps,
                         void* queue_ws, size_t queue_bytes);
+/* ---- batched posteriors: latent_predict / multi_gene_predict of B fitted LFMs in one launch ---------------------------
+ * B LFMs share X (N <= 128 rows) and the test inputs Xstar (T* rows); LFM b has its own CONSTRAINED theta (theta +
+ * b * P), observations (y, y_stride) and variances (variances, var_stride), with the meaning of lfm_batched_fit_het
+ * (stride 0: shared; N or more: one row per LFM).  `variances` is required, as for lfm_latent_posterior.  The
+ * duplicate-row compression of the batched fits (same rule for U and R, unique_rows_hint as there) with a noise c_i
+ * per point: omega_u = sum_{i in u} 1/c_i, cbar_u = R / omega_u, q_u = cbar_u sum_{i in u} z_i / c_i,
+ * M = diag(cbar) + R K_u = L L^T, beta = M^-1 q = P^T alpha, and P^T Sigma^-1 P = R M^-1.  With k_*u the
+ * cross-covariance of a test row with the U unique rows (the flag-aware pair function of lfm_cross_covariance):
+ *   latent (c_i = v_i + jitter):   mean = mean_t + k_*u^T beta,  var = k(t*,t*) + 2 jitter - R ||L^-1 k_*u||^2;
+ *   gene   (c_i = v_i + sigma^2):  mean = mean_t + k_*u^T beta,  cov = K_tt - R V^T V + jitter I, V = L^-1 K_ut,
+ *                                  var = diag(cov);
+ * mean_t, k(t*,t*) and the positional blocks T* / G as lfm_latent_posterior / lfm_gene_posterior.  Outputs are B x T*
+ * (out_mean, out_var) and B x T* x T* (out_cov, may be NULL; out_var of the gene posterior may be NULL too); info
+ * (B ints): 0, k > 0 the failing pivot of M, 1 some c_i <= 0 or NaN, -1 unique_rows_hint smaller than U.  A failed LFM
+ * gets NaN outputs and affects no other.  LFM b's outputs are bit-identical whatever B is and wherever b sits.  The
+ * workspace (lfm_batched_posterior_workspace_bytes, full_cov = out_cov != NULL) holds the structure of X and, with
+ * the full covariance, V of every LFM (B x U x T* doubles).  N > 128: LFM_ERR_UNSUPPORTED; Tstar % G must be 0 for the
+ * gene posterior. */
+size_t lfm_batched_posterior_workspace_bytes(int64_t B, int64_t N, int G, int64_t Tstar, int unique_rows_hint,
+                                             int full_cov);
+int lfm_batched_latent_posterior(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
+                                 int64_t y_stride, const double* variances, int64_t var_stride, const double* theta,
+                                 double jitter, int64_t Tstar, const double* Xstar, int unique_rows_hint, void* ws,
+                                 size_t ws_bytes, double* out_mean, double* out_var, int* info);
+int lfm_batched_gene_posterior(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
+                               int64_t y_stride, const double* variances, int64_t var_stride, const double* theta,
+                               double jitter, int64_t Tstar, const double* Xstar, int unique_rows_hint, void* ws,
+                               size_t ws_bytes, double* out_mean, double* out_cov, double* out_var, int* info);
+
 /* best_key (may be NULL): one device word that receives atomicMin over the batch of the order-preserving integer
  * image of each LFM's loss after the last step of this call (finite losses only; initialise it to INT64_MAX).
  * key(v) = bits(v) for v >= 0, bits(v) ^ 0x7fff...f otherwise -- monotone in v, so the global best objective of a
