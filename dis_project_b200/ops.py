@@ -4,6 +4,7 @@ path.  All calls are stream-ordered on torch's current stream and do not synchro
 """
 from __future__ import annotations
 
+import math
 from typing import Dict, Optional, Tuple
 
 import torch
@@ -345,15 +346,21 @@ def unique_rows(X) -> int:
     return int(_lib.lib().lfm_count_unique_rows(Xh.shape[0], Xh.ctypes.data))
 
 
+def _y_layout(shape, B: int, N: int) -> bool:
+    """Shape of the observations of B batched LFMs: (B, N) -> True, one row per LFM; N values -> False, shared by every
+    LFM.  Anything else raises ValueError."""
+    shape = tuple(int(n) for n in shape)
+    if shape == (B, N) and not (B == N == 1):
+        return True
+    if math.prod(shape) == N:
+        return False
+    raise ValueError(f"y must hold N={N} observations (shared) or be (B, N)=({B}, {N}) (one row per LFM), got {shape}")
+
+
 def _batched_y(y, B: int, N: int) -> Tuple[torch.Tensor, int]:
     """y (N,) shared by every LFM -> (y, 0); y (B, N), one row of observations per LFM -> (y, N)."""
     y = _dev(y)
-    if y.ndim == 2 and y.shape[0] == B and y.shape[1] == N and not (B == N and N == 1):
-        return y, N
-    y = y.reshape(-1)
-    if y.numel() != N:
-        raise ValueError(f"y must hold N={N} observations (shared) or be (B, N)=({B}, {N}) (one row per LFM), got {tuple(y.shape)}")
-    return y, 0
+    return (y, N) if _y_layout(y.shape, B, N) else (y.reshape(-1), 0)
 
 
 def _variance_layout(shape, B: int, N: int) -> bool:
@@ -573,6 +580,40 @@ def loss_key_to_float(keys):
     return out
 
 
+def _structure_cache(state: BatchedFitState, N: int, device) -> None:
+    """The device bytes that carry the structure of X from the first launch of a fit to the later ones, sized for the
+    state's unique-row hint and distinct-time bound (grown, never shrunk)."""
+    nb = max(int(_lib.lib().lfm_batched_structure_bytes(N, state.G, state.unique_hint, int(state.time_grid))), 16)
+    if state.struct_cache is None or state.struct_cache.numel() < nb:
+        state.struct_cache = torch.empty(nb, dtype=torch.uint8, device=device)
+
+
+def _bind_fit(state: BatchedFitState, X: torch.Tensor, y: torch.Tensor, y_stride: int, v: Optional[torch.Tensor],
+              var_stride: int, jitter: float, lr: float, b1: float, b2: float, eps: float, fix_params: bool,
+              steps_per_epoch: int, step_keys: Optional[torch.Tensor], queue_chunk: int):
+    """lfm_batched_fit_het over `state` with every argument bound but the stream, the step range and `best_key`: returns
+    launch(stream, first_step, steps, best_key_ptr).  Bound once per fit, so that a launch per optimiser step costs one
+    ctypes call.  `queue_chunk` > 0 only when one launch runs the whole fit: persistent workers over a device-side queue
+    of `queue_chunk`-step tasks (include/lfm_b200.h; the library ignores the queue where it does not pay)."""
+    l = _lib.lib()
+    qb = int(l.lfm_batched_queue_bytes(state.B, state.total_steps, int(queue_chunk))) if queue_chunk > 0 else 0
+    if qb > 0 and (state.queue_ws is None or state.queue_ws.numel() < qb):
+        state.queue_ws = torch.empty(qb, dtype=torch.uint8, device=X.device)
+    head = (state.B, X.shape[0], state.G, X.data_ptr(), y.data_ptr(), y_stride, v.data_ptr() if v is not None else None,
+            var_stride, state.u.data_ptr(), state.adam.data_ptr(), float(jitter), float(lr), float(b1), float(b2),
+            float(eps))
+    mid = (state.total_steps, int(bool(fix_params)), int(steps_per_epoch), state.unique_hint, int(state.time_grid),
+           state.hist.data_ptr(), state.hist.shape[1], state.theta.data_ptr(), state.info.data_ptr())
+    tail = (step_keys.data_ptr() if step_keys is not None else None, state.struct_cache.data_ptr(),
+            int(queue_chunk) if qb > 0 else 0, state.queue_ws.data_ptr() if qb > 0 else None, qb)
+    fit, check = l.lfm_batched_fit_het, _lib.check
+
+    def launch(stream: int, first_step: int, steps: int, best_key: Optional[int]) -> None:
+        check(fit(stream, *head, first_step, steps, *mid, best_key, *tail), "lfm_batched_fit_het")
+
+    return launch
+
+
 def batched_fit_steps(state: BatchedFitState, X, y, jitter: float, steps: int, *, lr: float = 0.01,
                       b1: float = 0.9, b2: float = 0.999, eps: float = 1e-8, fix_params: bool = True,
                       steps_per_epoch: int = 1000, best_key: Optional[torch.Tensor] = None,
@@ -583,8 +624,8 @@ def batched_fit_steps(state: BatchedFitState, X, y, jitter: float, steps: int, *
     one row per LFM (lfm_batched_fit_het, include/lfm_b200.h).
     `best_key`: one int64 device word, atomicMin of the loss keys after the last step of this call; `step_keys`:
     total_steps int64 device words, word s = atomicMin of the loss keys at step s (include/lfm_b200.h).
-    `queue_chunk` > 0 with the whole fit in this one call: lfm_batched_fit_queue (persistent workers, tasks of
-    `queue_chunk` steps)."""
+    `queue_chunk` > 0 with the whole fit in this one call: persistent workers over a task queue of `queue_chunk`-step
+    tasks (the queue mode of lfm_batched_fit_het)."""
     if state.unique_hint == 0:
         state.unique_hint = unique_rows(X)
         _check_training_flags(X)
@@ -596,66 +637,13 @@ def batched_fit_steps(state: BatchedFitState, X, y, jitter: float, steps: int, *
     if state.B == 0 or steps <= 0:
         return
     steps = min(steps, state.total_steps - state.step)
-    if state.struct_cache is None:
-        nb = int(_lib.lib().lfm_batched_structure_bytes(X.shape[0], state.G, state.unique_hint, int(state.time_grid)))
-        state.struct_cache = torch.empty(max(nb, 16), dtype=torch.uint8, device=X.device)  # written by the first launch
+    _structure_cache(state, X.shape[0], X.device)
     if step_keys is not None and step_keys.numel() < state.total_steps:
         raise ValueError("step_keys must hold one int64 word per step of the fit")
-    if v is not None:
-        _batched_fit_het(state, X, y, y_stride, v, v_stride, jitter, steps, lr, b1, b2, eps, fix_params, steps_per_epoch,
-                         best_key, step_keys, queue_chunk)
-        return
-    if queue_chunk > 0 and state.step == 0 and steps == state.total_steps:
-        # the whole fit in one launch: persistent workers + task queue where a static assignment would be unbalanced
-        # (lfm_batched_fit_queue, include/lfm_b200.h); the library ignores the queue where it does not pay
-        l = _lib.lib()
-        qb = int(l.lfm_batched_queue_bytes(state.B, state.total_steps, int(queue_chunk)))
-        if qb > 0:
-            if state.queue_ws is None or state.queue_ws.numel() < qb:
-                state.queue_ws = torch.empty(qb, dtype=torch.uint8, device=X.device)
-            _lib.check(l.lfm_batched_fit_queue(_stream(), state.B, X.shape[0], state.G, X.data_ptr(), y.data_ptr(), y_stride,
-                                               state.u.data_ptr(), state.adam.data_ptr(), float(jitter), lr, b1, b2, eps,
-                                               state.total_steps, int(bool(fix_params)), int(steps_per_epoch),
-                                               state.unique_hint, int(state.time_grid), state.hist.data_ptr(),
-                                               state.hist.shape[1], state.theta.data_ptr(), state.info.data_ptr(),
-                                               best_key.data_ptr() if best_key is not None else None,
-                                               step_keys.data_ptr() if step_keys is not None else None,
-                                               state.struct_cache.data_ptr(), int(queue_chunk), state.queue_ws.data_ptr(), qb),
-                       "lfm_batched_fit_queue")
-            state.step += steps
-            return
-    _lib.check(_lib.lib().lfm_batched_fit_trace(_stream(), state.B, X.shape[0], state.G, X.data_ptr(), y.data_ptr(),
-                                                y_stride, state.u.data_ptr(), state.adam.data_ptr(), float(jitter), lr,
-                                                b1, b2, eps, state.step, steps, state.total_steps,
-                                                int(bool(fix_params)), int(steps_per_epoch), state.unique_hint,
-                                                int(state.time_grid), state.hist.data_ptr(), state.hist.shape[1],
-                                                state.theta.data_ptr(), state.info.data_ptr(),
-                                                best_key.data_ptr() if best_key is not None else None,
-                                                step_keys.data_ptr() if step_keys is not None else None,
-                                                state.struct_cache.data_ptr()),
-               "lfm_batched_fit_trace")
-    state.step += steps
-
-
-def _batched_fit_het(state, X, y, y_stride, v, v_stride, jitter, steps, lr, b1, b2, eps, fix_params, steps_per_epoch,
-                     best_key, step_keys, queue_chunk) -> None:
-    """batched_fit_steps with variances: one entry point (lfm_batched_fit_het) for the chunked and the queue launches."""
-    l = _lib.lib()
-    qb = 0
-    if queue_chunk > 0 and state.step == 0 and steps == state.total_steps:
-        qb = int(l.lfm_batched_queue_bytes(state.B, state.total_steps, int(queue_chunk)))
-        if qb > 0 and (state.queue_ws is None or state.queue_ws.numel() < qb):
-            state.queue_ws = torch.empty(qb, dtype=torch.uint8, device=X.device)
-    _lib.check(l.lfm_batched_fit_het(_stream(), state.B, X.shape[0], state.G, X.data_ptr(), y.data_ptr(), y_stride,
-                                     v.data_ptr(), v_stride, state.u.data_ptr(), state.adam.data_ptr(), float(jitter), lr,
-                                     b1, b2, eps, state.step, steps, state.total_steps, int(bool(fix_params)),
-                                     int(steps_per_epoch), state.unique_hint, int(state.time_grid), state.hist.data_ptr(),
-                                     state.hist.shape[1], state.theta.data_ptr(), state.info.data_ptr(),
-                                     best_key.data_ptr() if best_key is not None else None,
-                                     step_keys.data_ptr() if step_keys is not None else None,
-                                     state.struct_cache.data_ptr(), int(queue_chunk) if qb > 0 else 0,
-                                     state.queue_ws.data_ptr() if qb > 0 else None, qb),
-               "lfm_batched_fit_het")
+    whole = state.step == 0 and steps == state.total_steps
+    launch = _bind_fit(state, X, y, y_stride, v, v_stride, jitter, lr, b1, b2, eps, fix_params, steps_per_epoch,
+                       step_keys, queue_chunk if whole else 0)
+    launch(_stream(), state.step, steps, best_key.data_ptr() if best_key is not None else None)
     state.step += steps
 
 

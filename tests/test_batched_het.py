@@ -192,8 +192,8 @@ def test_batched_het_fit_matches_oracle(cuda, R, fix, team, monkeypatch):
 @pytest.mark.parametrize("team", [1, 4, 0])
 def test_batched_het_per_lfm_variances(cuda, team, monkeypatch):
     """One row of observations AND one row of variances per LFM (candidate gene sets with their own measurement errors):
-    evaluation and a 30-step fit against the oracle on each LFM's own data; multi_start_fit on the planned host-buffer
-    path and on device tensors equals batched_fit_steps."""
+    evaluation and a 30-step fit against the oracle on each LFM's own data; multi_start_fit on host arrays and on device
+    tensors equals batched_fit_steps."""
     import torch
     from dis_project_b200 import ops
     from dis_project_b200.batched import multi_start_fit
@@ -223,7 +223,7 @@ def test_batched_het_per_lfm_variances(cuda, team, monkeypatch):
         for inputs in ((x, Y, V), tuple(torch.as_tensor(a, device="cuda") for a in (x, Y, V))):
             res = multi_start_fit(inputs[0], inputs[1], TH, 1e-4, num_iters=30, chunk=10, variances=inputs[2])
             assert relerr(res.history, hist) < 1e-12 and res.best_id == int(np.argmin(hist[:, -1]))
-        # shared variances through the planned path: (N,) and (N, 1) are the same fit
+        # shared variances: (N,) and (N, 1) are the same fit
         r1 = multi_start_fit(x, Y, TH, 1e-4, num_iters=30, chunk=None, trace=True, variances=V[2])
         r2 = multi_start_fit(x, Y, TH, 1e-4, num_iters=30, chunk=None, trace=True, variances=V[2].reshape(-1, 1))
         assert np.array_equal(r1.history, r2.history)

@@ -175,23 +175,27 @@ def test_multi_start_per_step_trace(cuda):
         assert np.array_equal(res.best_trace, colmin)
         assert res.best_id == ref.best_id and res.best_loss == colmin[-1]
         assert np.array_equal(res.best_theta, res.theta[res.best_id])
-    # device-resident inputs take the other staging path
+    # device-resident inputs are copied into the same plan's device buffer: the same fit
     res2 = multi_start_fit(torch.as_tensor(x).cuda(), torch.as_tensor(y).cuda(), TH, 1e-4, num_iters=40, chunk=1, trace=True)
     assert np.array_equal(res2.history, res.history) and np.array_equal(res2.best_trace, res.best_trace)
 
 
-def test_multi_start_cached_plan_matches_the_uncached_path(cuda, monkeypatch):
-    """Host inputs go through a cached per-shape plan (staging buffers, state, pointers built once); the results are those
-    of the uncached path bit for bit, a second fit on the same plan with another X / y / start points is not polluted by
-    the first, and the arrays handed back stay valid after later fits (they are not views of a reused buffer)."""
+def test_multi_start_cached_plan_matches_a_fresh_plan(cuda):
+    """Every fit runs over a per-shape plan (staging buffers, state, pointers built once) that later fits of the same shape
+    reuse; the results on a reused plan are those on a freshly built one bit for bit, a second fit on the same plan with
+    another X / y / start points is not polluted by the first, and the arrays handed back stay valid after later fits
+    (they are not views of a reused buffer)."""
     from dis_project_b200 import batched
     from dis_project_b200.batched import make_restarts, multi_start_fit
     TH = make_restarts(o.Params.reference_init(5).pack(), 12)
     sets = [o.synthetic_problem(5, 7, 3, seed=s)[:2] for s in (6, 9)]
+
+    def fresh(*args, **kw):
+        batched._PLANS.clear()
+        return multi_start_fit(*args, **kw)
+
     for kw in ({"chunk": 7}, {"chunk": None, "trace": True}, {"chunk": 10, "trace": True}):
-        monkeypatch.setenv("LFM_MSF_PLAN", "0")
-        refs = [multi_start_fit(x, y, TH, 1e-4, num_iters=30, **kw) for x, y in sets]
-        monkeypatch.setenv("LFM_MSF_PLAN", "1")
+        refs = [fresh(x, y, TH, 1e-4, num_iters=30, **kw) for x, y in sets]
         batched._PLANS.clear()
         got = [multi_start_fit(x, y, TH, 1e-4, num_iters=30, **kw) for x, y in sets]
         got.append(multi_start_fit(sets[0][0], sets[0][1], TH[::-1].copy(), 1e-4, num_iters=30, **kw))
@@ -203,11 +207,82 @@ def test_multi_start_cached_plan_matches_the_uncached_path(cuda, monkeypatch):
         assert np.array_equal(got[2].history[::-1], got[0].history)   # same data set, start points reversed
     # per-LFM observations through the plan
     Y = np.stack([sets[0][1] + 0.01 * b for b in range(12)])
-    monkeypatch.setenv("LFM_MSF_PLAN", "0")
-    r = multi_start_fit(sets[0][0], Y, TH, 1e-4, num_iters=20, chunk=None, trace=True)
-    monkeypatch.setenv("LFM_MSF_PLAN", "1")
+    r = fresh(sets[0][0], Y, TH, 1e-4, num_iters=20, chunk=None, trace=True)
+    multi_start_fit(sets[1][0], Y[::-1].copy(), TH, 1e-4, num_iters=20, chunk=None, trace=True)
     g = multi_start_fit(sets[0][0], Y, TH, 1e-4, num_iters=20, chunk=None, trace=True)
     assert np.array_equal(r.history, g.history) and np.array_equal(r.theta, g.theta)
+
+
+_TWO_RANK_RUNS = [(B, name, kw) for B in (12, 1) for name, kw in (("chunk7", {"chunk": 7}),
+                                                                   ("trace", {"chunk": None, "trace": True}))]
+
+
+def _two_rank_inputs():
+    from dis_project_b200.batched import make_restarts
+    x, y, _, _ = o.synthetic_problem(5, 7, 3, seed=6)
+    return x, y, make_restarts(o.Params.reference_init(5).pack(), 12)
+
+
+def _two_rank_worker(rank, port, q):
+    """One rank of test_multi_start_two_ranks_on_one_device: every run of _TWO_RANK_RUNS in a gloo world of two."""
+    import traceback
+    import torch.distributed as dist
+    try:
+        from dis_project_b200.batched import multi_start_fit
+        torch.cuda.set_device(0)
+        dist.init_process_group("gloo", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=2)
+        try:
+            x, y, TH = _two_rank_inputs()
+            out = {}
+            for B, name, kw in _TWO_RANK_RUNS:
+                r = multi_start_fit(x, y, TH[:B], 1e-4, num_iters=40, **kw)
+                out[(B, name)] = (r.lo, r.hi, r.history, r.theta, r.best_id, r.best_loss, r.best_theta, r.best_trace)
+        finally:
+            dist.destroy_process_group()
+        q.put((rank, out))
+    except Exception:
+        q.put((rank, traceback.format_exc()))
+
+
+def test_multi_start_two_ranks_on_one_device(cuda):
+    """The multi-rank logic of multi_start_fit -- shards, the side-stream MIN all-reduce of the per-chunk keys, the gather
+    of every rank's winner with the per-step trace, and an empty shard (B = 1 over two ranks) -- in a gloo world of two
+    processes that share cuda:0.  Each rank's shard is the matching rows of a one-process fit (the team size may differ
+    with the shard size, hence a tolerance), and both ranks report that fit's winner and best-objective trace exactly."""
+    import socket
+    import torch.multiprocessing as tmp
+    from dis_project_b200.batched import multi_start_fit, shard_bounds
+    with socket.socket() as sk:
+        sk.bind(("127.0.0.1", 0))
+        port = sk.getsockname()[1]
+    ctx = tmp.get_context("spawn")
+    q = ctx.Queue()
+    procs = [ctx.Process(target=_two_rank_worker, args=(r, port, q)) for r in range(2)]
+    try:
+        for p in procs:
+            p.start()
+        got = dict(q.get(timeout=600) for _ in procs)
+        for p in procs:
+            p.join(timeout=120)
+            assert p.exitcode == 0
+    finally:
+        for p in procs:
+            if p.is_alive():
+                p.kill()
+                p.join()
+    for rank in (0, 1):
+        assert isinstance(got[rank], dict), got[rank]
+    x, y, TH = _two_rank_inputs()
+    for B, name, kw in _TWO_RANK_RUNS:
+        ref = multi_start_fit(x, y, TH[:B], 1e-4, num_iters=40, **kw)
+        for rank in (0, 1):
+            lo, hi, hist, theta, best_id, best_loss, best_theta, best_trace = got[rank][(B, name)]
+            assert (lo, hi) == shard_bounds(B, rank, 2), (B, name, rank)
+            assert hist.shape == (hi - lo, 40) and theta.shape == (hi - lo, 17)
+            if hi > lo:
+                assert relerr(hist, ref.history[lo:hi]) < 1e-11 and relerr(theta, ref.theta[lo:hi]) < 1e-10, (B, name, rank)
+            assert best_id == ref.best_id and best_loss == ref.best_loss, (B, name, rank)
+            assert np.array_equal(best_theta, ref.best_theta) and np.array_equal(best_trace, ref.best_trace), (B, name, rank)
 
 
 def test_examples_main_runs_the_reference_script(cuda, tmp_path):

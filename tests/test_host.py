@@ -145,8 +145,8 @@ def test_adam_and_gpx_compat():
     assert np.array_equal(gd.stddev(), [1, 2, 3]) and np.array_equal(gd.mean(), np.arange(3.0))
 
 
-def test_restart_generation_and_sharding():
-    from dis_project_b200.batched import make_restarts, pack_best, shard_bounds
+def test_restart_generation_sharding_and_winner_reduction():
+    from dis_project_b200.batched import make_restarts, reduce_best_gathered, shard_bounds
     from oracle import lfm_oracle as o
 
     th0 = o.Params.reference_init(5).pack()
@@ -159,9 +159,8 @@ def test_restart_generation_and_sharding():
         b = [shard_bounds(B, r, w) for r in range(w)]
         assert b[0][0] == 0 and b[-1][1] == B and all(b[i][1] == b[i + 1][0] for i in range(w - 1))
         assert max(h - l for l, h in b) - min(h - l for l, h in b) <= 1
-    assert np.array_equal(pack_best(np.array([3.0, np.nan, 1.5]), np.array([7, 8, 9])), [1.5, 9.0])
-    assert pack_best(np.array([]), np.array([]))[1] == -1
-    from dis_project_b200.batched import reduce_best_gathered
+    assert np.array_equal(reduce_best_gathered(np.array([[3.0, 7.0], [np.nan, 8.0], [1.5, 9.0]])), [1.5, 9.0])
+    assert reduce_best_gathered(np.zeros((0, 2)))[1] == -1                 # an empty shard never wins
     rows = np.array([[2.0, 5.0, 0.0], [1.5, 9.0, 0.0], [np.nan, 1.0, 0.0], [1.5, 3.0, 0.0]])
     assert np.array_equal(reduce_best_gathered(rows), [1.5, 3.0])
     assert reduce_best_gathered(np.array([[np.inf, -1.0]]))[1] == -1
@@ -169,19 +168,28 @@ def test_restart_generation_and_sharding():
 
 def _gloo_worker(rank, world, port, q):
     import torch.distributed as dist
-    from dis_project_b200.batched import pack_best, reduce_best, shard_bounds
+    from dis_project_b200.batched import reduce_best_gathered, shard_bounds
 
     dist.init_process_group("gloo", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=world)
     B = 11
     losses = np.array([5.0, 4.0, 9.0, 3.5, 8.0, 3.5, 7.0, 6.0, np.nan, 10.0, 12.0])
     lo, hi = shard_bounds(B, rank, world)
-    best = reduce_best(pack_best(losses[lo:hi], np.arange(lo, hi)), dist)
-    q.put((rank, lo, hi, float(best[0]), int(best[1])))
+    # the shard's packed winner [loss, id, theta...] (lfm_batched_best on the device; theta stands in as 100 + id)
+    ids = np.arange(lo, hi, dtype=np.float64)
+    mine = reduce_best_gathered(np.stack([losses[lo:hi], ids], axis=1))
+    row = torch.tensor([mine[0], mine[1], 100.0 + mine[1]], dtype=torch.float64)
+    rows = [torch.empty(3, dtype=torch.float64) for _ in range(world)]
+    dist.all_gather(rows, row)
+    allp = torch.stack(rows).numpy()
+    best = reduce_best_gathered(allp)
+    owner = int(np.flatnonzero((allp[:, 0] == best[0]) & (allp[:, 1] == best[1]))[0])
+    q.put((rank, lo, hi, float(best[0]), int(best[1]), float(allp[owner, 2])))
     dist.destroy_process_group()
 
 
-def test_best_objective_allreduce_gloo_world2():
-    """N > 1 host logic on CPU: contiguous shards + MIN all-reduce of (loss, restart id), ties -> lowest id."""
+def test_best_objective_gather_gloo_world2():
+    """N > 1 host logic on CPU: contiguous shards, every rank's packed winner gathered through gloo and reduced as
+    multi_start_fit does (MIN on the loss, ties -> lowest id, NaN never wins)."""
     import torch.multiprocessing as tmp
 
     ctx = tmp.get_context("spawn")
@@ -195,7 +203,40 @@ def test_best_objective_allreduce_gloo_world2():
         p.join(timeout=60)
         assert p.exitcode == 0
     assert [(r[1], r[2]) for r in res] == [(0, 6), (6, 11)]
-    assert all(r[3] == 3.5 and r[4] == 3 for r in res)
+    assert all(r[3] == 3.5 and r[4] == 3 and r[5] == 103.0 for r in res)
+
+
+def test_multi_start_fit_rejects_bad_shapes_before_any_device_work(monkeypatch):
+    """multi_start_fit checks the shapes of X, y, the variances and the start points on the host and raises ValueError
+    before it touches a device, for numpy arrays and torch tensors alike; a y of one value is not broadcast to every
+    observation."""
+    from dis_project_b200 import _lib, batched
+    from dis_project_b200.batched import multi_start_fit
+    from oracle import lfm_oracle as o
+
+    def no_device():
+        raise AssertionError("multi_start_fit reached the device with inputs it should have rejected")
+
+    monkeypatch.setattr(_lib, "require_device", no_device)
+    x, y, var, _ = o.synthetic_problem(5, 7, 3, seed=6)
+    B, N = 4, x.shape[0]
+    TH = np.tile(o.Params.reference_init(5).pack(), (B, 1))
+    plans = dict(batched._PLANS)
+    bad = [((x, np.array([2.5]), TH), {}),                        # one value for N = 105 observations
+           ((x, y[:-1], TH), {}),                                  # wrong length
+           ((x, np.tile(y, (B + 1, 1)), TH), {}),                  # (B + 1, N)
+           ((x[:, :2], y, TH), {}),                                # X not (N, 3)
+           ((x.reshape(-1), y, TH), {}),
+           ((x, y, TH), {"variances": var[:-1]}),                  # variances neither (N,), (N, 1) nor (B, N)
+           ((x, y, TH), {"variances": np.tile(var, (B + 1, 1))}),
+           ((x, y, TH[:, :-1]), {})]                               # start points not (B, 3G+2)
+    for args, kw in bad:
+        with pytest.raises(ValueError):
+            multi_start_fit(*args, 1e-4, num_iters=5, **kw)
+        with pytest.raises(ValueError):   # the same shapes as CPU tensors
+            multi_start_fit(*(torch.as_tensor(a) for a in args[:2]), args[2], 1e-4, num_iters=5,
+                            **{k: torch.as_tensor(v) for k, v in kw.items()})
+    assert batched._PLANS == plans
 
 
 def test_count_distinct_times():
