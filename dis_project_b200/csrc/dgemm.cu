@@ -7,23 +7,18 @@
 // in both operand orientations.  Per-tile k-ranges (kmode) let the same kernel serve every
 // triangular Level-3 shape of the blocked Cholesky / inverse (SYRK, TRMM, LAUUM, TRSM via
 // inverted diagonal blocks) without multiplying structural zeros at tile granularity.
-#include <cstdlib>
 #include <cstring>
 #include "lfm_common.cuh"
 
 #define BK 16
 #define STAGES 4
-// k4-steps of a unit (of 8) over which the next unit's cp.async are issued in the SPREAD instantiations.  Spreading
-// them over all 8 steps issued the last eighth one k4-step (~300 cycles) before the barrier that needs it -- less than
-// an L2 round trip, so every unit boundary stalled on its latest loads; over the first 4 steps every load has at least
-// half a unit to land.  Measured on B200 (N = 4000 evaluation, ms per step): 8 steps 3.40, 6: 3.35, 5: 3.33, 4: 3.33,
-// 3: 3.34, 2: 3.34, one burst behind the barrier (no SPREAD) 3.50; largest rank-128 update 23.7 -> 24.6 TF/s.
-#ifndef SPREAD_STEPS
+// k4-steps of a unit (of 8) over which the next unit's cp.async are issued.  Spreading them over all 8 steps issued the
+// last eighth one k4-step (~300 cycles) before the barrier that needs it -- less than an L2 round trip, so every unit
+// boundary stalled on its latest loads; over the first 4 steps every load has at least half a unit to land.  Measured on
+// B200 (N = 4000 evaluation, ms per step): 8 steps 3.40, 6: 3.35, 5: 3.33, 4: 3.33, 3: 3.34, 2: 3.34, one burst behind
+// the barrier 3.50; largest rank-128 update 23.7 -> 24.6 TF/s.  Over 4 steps spreading also beats one burst at large K:
+// plain 8192^3 product 32.4 -> 34.8 TF/s = 0.98 of cuBLAS Dgemm, N = 32768 evaluation 1.116 -> 1.056 s.
 #define SPREAD_STEPS 4
-#endif
-#ifndef LFM_GEMM_WS_DEFAULT
-#define LFM_GEMM_WS_DEFAULT 0
-#endif
 #define LDK (BK + 4)    // [row][k] layout: 20 doubles per row, == 4 (mod 16) -> conflict-free fragment reads
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
@@ -64,7 +59,7 @@ __device__ __forceinline__ void load_tile(double* s, const double* __restrict__ 
 //   <8,4,2> 128 x 128, 8 warps     <4,4,4> 128 x 128, 16 warps (4 per scheduler: better DMMA/LDS overlap)
 //   <4,4,2> 64 x 128 (in-place panel)       <4,2,2> 64 x 64 (small problems, 2 CTAs / SM)
 //   <1,4,2> 16 x 128 (one 128-row panel spread over 8 CTAs: the look-ahead chain of the factorisation)
-template <int TA, int TBN, int WM, int WN, int GM, bool SPREAD>  // TA: op(A)=A^T ; TBN = 1: B stored N x K ("NT"), 0: K x N
+template <int TA, int TBN, int WM, int WN, int GM>  // TA: op(A)=A^T ; TBN = 1: B stored N x K ("NT"), 0: K x N
 __global__ void __launch_bounds__(128 * GM, (WM * WN * GM <= 16) ? 2 : 1) lfm_dgemm_kernel(LfmGemm g, int tiles_n) {
   constexpr int BM = 8 * WM * GM, BN = 32 * WN, NT = 128 * GM;
   constexpr int A_STAGE = BM * LDK, B_STAGE = BN * LDK;  // >= 16 * (BM + 4), 16 * (BN + 4)
@@ -134,9 +129,8 @@ __global__ void __launch_bounds__(128 * GM, (WM * WN * GM <= 16) ? 2 : 1) lfm_dg
 
   // Two k-tiles (32 deep) per barrier: the four stages form two units; unit u is computed while unit u+1 streams
   // in, so there is one wait_group + one __syncthreads per 256 DMMAs of every warp.  The cp.async of unit u+1 are
-  // issued from per-thread pointers computed once; with SPREAD (short and medium K, where unit boundaries are a
-  // visible share of a tile) not in one burst behind the barrier but in PIECES after each of the first SPREAD_STEPS
-  // k4-steps of unit u.
+  // issued from per-thread pointers computed once, not in one burst behind the barrier but in PIECES after each of the
+  // first SPREAD_STEPS k4-steps of unit u.
   constexpr int PA = (BM * 8 + NT - 1) / NT;   // 16-byte chunks per thread and k-tile, operand A
   constexpr int PB = (BN * 8 + NT - 1) / NT;   //                                         operand B
   constexpr int PP = 2 * (PA + PB);            // chunks per thread and unit
@@ -209,7 +203,7 @@ __global__ void __launch_bounds__(128 * GM, (WM * WN * GM <= 16) ? 2 : 1) lfm_dg
     // the unit's (up to) 8 k4-steps with explicitly double-buffered fragments: the LDS of step s+1
     // are issued before the 32 DMMAs of step s
     const int nsteps = (2 * u + 1 < nk) ? 8 : 4;
-    const bool spread = SPREAD && nsteps == 8;
+    const bool spread = nsteps == 8;
     if (!spread) issue_unit((u + 1) & 1, 2 * (u + 1));
     const double* a_u = sA + ((u & 1) * 2) * A_STAGE;
     const double* b_u = sB + ((u & 1) * 2) * B_STAGE;
@@ -240,7 +234,6 @@ __global__ void __launch_bounds__(128 * GM, (WM * WN * GM <= 16) ? 2 : 1) lfm_dg
           for (int j = 0; j < WN; ++j) dmma884(acc[i][j][0], acc[i][j][1], af[step & 1][i], bf[step & 1][j]);
         if (spread) {
           // this step's share of the next unit's loads (slot (u+1)&1 was last read before this iteration's barrier)
-#pragma unroll
           if (step < SPREAD_STEPS) {
 #pragma unroll
             for (int q = step * PP / SPREAD_STEPS; q < (step + 1) * PP / SPREAD_STEPS; ++q) issue_piece((u + 1) & 1, 2 * (u + 1), q);
@@ -254,278 +247,6 @@ __global__ void __launch_bounds__(128 * GM, (WM * WN * GM <= 16) ? 2 : 1) lfm_dg
   if (stamp) stamp[3] = clock64();
 
   // epilogue: thread holds C[row = 8i + lane/4][col = 8j + 2*(lane%4) + {0,1}]
-  const double alpha = g.alpha, beta = g.beta;
-#pragma unroll
-  for (int i = 0; i < WM; ++i) {
-    const int64_t r = row0 + wm + i * 8 + fr;
-#pragma unroll
-    for (int j = 0; j < WN; ++j) {
-      const int64_t c = col0 + wn + j * 8 + fc * 2;
-      double2* p = reinterpret_cast<double2*>(gC + r * g.ldc + c);
-      double2 o;
-      if (c_in_acc) {
-        o.x = flip(acc[i][j][0]);
-        o.y = flip(acc[i][j][1]);
-      } else {
-        o.x = alpha * acc[i][j][0];
-        o.y = alpha * acc[i][j][1];
-      }
-      if (c_mode != 0 && !c_in_acc) {
-        const double2 old = *p;
-        o.x += beta * old.x;
-        o.y += beta * old.y;
-      }
-      *p = o;
-    }
-  }
-  if (stamp) {
-    long long gt;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-    stamp[4] = clock64(); stamp[6] = gt;
-  }
-}
-
-// ---- warp-specialised variant (opt-in, LFM_GEMM_WS = 1 / 2): cp.async.bulk (TMA unit, SASS UBLKCP) + per-stage mbarriers ------
-// The kernel above stops ALL its warps at one __syncthreads per 32-deep unit; `tools/tile_life.py` had a CTA alone on its SM
-// run its mainloop at 81-84 % of the DMMA pipe, and two co-resident CTAs of the same launch reach their barriers together.
-// Here producer warps (two: one per operand) stage the operands -- one bulk copy per operand row (256 B of a [row][k] operand,
-// BM * 8 B of a [k][row] operand) into the same padded, conflict-free layouts, completion counted in bytes on the stage's FULL
-// mbarrier; or, LDG = true, 16-byte cp.async with cp.async.mbarrier.arrive -- and the consumer warps never meet: each waits for
-// FULL[s], runs its 8 k4-steps, and arrives on EMPTY[s]; the producers refill a stage when all consumer warps have left it.
-// Three stages of 32 k: two units (64 k) in flight per CTA.  MEASURED SLOWER than the kernel above and therefore off by default
-// (profiles/gemm_ws_tma_r2c.md: a row-granular bulk copy costs its warp 70-80 cycles, and the barrier was not the bound).
-#define WS_BK 32
-#define WS_LDK (WS_BK + 4)   // 36 doubles = 72 banks == 8 (mod 32): the 4 rows of a half-warp's LDS.64 hit disjoint banks
-#define WS_STAGES 3
-#define WS_BAR_BYTES 128
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  do {
-    asm volatile(
-        "{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  } while (!ok);
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(dst), "l"(src),
-               "r"(bytes), "r"(bar)
-               : "memory");
-}
-
-// NPW producer warps: 1 (both operands) or 2 (A | B).  LDG: the producers stage with per-thread 16-byte cp.async (LDGSTS) whose completion
-// is counted on the FULL barrier by cp.async.mbarrier.arrive.noinc, instead of bulk copies.
-template <int TA, int TBN, int WM, int WN, int GM, int NPW, bool LDG>
-__global__ void __launch_bounds__(128 * GM + 32 * NPW, (WM * WN * GM <= 16) ? 2 : 1) lfm_dgemm_ws_kernel(LfmGemm g, int tiles_n) {
-  constexpr int BM = 8 * WM * GM, BN = 32 * WN, NCW = 4 * GM;
-  constexpr int A_STAGE = TA ? WS_BK * (BM + 4) : BM * WS_LDK;    // doubles
-  constexpr int B_STAGE = TBN ? BN * WS_LDK : WS_BK * (BN + 4);
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  double* sA = reinterpret_cast<double*>(smem_raw + WS_BAR_BYTES);
-  double* sB = sA + WS_STAGES * A_STAGE;
-  const uint32_t bar0 = smem_u32(smem_raw);   // FULL[s] at bar0 + 8 s, EMPTY[s] at bar0 + 8 (WS_STAGES + s)
-  const int tid = threadIdx.x;
-  const int lane = tid & 31;
-  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);   // a broadcast: ptxas treats the warp index (and the role branch) as uniform
-  long long* const stamp = (g.stamps && tid == 0) ? g.stamps + 8 * (int64_t)blockIdx.x : nullptr;
-  if (stamp) {
-    unsigned smid; long long gt;
-    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-    stamp[0] = smid; stamp[1] = clock64(); stamp[5] = gt;
-  }
-  if (tid == 0) {
-#pragma unroll
-    for (int s = 0; s < WS_STAGES; ++s) {
-      mbar_init(bar0 + 8 * s, LDG ? 32 * NPW : NPW);
-      mbar_init(bar0 + 8 * (WS_STAGES + s), NCW);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
-  }
-  int tm, tn;
-  if (g.lower_only) {
-    const int64_t srows = g.tri_skip / BM;
-    const int64_t skipped = srows * (srows + 1) / 2;
-    const int64_t total = (int64_t)gridDim.x;
-    const bool asc = (g.kmode == LFM_K_GE_ROW || g.kmode == LFM_K_GE_ROWCOL || g.kmode == LFM_K_LAUUM_LATE);
-    const int64_t t = skipped + (asc ? (int64_t)blockIdx.x : total - 1 - (int64_t)blockIdx.x);
-    int64_t i = (int64_t)((sqrtf(8.0f * (float)t + 1.0f) - 1.0f) * 0.5f);
-    while ((i + 1) * (i + 2) / 2 <= t) ++i;
-    while (i * (i + 1) / 2 > t) --i;
-    tm = (int)i;
-    tn = (int)(t - i * (i + 1) / 2);
-  } else {
-    tm = blockIdx.x / tiles_n;
-    tn = blockIdx.x % tiles_n;
-  }
-  const int64_t row0 = (int64_t)tm * BM, col0 = (int64_t)tn * BN;
-  const double* __restrict__ gA = g.A + (int64_t)blockIdx.y * g.strideA;
-  const double* __restrict__ gB = g.B + (int64_t)blockIdx.y * g.strideB;
-  double* __restrict__ gC = g.C + (int64_t)blockIdx.y * g.strideC;
-  int64_t kb = 0, ke = g.K;
-  switch (g.kmode) {
-    case LFM_K_LE_ROW: ke = min(g.K, row0 + BM); break;
-    case LFM_K_GE_COL: kb = col0; break;
-    case LFM_K_GE_ROW: kb = row0; break;
-    case LFM_K_GE_ROWCOL: kb = max(row0, col0); break;
-    case LFM_K_LAUUM_LATE: kb = row0 < g.k_split ? g.k_split : max(row0, col0); break;
-    default: break;
-  }
-  const int c_mode = g.kmode == LFM_K_LAUUM_LATE ? (row0 < g.k_split ? 2 : 0) : g.c_mode;
-  kb = max(kb, g.k_lo);
-  ke = min(ke, g.k_hi);
-  const int nk = ke > kb ? (int)((ke - kb) / BK) : 0;   // 16-deep k-tiles; a unit is two of them (the last one may be one)
-  if (nk == 0 && c_mode >= 2) return;
-  const int nu = (nk + 1) >> 1;
-  __syncthreads();   // barriers initialised; the only CTA-wide barrier of the kernel
-
-  if (warp >= NCW) {
-    // ---- producer warp(s): lane l copies operand rows l, l + 32, ... of every unit
-    const bool doA = NPW == 1 || warp == NCW, doB = NPW == 1 || warp != NCW;
-    int s = 0;
-    uint32_t ph = 1;   // parity the EMPTY barrier of a stage must have completed: a fresh barrier passes parity 1
-    for (int u = 0; u < nu; ++u) {
-      const int kw = (2 * u + 1 < nk) ? WS_BK : BK;
-      const uint32_t full = bar0 + 8 * s;
-      mbar_wait(bar0 + 8 * (WS_STAGES + s), ph);
-      if (LDG) {
-        const int64_t k0 = kb + (int64_t)u * WS_BK;
-        const int p = (warp - NCW) * 32 + lane;        // producer thread
-        double* a_st = sA + s * A_STAGE;
-        double* b_st = sB + s * B_STAGE;
-        // [row][k] operand: 16 chunks of 16 bytes per row and unit; [k][row] operand: rows / 2 chunks per k-row
-#pragma unroll 4
-        for (int id = p; id < BM * 16; id += 32 * NPW) {
-          if (TA == 0) {
-            const int r = id >> 4, kc = id & 15;
-            if (kc * 2 < kw) cp_async16(a_st + r * WS_LDK + kc * 2, gA + (row0 + r) * g.lda + k0 + kc * 2);
-          } else {
-            const int kr = id / (BM / 2), mc = id % (BM / 2);
-            if (kr < kw) cp_async16(a_st + kr * (BM + 4) + mc * 2, gA + (k0 + kr) * g.lda + row0 + mc * 2);
-          }
-        }
-#pragma unroll 4
-        for (int id = p; id < BN * 16; id += 32 * NPW) {
-          if (TBN) {
-            const int r = id >> 4, kc = id & 15;
-            if (kc * 2 < kw) cp_async16(b_st + r * WS_LDK + kc * 2, gB + (col0 + r) * g.ldb + k0 + kc * 2);
-          } else {
-            const int kr = id / (BN / 2), mc = id % (BN / 2);
-            if (kr < kw) cp_async16(b_st + kr * (BN + 4) + mc * 2, gB + (k0 + kr) * g.ldb + col0 + mc * 2);
-          }
-        }
-        asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];\n" ::"r"(full) : "memory");
-      } else {
-        if (lane == 0) mbar_expect_tx(full, (uint32_t)(((doA ? BM : 0) + (doB ? BN : 0)) * kw * 8));
-        __syncwarp();
-        const int64_t k0 = kb + (int64_t)u * WS_BK;
-        const uint32_t a_s = smem_u32(sA + s * A_STAGE), b_s = smem_u32(sB + s * B_STAGE);
-        // one elected lane issues every copy of the unit from warp-uniform addresses: UBLKCP takes uniform registers, and a
-        // copy per LANE is serialised by ptxas into an ELECT / 5 x R2UR / UBLKCP loop that costs ~80 cycles per copy (measured:
-        // 64 copies per warp and unit = 5.4 k cycles, more than the unit's DMMAs take)
-        if (doA) {
-          const double* src = TA == 0 ? gA + row0 * g.lda + k0 : gA + k0 * g.lda + row0;
-          const int n = TA == 0 ? BM : kw;
-          const uint32_t bytes = TA == 0 ? kw * 8 : BM * 8, pitch = TA == 0 ? WS_LDK * 8 : (BM + 4) * 8;
-          if (lane == 0) {
-#pragma unroll 4
-            for (int r = 0; r < n; ++r) bulk_g2s(a_s + r * pitch, src + r * g.lda, bytes, full);
-          }
-        }
-        if (doB) {
-          const double* src = TBN ? gB + col0 * g.ldb + k0 : gB + k0 * g.ldb + col0;
-          const int n = TBN ? BN : kw;
-          const uint32_t bytes = TBN ? kw * 8 : BN * 8, pitch = TBN ? WS_LDK * 8 : (BN + 4) * 8;
-          if (lane == 0) {
-#pragma unroll 4
-            for (int r = 0; r < n; ++r) bulk_g2s(b_s + r * pitch, src + r * g.ldb, bytes, full);
-          }
-        }
-      }
-      if (++s == WS_STAGES) { s = 0; ph ^= 1; }
-    }
-    if (LDG) cp_async_wait<0>();   // (the thread's copies are tracked by its own scoreboard: land them before it exits)
-    return;
-  }
-
-  // ---- consumer warps
-  double acc[WM][WN][2];
-#pragma unroll
-  for (int i = 0; i < WM; ++i)
-#pragma unroll
-    for (int j = 0; j < WN; ++j) { acc[i][j][0] = 0.0; acc[i][j][1] = 0.0; }
-  const int wm = (warp >> 2) * (8 * WM);
-  const int wn = (warp & 3) * (8 * WN);
-  const int fr = lane >> 2, fc = lane & 3;
-  if (stamp) stamp[7] = clock64();
-  const bool c_in_acc = c_mode >= 2 && nk > 0;
-  const int sgn = c_mode == 3 ? (int)0x80000000 : 0;
-  auto flip = [&](double x) { return __hiloint2double(__double2hiint(x) ^ sgn, __double2loint(x)); };
-  if (c_in_acc) {
-#pragma unroll
-    for (int i = 0; i < WM; ++i) {
-      const int64_t r = row0 + wm + i * 8 + fr;
-#pragma unroll
-      for (int j = 0; j < WN; ++j) {
-        const int64_t c = col0 + wn + j * 8 + fc * 2;
-        const double2 old = __ldcg(reinterpret_cast<const double2*>(gC + r * g.ldc + c));
-        acc[i][j][0] = flip(old.x);
-        acc[i][j][1] = flip(old.y);
-      }
-    }
-  }
-  // per-thread fragment bases inside a stage (doubles)
-  const int a_off = TA ? (fc * (BM + 4) + wm + fr) : ((wm + fr) * WS_LDK + fc);
-  const int b_off = TBN ? ((wn + fr) * WS_LDK + fc) : (fc * (BN + 4) + wn + fr);
-  constexpr int A_I = TA ? 8 : 8 * WS_LDK, A_K4 = TA ? 4 * (BM + 4) : 4;   // stride of fragment i / of a k4-step
-  constexpr int B_J = TBN ? 8 * WS_LDK : 8, B_K4 = TBN ? 4 : 4 * (BN + 4);
-  {
-    int s = 0;
-    uint32_t ph = 0;
-    for (int u = 0; u < nu; ++u) {
-      mbar_wait(bar0 + 8 * s, ph);
-      if (stamp && u == 0) stamp[2] = clock64();
-      const int nsteps = (2 * u + 1 < nk) ? 8 : 4;
-      const double* a_u = sA + s * A_STAGE + a_off;
-      const double* b_u = sB + s * B_STAGE + b_off;
-      double af[2][WM], bf[2][WN];
-      auto load_frags = [&](int buf, int step) {
-#pragma unroll
-        for (int i = 0; i < WM; ++i) af[buf][i] = a_u[step * A_K4 + i * A_I];
-#pragma unroll
-        for (int j = 0; j < WN; ++j) bf[buf][j] = b_u[step * B_K4 + j * B_J];
-      };
-      load_frags(0, 0);
-#pragma unroll
-      for (int step = 0; step < 8; ++step) {
-        if (step < nsteps) {
-          if (step + 1 < nsteps) load_frags((step + 1) & 1, step + 1);
-#pragma unroll
-          for (int i = 0; i < WM; ++i)
-#pragma unroll
-            for (int j = 0; j < WN; ++j) dmma884(acc[i][j][0], acc[i][j][1], af[step & 1][i], bf[step & 1][j]);
-        }
-      }
-      // every lane's last fragment of the stage is in registers (its DMMAs were issued): hand the stage back
-      __syncwarp();
-      if (lane == 0) mbar_arrive(bar0 + 8 * (WS_STAGES + s));
-      if (++s == WS_STAGES) { s = 0; ph ^= 1; }
-    }
-  }
-  if (stamp) stamp[3] = clock64();
-
   const double alpha = g.alpha, beta = g.beta;
 #pragma unroll
   for (int i = 0; i < WM; ++i) {
@@ -641,8 +362,8 @@ extern "C" int lfm_debug_profile_end(double* total_ms, double* exec_flops, long 
     char buf[256];
     for (const auto& kv : per) {
       const int v = kv.first;
-      snprintf(buf, sizeof buf, "%s{\"variant\": \"lfm_dgemm%s_kernel<%d,%d,%d,%d,%d>\", \"tile\": \"%dx%d\", \"launches\": %lld, "
-               "\"ms_sum\": %.6f, \"executed_flops\": %.6e}", js.size() > 1 ? ", " : "", v / 100000 ? "_ws" : "", v / 10000 % 10, v / 1000 % 10, v / 100 % 10,
+      snprintf(buf, sizeof buf, "%s{\"variant\": \"lfm_dgemm_kernel<%d,%d,%d,%d,%d>\", \"tile\": \"%dx%d\", \"launches\": %lld, "
+               "\"ms_sum\": %.6f, \"executed_flops\": %.6e}", js.size() > 1 ? ", " : "", v / 10000 % 10, v / 1000 % 10, v / 100 % 10,
                v / 10 % 10, v % 10, 8 * (v / 100 % 10) * (v % 10), 32 * (v / 10 % 10), kv.second.second.second, kv.second.first,
                kv.second.second.first);
       js += buf;
@@ -691,15 +412,11 @@ static cudaEvent_t prof_event() {
   return g_prof.ev[g_prof.used++];
 }
 
-template <int TA, int TBN, int WM, int WN, int GM, bool SPREAD, int WS = 0>   // WS: 1 / 2: warp-specialised kernel, bulk-copy / cp.async producers
+template <int TA, int TBN, int WM, int WN, int GM>
 static int launch(cudaStream_t st, const LfmGemm& g) {
   constexpr int BM = 8 * WM * GM, BN = 32 * WN;
-  constexpr int WS_A = TA ? WS_BK * (BM + 4) : BM * WS_LDK, WS_B = TBN ? BN * WS_LDK : WS_BK * (BN + 4);
-  constexpr int SMEM = WS ? WS_BAR_BYTES + WS_STAGES * (WS_A + WS_B) * 8 : STAGES * (BM + BN) * LDK * 8;
-  auto* const kernel = [] {
-    if constexpr (WS > 0) return &lfm_dgemm_ws_kernel<TA, TBN, WM, WN, GM, 2, WS == 2>;
-    else return &lfm_dgemm_kernel<TA, TBN, WM, WN, GM, SPREAD>;
-  }();
+  constexpr int SMEM = STAGES * (BM + BN) * LDK * 8;
+  auto* const kernel = &lfm_dgemm_kernel<TA, TBN, WM, WN, GM>;
   static LfmSmemConfig smem_cfg;
   {
     // Every tile variant asks for the LARGEST shared-memory carveout, whatever its own footprint: CTAs of two variants
@@ -711,8 +428,7 @@ static int launch(cudaStream_t st, const LfmGemm& g) {
     if (dev < 0 || smem_cfg.bytes[dev].load(std::memory_order_acquire) < (size_t)SMEM)
       LFM_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   }
-  const size_t smem_total = (size_t)SMEM + (size_t)(g.smem_pad > 0 ? g.smem_pad : 0);
-  LFM_CUDA_OK(lfm_ensure_smem(kernel, smem_cfg, smem_total));
+  LFM_CUDA_OK(lfm_ensure_smem(kernel, smem_cfg, SMEM));
   const int64_t tm = g.M / BM, tn = g.N / BN;
   int64_t tiles = g.lower_only ? tm * (tm + 1) / 2 : tm * tn;
   if (g.lower_only && g.tri_skip > 0) {
@@ -732,7 +448,7 @@ static int launch(cudaStream_t st, const LfmGemm& g) {
     const double f = gemm_exec_flops(g, BM, BN) * (g.batch > 1 ? g.batch : 1);
     const bool chain = BM == 16;
     g_prof.is_chain.push_back(chain ? 1 : 0);
-    g_prof.variant.push_back(WS * 100000 + TA * 10000 + TBN * 1000 + WM * 100 + WN * 10 + GM);
+    g_prof.variant.push_back(TA * 10000 + TBN * 1000 + WM * 100 + WN * 10 + GM);
     g_prof.pair_flops.push_back(f);
     if (chain) { g_prof.chain_flops += f; g_prof.chain_launches += 1; }
     else { g_prof.flops += f; g_prof.launches += 1; }
@@ -743,7 +459,7 @@ static int launch(cudaStream_t st, const LfmGemm& g) {
     // kernel nodes otherwise run without one, and the panel stream's CTAs queued behind every pending CTA of a trailing
     // update instead of taking the next free slot (CUPTI timelines, eager vs graph, round 2).
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = dim3(128 * GM + (WS ? 64 : 0)); cfg.dynamicSmemBytes = smem_total; cfg.stream = st;
+    cfg.gridDim = grid; cfg.blockDim = dim3(128 * GM); cfg.dynamicSmemBytes = SMEM; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     int prio = 0;
     unsigned nattr = 0;
@@ -763,48 +479,12 @@ static int launch(cudaStream_t st, const LfmGemm& g) {
   return LFM_OK;
 }
 
-template <int WM, int WN, int GM, bool SPREAD>
-static int dispatch2(cudaStream_t st, const LfmGemm& g) {
-  if (g.transA == 0 && g.transB == 1) return launch<0, 1, WM, WN, GM, SPREAD>(st, g);
-  if (g.transA == 0 && g.transB == 0) return launch<0, 0, WM, WN, GM, SPREAD>(st, g);
-  if (g.transA == 1 && g.transB == 0) return launch<1, 0, WM, WN, GM, SPREAD>(st, g);
-  return launch<1, 1, WM, WN, GM, SPREAD>(st, g);
-}
-static int64_t spread_max_k() {
-  static int64_t v = -1;
-  // (with the loads of a unit spread over all 8 of its k4-steps, spreading lost to one burst for K >= 8192 and the switch
-  // sat at 4096; over the first SPREAD_STEPS = 4 steps it wins at every K: plain 8192^3 product 32.4 -> 34.8 TF/s = 0.98 of
-  // cuBLAS Dgemm, N = 32768 evaluation 1.116 -> 1.056 s.  LFM_GEMM_SPREAD_K = K above which one burst is used instead.)
-  if (v < 0) { const char* e = getenv("LFM_GEMM_SPREAD_K"); v = e ? atoll(e) : ((int64_t)1 << 62); }
-  return v;
-}
-// LFM_GEMM_WS: bit 0: the 64 x 64 tiles run the warp-specialised kernel (cp.async.bulk + mbarrier pipeline) instead of the
-// cp.async kernel.  (The 16-warp 128 x 128 tile has no room for a 17th warp: five warps on one scheduler cap a thread at
-// 96 registers and ptxas spills the accumulators.)
-static int ws_mask() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("LFM_GEMM_WS"); v = e ? atoi(e) : LFM_GEMM_WS_DEFAULT; }
-  return v;
-}
-template <int WM, int WN, int GM, int WS>
-static int dispatch_ws(cudaStream_t st, const LfmGemm& g) {
-  if (g.transA == 0 && g.transB == 1) return launch<0, 1, WM, WN, GM, true, WS>(st, g);
-  if (g.transA == 0 && g.transB == 0) return launch<0, 0, WM, WN, GM, true, WS>(st, g);
-  if (g.transA == 1 && g.transB == 0) return launch<1, 0, WM, WN, GM, true, WS>(st, g);
-  return launch<1, 1, WM, WN, GM, true, WS>(st, g);
-}
 template <int WM, int WN, int GM>
 static int dispatch(cudaStream_t st, const LfmGemm& g) {
-  if constexpr (WM == 4 && WN == 2 && GM == 2) {
-    if (ws_mask() == 1) return dispatch_ws<WM, WN, GM, 1>(st, g);
-    if (ws_mask() == 2) return dispatch_ws<WM, WN, GM, 2>(st, g);
-  }
-  return g.K <= spread_max_k() ? dispatch2<WM, WN, GM, true>(st, g) : dispatch2<WM, WN, GM, false>(st, g);
-}
-static int big_variant() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("LFM_GEMM_BIG"); v = e ? atoi(e) : 1; }
-  return v;
+  if (g.transA == 0 && g.transB == 1) return launch<0, 1, WM, WN, GM>(st, g);
+  if (g.transA == 0 && g.transB == 0) return launch<0, 0, WM, WN, GM>(st, g);
+  if (g.transA == 1 && g.transB == 0) return launch<1, 0, WM, WN, GM>(st, g);
+  return launch<1, 1, WM, WN, GM>(st, g);
 }
 
 // Tile-shape heuristic: 128 x 128 tiles once they fill >= 3 waves of the 148 SMs, else 64 x 64 tiles
@@ -828,12 +508,7 @@ int lfm_dgemm(cudaStream_t st, const LfmGemm& g) {
     if (t128 >= 148) return dispatch<8, 4, 2>(st, g);
     return (g.M / 64 >= 148) ? dispatch<4, 4, 2>(st, g) : dispatch<2, 4, 2>(st, g);  // 64- or 32-row tiles: fill the SMs
   }
-  static int force = -1;
-  if (force < 0) { const char* e = getenv("LFM_GEMM_FORCE"); force = e ? atoi(e) : 0; }
-  if (force == 1) return dispatch<4, 4, 4>(st, g);
-  if (force == 2) return dispatch<8, 4, 2>(st, g);
-  if (force == 3) return dispatch<4, 2, 2>(st, g);
   if (g.tri_skip > 0) return dispatch<4, 2, 2>(st, g);  // rank-128 trailing updates: 64 x 64 tiles measured fastest
-  if (t128 >= 3 * 148) return big_variant() ? dispatch<4, 4, 4>(st, g) : dispatch<8, 4, 2>(st, g);
+  if (t128 >= 3 * 148) return dispatch<4, 4, 4>(st, g);
   return dispatch<4, 2, 2>(st, g);
 }

@@ -157,12 +157,7 @@ int lfm_launch_sigma_lower(cudaStream_t st, int64_t N, int64_t Npad, const doubl
 // Column tiles per work item: few enough that the launch fills both CTA slots of every SM for more than one wave
 // (N = 4000: 63 row tiles -> 1040 work items of <= 2 tiles instead of 156 of <= 16 on 296 slots; measured 3.83 -> 3.65 ms per evaluation), many for large N where
 // the row partials (one N64 x 2 slab per chunk) would otherwise dominate the scratch.
-static int lfm_gc_tiles(int64_t ntile) {
-  static int forced = -1;
-  if (forced < 0) { const char* e = getenv("LFM_GC_TILES"); forced = e ? atoi(e) : 0; }
-  if (forced > 0) return forced;
-  return ntile <= 128 ? 2 : 16;
-}
+static int lfm_gc_tiles(int64_t ntile) { return ntile <= 128 ? 2 : 16; }
 
 template <bool TAB>
 __global__ void __launch_bounds__(256, TAB ? LFM_GC_MINB : 1) lfm_grad_contract_kernel(int64_t N, const double* __restrict__ X, int G,

@@ -101,7 +101,6 @@ struct LfmGemm {
                        // with the co-resident CTA's DMMAs): 0: beta == 0; 1: general beta; 2 / 3: beta == 1 and alpha == +1 / -1 (C starts in the accumulators, signs by integer XOR)
   long long* stamps = nullptr;   // debug (lfm_debug_syrk_stamps, include/lfm_b200.h): 8 words per CTA -- SM id, clock64 at entry / first unit
                                  // landed / last DMMA issued / stores issued, globaltimer at entry and exit, clock64 when the addresses are set up
-  int smem_pad = 0;    // extra dynamic shared memory (bytes) the launch asks for and never touches: caps the CTAs of this launch per SM
   int64_t k_lo = 0, k_hi = ((int64_t)1 << 62);   // k-window: a tile's k-range (after kmode) is clipped to [k_lo, k_hi), multiples of 16;
                        // with beta == 1 a tile whose clipped range is empty is left untouched (K-chunked accumulation)
 };

@@ -301,9 +301,7 @@ static int nlml_factor(cudaStream_t st, int64_t N, int G, const double* X, const
   // Sigma is built in two launches -- its first two block columns (all the first leaf and the first chain step read),
   // then the rest -- and the dependent chain starts behind the first one: ~50 us of an N = 4000 evaluation in which the
   // chain partition used to wait for 8 N^2 bytes of Sigma it does not touch.
-  static int split = -1;
-  if (split < 0) { const char* e = getenv("LFM_SIGMA_SPLIT"); split = e ? atoi(e) : 1; }
-  if (grad && split && chain_ready && lfm_potrf_trtri_is_one_sweep(s.Np) && s.Np >= 8 * LFM_NB) {
+  if (grad && chain_ready && lfm_potrf_trtri_is_one_sweep(s.Np) && s.Np >= 8 * LFM_NB) {
     LFM_CUDA_OK(cudaMemsetAsync(info, 0, sizeof(int), st));
     LFM_TRY(lfm_launch_sigma_lower(st, N, s.Np, X, G, theta, variances, jitter, 1, s.A, s.Np, grid, 0, 2 * LFM_NB));
     LFM_CUDA_OK(cudaEventRecord(chain_ready, st));
@@ -494,8 +492,6 @@ extern "C" int lfm_debug_syrk_stamps(lfm_stream_t stream, int64_t m, int64_t K, 
   g.C = Cm; g.ldc = ldc; g.alpha = -1.0; g.beta = 1.0; g.lower_only = 1; g.kmode = LFM_K_FULL;
   g.batch = 1; g.strideA = g.strideB = g.strideC = 0;
   g.stamps = stamps;
-  if (getenv("LFM_DEBUG_SYRK_BETA0")) g.beta = 0.0;   // experiment: the same launch without the read of C
-  if (const char* e = getenv("LFM_DEBUG_SYRK_PAD")) g.smem_pad = atoi(e);   // experiment: 40960 = one CTA per SM
   return lfm_dgemm((cudaStream_t)stream, g);
 }
 extern "C" int lfm_debug_potrf_potri(lfm_stream_t stream, int64_t n, double* A, double* W, double* Sinv,

@@ -405,9 +405,7 @@ int lfm_debug_potrf_potri(lfm_stream_t stream, int64_t n, double* A, double* W, 
 int lfm_debug_syrk(lfm_stream_t stream, int64_t m, int64_t K, const double* P, int64_t ldp, double* C, int64_t ldc);
 /* The same launch with 8 debug words per CTA in `stamps` (tiles of the launch x 8 int64): [0] SM id, clock64 at [1] entry,
  * [2] first operand unit landed, [3] last DMMA issued, [4] stores issued, [7] address set-up done (nothing requested yet);
- * globaltimer at [5] entry and [6] exit (tools/tile_life.py).  LFM_DEBUG_SYRK_BETA0 in the environment: the same launch
- * with beta = 0, i.e. without the read of C; LFM_DEBUG_SYRK_PAD=<bytes> of untouched dynamic shared memory (40960: one CTA
- * per SM instead of two). */
+ * globaltimer at [5] entry and [6] exit (tools/tile_life.py). */
 int lfm_debug_syrk_stamps(lfm_stream_t stream, int64_t m, int64_t K, const double* P, int64_t ldp, double* C, int64_t ldc,
                           long long* stamps);
 

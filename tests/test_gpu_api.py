@@ -637,34 +637,6 @@ def test_sm_partition_is_a_scheduling_choice_only(cuda, tmp_path):
     assert np.array_equal(other, got)
 
 
-@pytest.mark.parametrize("ws", [1, 2])
-def test_warp_specialised_gemm_is_bit_identical(cuda, tmp_path, ws):
-    """LFM_GEMM_WS=1 / 2 (opt-in, csrc/dgemm.cu: lfm_dgemm_ws_kernel) runs every 64 x 64-tile GEMM launch -- trailing
-    updates, inverse products, all four operand orientations -- with producer warps and per-stage mbarriers instead of
-    cp.async groups and __syncthreads: 1 stages the operands with cp.async.bulk (one bulk copy per operand row, byte-counted
-    on the stage's mbarrier), 2 with cp.async + cp.async.mbarrier.arrive.  The DMMAs of a tile run over the same k in the
-    same order, so an N = 2048 evaluation in a child process must equal this process's bit for bit."""
-    import subprocess
-    import sys
-    from dis_project_b200 import ops
-    G, T = 32, 64
-    x, y, var, _ = o.synthetic_problem(G, T, 1, seed=62)
-    th = o.Params.reference_init(G).pack()
-    out, info = ops.nlml_grad(x, y, th, 1e-4, G)
-    assert int(info.item()) == 0
-    got = out.cpu().numpy()
-    np.savez(tmp_path / "in.npz", x=x, y=y, th=th)
-    code = ("import sys, numpy as np; sys.path.insert(0, %r); from dis_project_b200 import ops; "
-            "d = np.load(%r); out, info = ops.nlml_grad(d['x'], d['y'], d['th'], 1e-4, %d); "
-            "np.save(%r, out.cpu().numpy())"
-            % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), str(tmp_path / "in.npz"), G,
-               str(tmp_path / "out.npy")))
-    env = dict(os.environ, LFM_GEMM_WS=str(ws))
-    subprocess.run([sys.executable, "-c", code], check=True, env=env, timeout=300)
-    other = np.load(tmp_path / "out.npy")
-    assert np.array_equal(other, got)
-
-
 def test_configs_3_and_5_full_size_oracle_parity(cuda, tmp_path):
     """BASELINE configs 3 and 5 against the oracle at FULL size (N = 32768; 102 400 test times, the oracle on a sample of
     256 of them): 1e-9 relative, north_star's tolerance.  The oracle takes minutes of host time (about 2.5 on 16 cores,

@@ -1,5 +1,5 @@
-"""One rank-128 trailing update C -= P P^T (lower tiles, m = 3840, the 64 x 64-tile variant) after two warm-ups: target for
-`ncu --set full` (`LFM_GEMM_FORCE=3 ncu -k regex:lfm_dgemm_kernel -s 2 -c 1 ...`)."""
+"""One rank-128 trailing update C -= P P^T (lower tiles, m = 3840, the tile variant lfm_dgemm's heuristic picks) after two
+warm-ups: target for `ncu --set full` (`ncu -k regex:lfm_dgemm_kernel -s 2 -c 1 ...`)."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

@@ -1,7 +1,7 @@
-"""What a tile's life is made of in the rank-128 trailing update (64 x 64 tiles, two CTAs per SM): per-CTA debug words of
-lfm_debug_syrk_stamps (SM id, clock64 at entry / first operand unit landed / last DMMA issued / stores issued, globaltimer at
-entry / exit).  Prints the distribution of the phases over the CTAs of the launch and, per SM, the gaps between one CTA leaving
-a slot and the next one entering.  Run with LFM_GEMM_FORCE=3."""
+"""What a tile's life is made of in the rank-128 trailing update (the tile variant lfm_dgemm's heuristic picks): per-CTA debug
+words of lfm_debug_syrk_stamps (SM id, clock64 at entry / first operand unit landed / last DMMA issued / stores issued,
+globaltimer at entry / exit).  Prints the distribution of the phases over the CTAs of the launch and, per SM, the gaps between
+one CTA leaving a slot and the next one entering."""
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -10,7 +10,7 @@ l = _lib.lib(); dev = torch.device("cuda:0"); st = torch.cuda.current_stream().c
 n, m = 4096, int(sys.argv[1]) if len(sys.argv) > 1 else 3840
 K = int(sys.argv[2]) if len(sys.argv) > 2 else 128
 A = torch.randn(n, n, dtype=torch.float64, device=dev)
-T = (m // 64) * (m // 64 + 1) // 2
+T = (m // 64) * (m // 64 + 1) // 2   # 8 words per CTA for the smallest tiles; the rows the launch wrote are kept below
 S = torch.zeros(T * 8, dtype=torch.int64, device=dev)
 def run(stamps):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -22,8 +22,11 @@ def run(stamps):
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) * 1e3
 for _ in range(3): run(False)
-print("launch us: plain", round(min(run(False) for _ in range(4)), 1), "with stamps", round(min(run(True) for _ in range(4)), 1), "tiles", T, "beta0" if os.environ.get("LFM_DEBUG_SYRK_BETA0") else "")
+plain, stamped = round(min(run(False) for _ in range(4)), 1), round(min(run(True) for _ in range(4)), 1)
 s = S.cpu().numpy().reshape(T, 8)
+s = s[s[:, 6] != 0]   # CTAs of the launch (exit globaltimer written)
+T = len(s)
+print("launch us: plain", plain, "with stamps", stamped, "tiles", T)
 smid, t0, t1, t2, t3, g0, g1 = (s[:, i] for i in range(7))
 q = lambda x: [int(v) for v in np.percentile(x, [5, 25, 50, 75, 95])]
 print("cycles, percentiles 5/25/50/75/95 over the CTAs")
