@@ -128,12 +128,28 @@ __device__ __forceinline__ void w_h_core(const LfmPoint& pa, const LfmPoint& pb,
   }
 }
 
+// The small one of erf(x) / erfc(|x|): erfc(|x|) beyond 0.5, erf(x) inside (the other is 1 - it, with x's sign).
+__device__ __forceinline__ double w_erf_small(double x) {
+  const double ax = fabs(x);
+  return ax > 0.5 ? erfc(ax) : erf(x);
+}
+// x3 = t/l - gamma, formed the same way wherever its small erf value is evaluated or read back
+__device__ __forceinline__ double w_x3(double t, double inv_l, double gam) { return __fma_rn(t, inv_l, -gam); }
+// R2 = erf(x3) + erf(gamma) (the point's q, "second_erf_terms") from v3 = w_erf_small(x3) and vg = w_erf_small(gamma),
+// gamma > 0, by lfm_erfsum's rule: erfc(-x3) - erfc(gamma) when x3 < -0.5 and gamma > 0.5, where the literal sum
+// cancels (by up to 1 - erf(gamma), which exp(gamma^2) then multiplies)
+__device__ __forceinline__ double w_second_erfsum(double x3, double v3, double gam, double vg) {
+  const bool big3 = fabs(x3) > 0.5, bigg = gam > 0.5;
+  if (x3 < 0.0 && big3 && bigg) return v3 - vg;
+  return (big3 ? copysign(1.0 - v3, x3) : v3) + (bigg ? 1.0 - vg : vg);
+}
+
 // Stage-1 work items of an optimiser step (team kernels): every item is ONE transcendental of (theta, l, times).
 // Flat item f -> (kind << 24) | (gene << 16) | index:
-//   kind 0 / 1 / 2 : per gene: gamma and exp(gamma^2) / erf(gamma) / 2/sqrt(pi) exp(-gamma^2)
+//   kind 0 / 1 / 2 : per gene: gamma and exp(gamma^2) / erf or erfc of gamma / 2/sqrt(pi) exp(-gamma^2)
 //   kind 3         : per time i: exp(-t_i^2 / l^2)
 //   kind 4         : per time pair p: exp(-(t_ib - t_ia)^2 / l^2)
-//   kind 5 / 6 / 7 : per (gene, time i): exp(-d t) / erf and erfc of t/l + gamma / erf(t/l - gamma)
+//   kind 5 / 6 / 7 : per (gene, time i): exp(-d t) / erf and erfc of t/l + gamma / erf or erfc of t/l - gamma
 //   kind 8         : per (gene, distinct time difference k): erf or erfc of dt/l - gamma
 __device__ __forceinline__ int stage1_items(int G, int Tu, int nD) { return 3 * G + Tu + Tu * Tu + 3 * G * Tu + G * nD; }
 __device__ __forceinline__ unsigned stage1_decode(int f, int G, int Tu, int nD) {
@@ -153,23 +169,23 @@ __device__ __forceinline__ unsigned stage1_decode(int f, int G, int Tu, int nD) 
 }
 
 // The same items enumerated by cost class, so that a warp's 32 items of a round run ONE transcendental routine instead of
-// diverging over three: class 0 = erf-or-erfc (kinds 6, 8), class 1 = erf (kinds 1, 7), class 2 = exp (kinds 0, 2, 3, 4, 5).
+// diverging over two: class 0 = erf-or-erfc (kinds 1, 6, 7, 8), class 1 = exp (kinds 0, 2, 3, 4, 5).
 #define STAGE1_SKIP (15u << 24)
+#define STAGE1_CLASSES 2
 __device__ __forceinline__ int stage1_class_count(int cls, int G, int Tu, int nD) {
-  return cls == 0 ? G * Tu + G * nD : (cls == 1 ? G + G * Tu : 2 * G + Tu + Tu * Tu + G * Tu);
+  return cls == 0 ? G + 2 * G * Tu + G * nD : 2 * G + Tu + Tu * Tu + G * Tu;
 }
 __device__ __forceinline__ unsigned stage1_class_decode(int cls, int i, int G, int Tu, int nD) {
   if (cls == 0) {
-    if (i < G * Tu) { const int b = i / Tu; return (6u << 24) | ((unsigned)b << 16) | (unsigned)(i - b * Tu); }
-    i -= G * Tu;
-    const int b = i / nD;
-    return (8u << 24) | ((unsigned)b << 16) | (unsigned)(i - b * nD);
-  }
-  if (cls == 1) {
     if (i < G) return (1u << 24) | ((unsigned)i << 16);
     i -= G;
-    const int b = i / Tu;
-    return (7u << 24) | ((unsigned)b << 16) | (unsigned)(i - b * Tu);
+    if (i < 2 * G * Tu) {
+      const int e = i >> 1, b = e / Tu;
+      return ((i & 1 ? 7u : 6u) << 24) | ((unsigned)b << 16) | (unsigned)(e - b * Tu);
+    }
+    i -= 2 * G * Tu;
+    const int b = i / nD;
+    return (8u << 24) | ((unsigned)b << 16) | (unsigned)(i - b * nD);
   }
   if (i < G) return (0u << 24) | ((unsigned)i << 16);
   i -= G;
@@ -435,7 +451,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
   tsync<NW>();
   if constexpr (NW > 1) {
     // Stage-1 schedule: the items of a class are cut into chunks of 32 (one warp, one round), the chunks are handed
-    // heaviest class first to the least loaded warp (erf-or-erfc 8, erf 5, exp 2 cost units, measured order of
+    // heaviest class first to the least loaded warp (erf-or-erfc 8, exp 2 cost units, measured order of
     // magnitude), and slot (round r, warp w) of itab receives its chunk: itab[(r * NW + w) * 32 + lane].  A problem
     // whose chunks do not fit ITAB keeps s1_rounds = 0 and decodes the flat item list on the fly.
     __shared__ int sched_sh[ITAB / 32 + 1];
@@ -444,8 +460,8 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       for (int w = 0; w < NW; ++w) { load[w] = 0; used[w] = 0; }
       for (int sl = 0; sl < ITAB / 32; ++sl) sched_sh[sl] = -1;
       int ok = 1, rounds = 0;
-      for (int cls = 0; cls < 3 && ok; ++cls) {
-        const int cnt = stage1_class_count(cls, G, Tu, nD), wgt = cls == 0 ? 8 : (cls == 1 ? 5 : 2);
+      for (int cls = 0; cls < STAGE1_CLASSES && ok; ++cls) {
+        const int cnt = stage1_class_count(cls, G, Tu, nD), wgt = cls == 0 ? 8 : 2;
         for (int j = 0; j * 32 < cnt; ++j) {
           int best = 0;
           for (int w = 1; w < NW; ++w) if (load[w] < load[best]) best = w;
@@ -550,14 +566,15 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
     WSTAMP();
     // ---- B. unique points, q = P^T z, z^T z ------------------------------------------------------
     // Transcendentals, factored so that each is evaluated once per distinct argument:
-    //   per gene b          : gamma_b, exp(gamma_b^2), erf(gamma_b), g4_b = 2/sqrt(pi) exp(-gamma_b^2)
+    //   per gene b          : gamma_b, exp(gamma_b^2), erf or erfc of gamma_b, g4_b = 2/sqrt(pi) exp(-gamma_b^2)
     //   per time i          : Gt_i = exp(-t_i^2 / l^2)
-    //   per (b, i)          : Em = exp(-d_b t_i), Ep = 1 / Em, erf / erfc of t_i/l + gamma_b, erf(t_i/l - gamma_b),
+    //   per (b, i)          : Em = exp(-d_b t_i), Ep = 1 / Em, erf / erfc of t_i/l + gamma_b, erf or erfc of t_i/l - gamma_b,
     //                         g2 = g4_b Gt_i Em, g3 = g4_b Gt_i Ep           (2 gamma_b / l = d_b)
     //   per time pair       : Gd = exp(-(t_ib - t_ia)^2 / l^2)
     //   per (b, difference) : erf or erfc of (t_ib - t_ia)/l - gamma_b
     // and per table entry (b, ia, ib) only products remain: A1 = Em[ib] Ep[ia], A1 g1 = g4_b Gd.
     // |d_b t_i| > 600 (Ep would overflow) switches the whole team to direct evaluation of A1 and g1.
+    // The point's q = erf(t_i/l - gamma_b) + erf(gamma_b) is formed from the erf-or-erfc values (w_second_erfsum).
     // Stage 1: every item is ONE transcendental of (theta, l, times) alone; stage 2: the products.
     int slow = 0;
     double zz = 0.0;
@@ -570,7 +587,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       const double gam = th[m] * l * 0.5;
       gterm[4 * m + 0] = gam;
       gterm[4 * m + 1] = exp(gam * gam);
-      gterm[4 * m + 2] = erf(gam);
+      gterm[4 * m + 2] = w_erf_small(gam);
       gterm[4 * m + 3] = LFM_TWO_OVER_SQRT_PI * exp(-gam * gam);
     }
     for (int i = lane; i < Tu; i += 32) { const double tl = utime[i] * inv_l; Gt[i] = exp(-tl * tl); }
@@ -586,10 +603,10 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       const double em = exp(-d_b * t), ep = 1.0 / em;
       Em[b * MT + i] = em;
       Ep[b * MT + i] = ep;
-      const double x2 = t * inv_l + gam, x3 = t * inv_l - gam;
+      const double x2 = t * inv_l + gam;
       e2[b * MT + i] = erf(x2);
       c2[b * MT + i] = erfc(fabs(x2));
-      e3[b * MT + i] = erf(x3);
+      e3[b * MT + i] = w_erf_small(w_x3(t, inv_l, gam));
       g2[b * MT + i] = g4b * Gt[i] * em;
       g3t[b * MT + i] = g4b * Gt[i] * ep;
     }
@@ -613,10 +630,10 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       p.s = th[G + p.gene];
       p.gam = gterm[4 * p.gene + 0];
       p.eg2 = gterm[4 * p.gene + 1];
-      p.erfg = gterm[4 * p.gene + 2];
+      p.erfg = gterm[4 * p.gene + 2];   // (the small one of erf / erfc of gamma)
       p.g4 = gterm[4 * p.gene + 3];
       p.e = Em[p.gene * MT + p.ti];
-      p.q = e3[p.gene * MT + p.ti] + p.erfg;
+      p.q = w_second_erfsum(w_x3(p.t, inv_l, p.gam), e3[p.gene * MT + p.ti], p.gam, p.erfg);
       p.g3 = slow ? LFM_TWO_OVER_SQRT_PI * exp(-(p.t * inv_l - p.gam) * (p.t * inv_l - p.gam)) : g3t[p.gene * MT + p.ti];
       pts[r] = p;
       pgene[r] = p.gene;
@@ -656,23 +673,26 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
         const int kind = (int)(code >> 24), b = (int)((code >> 16) & 255u), idx = (int)(code & 0xffffu);
         if (kind == 15) continue;
         const double gam = th[b] * l * 0.5;
-        // ONE call site per routine (exp / erf / erf-or-erfc): the lanes of a scheduled chunk differ in how the argument
+        // ONE call site per routine (exp / erf-or-erfc): the lanes of a scheduled chunk differ in how the argument
         // is formed and where the value goes, not in the routine they run
-        if (kind == 1 || kind == 7) {
-          const double x = (kind == 1) ? gam : utime[idx] * inv_l - gam;
-          const double v = erf(x);
-          if (kind == 1) gterm[4 * b + 2] = v; else e3[b * MT + idx] = v;
-        } else if (kind == 6 || kind == 8) {
-          // the small one of erf(x) / erfc(|x|) is evaluated, the other is 1 - it (kind 6 keeps both, kind 8 the small one)
-          const double x = (kind == 6) ? utime[idx] * inv_l + gam : dval[idx] * inv_l - gam;
+        if (kind == 1 || kind >= 6) {
+          // the small one of erf(x) / erfc(|x|) is evaluated, the other is 1 - it (kind 6 keeps both, kinds 1, 7, 8 the
+          // small one)
+          const double x = kind == 6 ? utime[idx] * inv_l + gam
+                         : kind == 8 ? dval[idx] * inv_l - gam
+                         : kind == 7 ? w_x3(utime[idx], inv_l, gam) : gam;
           const double ax = fabs(x);
           const bool big = ax > 0.5;
           const double v = big ? erfc(ax) : erf(x);
           if (kind == 6) {
             e2[b * MT + idx] = big ? copysign(1.0 - v, x) : v;
             c2[b * MT + idx] = big ? v : 1.0 - fabs(v);
-          } else {
+          } else if (kind == 8) {
             er1[b * MT * MT + idx] = v;
+          } else if (kind == 7) {
+            e3[b * MT + idx] = v;
+          } else {
+            gterm[4 * b + 2] = v;
           }
         } else {
           double arg;
@@ -726,10 +746,10 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
         p.s = th[G + p.gene];
         p.gam = gterm[4 * p.gene + 0];
         p.eg2 = gterm[4 * p.gene + 1];
-        p.erfg = gterm[4 * p.gene + 2];
+        p.erfg = gterm[4 * p.gene + 2];   // (the small one of erf / erfc of gamma)
         p.g4 = gterm[4 * p.gene + 3];
         p.e = Em[p.gene * MT + p.ti];
-        p.q = e3[p.gene * MT + p.ti] + p.erfg;
+        p.q = w_second_erfsum(w_x3(p.t, inv_l, p.gam), e3[p.gene * MT + p.ti], p.gam, p.erfg);
         p.g3 = slow ? LFM_TWO_OVER_SQRT_PI * exp(-(p.t * inv_l - p.gam) * (p.t * inv_l - p.gam))
                     : p.g4 * Gt[p.ti] * (1.0 / p.e);
         pts[r] = p;

@@ -15,7 +15,7 @@ struct LfmPoint {
   double eg2;   // exp(gamma_j^2)
   double erfg;  // erf(gamma_j)
   double e;     // exp(-D_j t)
-  double q;     // erf(t/l - gamma_j) + erf(gamma_j)           ("second_erf_terms", model.py:355-357)
+  double q;     // erf(t/l - gamma_j) + erf(gamma_j)           ("second_erf_terms", model.py:355-357; lfm_erfsum)
   double g3;    // 2/sqrt(pi) exp(-(t/l - gamma_j)^2)           (gradient only)
   double g4;    // 2/sqrt(pi) exp(-gamma_j^2)                   (gradient only)
   int gene;     // resolved gene index
@@ -30,6 +30,21 @@ __device__ __forceinline__ int lfm_resolve_gene(double gcol, int G) {
   g = g < 0 ? 0 : g;
   g = g >= G ? G - 1 : g;
   return g;
+}
+
+// erf(a) + erf(b) without catastrophic cancellation.  In h and k_xf the first sum R1 multiplies
+// exp(-D dt) with dt < 0 (up to e^13 in the p53 regime) exactly when erf(a) ~ -1 and erf(b) ~ +1
+// (SURVEY Q7): the literal sum then carries ~1e-16 * e^(D|dt|) absolute noise.  The second sum of h,
+// R2 = erf(t/l - gamma) + erf(gamma), cancels for t/l < gamma and is multiplied by exp(gamma^2): the
+// literal form loses ~1e-16 * exp(gamma^2) (5e-11 of the covariance scale at gamma = 4.4, 4e-2 at 7).
+// For opposite-sign arguments that are both beyond 0.5 the identical quantity erfc(-n) - erfc(p) is
+// used instead.  The oracle (oracle/lfm_oracle.py:erfsum) uses the same rule with the same threshold.
+__device__ __forceinline__ double lfm_erfsum(double a, double b) {
+  if (a * b < 0.0 && fmin(fabs(a), fabs(b)) > 0.5) {
+    const double p = fmax(a, b), n = fmin(a, b);
+    return erfc(-n) - erfc(p);
+  }
+  return erf(a) + erf(b);
 }
 
 __device__ __forceinline__ LfmPoint lfm_make_point(const double* __restrict__ row3, int G,
@@ -47,7 +62,7 @@ __device__ __forceinline__ LfmPoint lfm_make_point(const double* __restrict__ ro
   p.erfg = erf(p.gam);
   p.e = exp(-p.d * p.t);
   const double x3 = p.t / l - p.gam;
-  p.q = erf(x3) + p.erfg;
+  p.q = lfm_erfsum(x3, p.gam);
   if (grad) {
     p.g3 = LFM_TWO_OVER_SQRT_PI * exp(-x3 * x3);
     p.g4 = LFM_TWO_OVER_SQRT_PI * exp(-p.gam * p.gam);
@@ -56,19 +71,6 @@ __device__ __forceinline__ LfmPoint lfm_make_point(const double* __restrict__ ro
     p.g4 = 0.0;
   }
   return p;
-}
-
-// erf(a) + erf(b) without catastrophic cancellation.  In h and k_xf this sum multiplies
-// exp(-D dt) with dt < 0 (up to e^13 in the p53 regime) exactly when erf(a) ~ -1 and erf(b) ~ +1
-// (SURVEY Q7): the literal sum then carries ~1e-16 * e^(D|dt|) absolute noise.  For opposite-sign
-// arguments that are both beyond 0.5 the identical quantity erfc(-n) - erfc(p) is used instead.  The
-// oracle (oracle/lfm_oracle.py:erfsum) uses the same rule with the same threshold.
-__device__ __forceinline__ double lfm_erfsum(double a, double b) {
-  if (a * b < 0.0 && fmin(fabs(a), fabs(b)) > 0.5) {
-    const double p = fmax(a, b), n = fmin(a, b);
-    return erfc(-n) - erfc(p);
-  }
-  return erf(a) + erf(b);
 }
 
 // H(a,b,u,v) = h(j=a, k=b, t1=u, t2=v) of model.py:315-365, with "b" the gene whose gamma enters.
