@@ -33,6 +33,15 @@ _lib: Optional[C.CDLL] = None
 
 _i64, _int, _dbl, _ptr, _sz = C.c_int64, C.c_int, C.c_double, C.c_void_p, C.c_size_t
 
+
+class GemmDesc(C.Structure):
+    """lfm_gemm_desc of include/lfm_b200.h (lfm_debug_dgemm)."""
+    _fields_ = [("transA", _int), ("transB", _int), ("M", _i64), ("N", _i64), ("K", _i64),
+                ("A", _ptr), ("lda", _i64), ("B", _ptr), ("ldb", _i64), ("C", _ptr), ("ldc", _i64),
+                ("alpha", _dbl), ("beta", _dbl), ("lower_only", _int), ("kmode", _int), ("batch", _int),
+                ("strideA", _i64), ("strideB", _i64), ("strideC", _i64), ("tile", _int), ("tri_skip", _int),
+                ("k_split", _i64), ("k_lo", _i64), ("k_hi", _i64)]
+
 # name -> (restype, argtypes); mirrors include/lfm_b200.h one to one
 SIGNATURES = {
     "lfm_abi_version": (_int, []),
@@ -126,6 +135,7 @@ SIGNATURES = {
     "lfm_debug_profile_variants": (_sz, [C.c_char_p, _sz]),
     "lfm_debug_profile_chain": (_int, [C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_longlong)]),
     "lfm_debug_dgemm_nt": (_int, [_ptr, _i64, _i64, _i64, _ptr, _ptr, _ptr]),
+    "lfm_debug_dgemm": (_int, [_ptr, _ptr, C.POINTER(_int)]),
     "lfm_debug_potrf_potri": (_int, [_ptr, _i64, _ptr, _ptr, _ptr, _ptr]),
     "lfm_debug_syrk": (_int, [_ptr, _i64, _i64, _ptr, _i64, _ptr, _i64]),
     "lfm_debug_syrk_stamps": (_int, [_ptr, _i64, _i64, _ptr, _i64, _ptr, _i64, _ptr]),

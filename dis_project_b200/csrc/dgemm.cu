@@ -104,7 +104,6 @@ __global__ void __launch_bounds__(128 * GM, (WM * WN * GM <= 16) ? 2 : 1) lfm_dg
   int64_t kb = 0, ke = g.K;
   switch (g.kmode) {
     case LFM_K_LE_ROW: ke = min(g.K, row0 + BM); break;
-    case LFM_K_GE_COL: kb = col0; break;
     case LFM_K_GE_ROW: kb = row0; break;
     case LFM_K_GE_ROWCOL: kb = max(row0, col0); break;
     case LFM_K_LAUUM_LATE: kb = row0 < g.k_split ? g.k_split : max(row0, col0); break;
@@ -314,7 +313,6 @@ static double gemm_exec_flops(const LfmGemm& g, int BM, int BN) {
       const int64_t row0 = i * BM, col0 = j * BN;
       switch (g.kmode) {
         case LFM_K_LE_ROW: ke = g.K < row0 + BM ? g.K : row0 + BM; break;
-        case LFM_K_GE_COL: kb = col0; break;
         case LFM_K_GE_ROW: kb = row0; break;
         case LFM_K_GE_ROWCOL: kb = row0 > col0 ? row0 : col0; break;
         case LFM_K_LAUUM_LATE: kb = row0 < g.k_split ? g.k_split : (row0 > col0 ? row0 : col0); break;
@@ -412,9 +410,12 @@ static cudaEvent_t prof_event() {
   return g_prof.ev[g_prof.used++];
 }
 
+// `variant` (may be NULL) receives the instantiation's code TA TBN WM WN GM as decimal digits (the profiler's code)
 template <int TA, int TBN, int WM, int WN, int GM>
-static int launch(cudaStream_t st, const LfmGemm& g) {
+static int launch(cudaStream_t st, const LfmGemm& g, int* variant) {
   constexpr int BM = 8 * WM * GM, BN = 32 * WN;
+  constexpr int VARIANT = TA * 10000 + TBN * 1000 + WM * 100 + WN * 10 + GM;
+  if (variant) *variant = VARIANT;
   constexpr int SMEM = STAGES * (BM + BN) * LDK * 8;
   auto* const kernel = &lfm_dgemm_kernel<TA, TBN, WM, WN, GM>;
   static LfmSmemConfig smem_cfg;
@@ -448,7 +449,7 @@ static int launch(cudaStream_t st, const LfmGemm& g) {
     const double f = gemm_exec_flops(g, BM, BN) * (g.batch > 1 ? g.batch : 1);
     const bool chain = BM == 16;
     g_prof.is_chain.push_back(chain ? 1 : 0);
-    g_prof.variant.push_back(TA * 10000 + TBN * 1000 + WM * 100 + WN * 10 + GM);
+    g_prof.variant.push_back(VARIANT);
     g_prof.pair_flops.push_back(f);
     if (chain) { g_prof.chain_flops += f; g_prof.chain_launches += 1; }
     else { g_prof.flops += f; g_prof.launches += 1; }
@@ -480,35 +481,74 @@ static int launch(cudaStream_t st, const LfmGemm& g) {
 }
 
 template <int WM, int WN, int GM>
-static int dispatch(cudaStream_t st, const LfmGemm& g) {
-  if (g.transA == 0 && g.transB == 1) return launch<0, 1, WM, WN, GM>(st, g);
-  if (g.transA == 0 && g.transB == 0) return launch<0, 0, WM, WN, GM>(st, g);
-  if (g.transA == 1 && g.transB == 0) return launch<1, 0, WM, WN, GM>(st, g);
-  return launch<1, 1, WM, WN, GM>(st, g);
+static int dispatch(cudaStream_t st, const LfmGemm& g, int* variant) {
+  if (g.transA == 0 && g.transB == 1) return launch<0, 1, WM, WN, GM>(st, g, variant);
+  if (g.transA == 0 && g.transB == 0) return launch<0, 0, WM, WN, GM>(st, g, variant);
+  if (g.transA == 1 && g.transB == 0) return launch<1, 0, WM, WN, GM>(st, g, variant);
+  return launch<1, 1, WM, WN, GM>(st, g, variant);
 }
 
-// Tile-shape heuristic: 128 x 128 tiles once they fill >= 3 waves of the 148 SMs, else 64 x 64 tiles
-// (two CTAs per SM) so that small trailing updates and panels still spread over the whole chip.
-// C aliasing A (in-place panel multiply) needs one tile across the full width N = 128.
-int lfm_dgemm(cudaStream_t st, const LfmGemm& g) {
+// Tile shape of a launch, WM WN GM as decimal digits, or a negative lfm_status.  Heuristic: 128 x 128 tiles once they
+// fill >= 3 waves of the 148 SMs, else 64 x 64 tiles (two CTAs per SM) so that small trailing updates and panels still
+// spread over the whole chip.  C aliasing A (in-place panel multiply) needs one tile across the full width N = 128; those
+// tiles are not square, so they cannot serve lower_only.
+static int dgemm_tile(const LfmGemm& g) {
+  if ((g.transA | g.transB) & ~1) return LFM_ERR_INVALID;
+  if (g.kmode != LFM_K_FULL && g.kmode != LFM_K_LE_ROW && g.kmode != LFM_K_GE_ROW && g.kmode != LFM_K_GE_ROWCOL &&
+      g.kmode != LFM_K_LAUUM_LATE)
+    return LFM_ERR_INVALID;
+  if (g.M < 0 || g.N < 0 || g.K < 0 || g.tri_skip < 0) return LFM_ERR_INVALID;
   if (g.M % 128 || g.N % 128 || g.K % BK) return LFM_ERR_INVALID;
+  if (g.k_lo % BK || g.k_hi % BK || g.k_split % BK) return LFM_ERR_INVALID;
   if (g.lower_only && g.M != g.N) return LFM_ERR_INVALID;
   const int64_t nb = g.batch > 1 ? g.batch : 1;
   if (nb > 65535) return LFM_ERR_UNSUPPORTED;
   const int64_t t128 = nb * (g.lower_only ? (g.M / 128) * (g.M / 128 + 1) / 2 : (g.M / 128) * (g.N / 128));
   const bool inplace = (const double*)g.C == g.A;
   if (g.tile == 1) {
-    if (g.N % 128 || g.lower_only) return LFM_ERR_INVALID;
-    return dispatch<1, 4, 2>(st, g);
+    if (g.lower_only) return LFM_ERR_INVALID;
+    return 142;
   }
-  if (g.tile == 2 && !inplace) return dispatch<4, 4, 4>(st, g);   // 128 x 128 tiles whatever the tile count
-  if (g.tile == 3 && !inplace) return dispatch<4, 2, 2>(st, g);   // 64 x 64 tiles (two CTAs per SM)
+  if (g.tile == 2 && !inplace) return 444;   // 128 x 128 tiles whatever the tile count
+  if (g.tile == 3 && !inplace) return 422;   // 64 x 64 tiles (two CTAs per SM)
   if (inplace) {
-    if (g.N != 128) return LFM_ERR_INVALID;
-    if (t128 >= 148) return dispatch<8, 4, 2>(st, g);
-    return (g.M / 64 >= 148) ? dispatch<4, 4, 2>(st, g) : dispatch<2, 4, 2>(st, g);  // 64- or 32-row tiles: fill the SMs
+    if (g.N != 128 || g.lower_only) return LFM_ERR_INVALID;
+    if (t128 >= 148) return 842;
+    return (g.M / 64 >= 148) ? 442 : 242;    // 64- or 32-row tiles: fill the SMs
   }
-  if (g.tri_skip > 0) return dispatch<4, 2, 2>(st, g);  // rank-128 trailing updates: 64 x 64 tiles measured fastest
-  if (t128 >= 3 * 148) return dispatch<4, 4, 4>(st, g);
-  return dispatch<4, 2, 2>(st, g);
+  if (g.tri_skip > 0) return 422;  // rank-128 trailing updates: 64 x 64 tiles measured fastest
+  if (t128 >= 3 * 148) return 444;
+  return 422;
+}
+
+static int dgemm_run(cudaStream_t st, const LfmGemm& g, int* variant) {
+  const int t = dgemm_tile(g);
+  switch (t) {
+    case 142: return dispatch<1, 4, 2>(st, g, variant);
+    case 242: return dispatch<2, 4, 2>(st, g, variant);
+    case 422: return dispatch<4, 2, 2>(st, g, variant);
+    case 442: return dispatch<4, 4, 2>(st, g, variant);
+    case 444: return dispatch<4, 4, 4>(st, g, variant);
+    case 842: return dispatch<8, 4, 2>(st, g, variant);
+    default: return t < 0 ? t : LFM_ERR_INVALID;
+  }
+}
+
+int lfm_dgemm(cudaStream_t st, const LfmGemm& g) { return dgemm_run(st, g, nullptr); }
+
+// Debug: any launch lfm_dgemm can make, from a plain C descriptor.  What the kernel's 16-byte copies need is checked here,
+// before anything is launched: aligned base pointers, even leading dimensions and batch strides.
+extern "C" int lfm_debug_dgemm(lfm_stream_t stream, const lfm_gemm_desc* d, int* variant) {
+  if (variant) *variant = 0;
+  if (!d || !d->A || !d->B || !d->C) return LFM_ERR_INVALID;
+  auto misaligned = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) != 0; };
+  if (misaligned(d->A) || misaligned(d->B) || misaligned(d->C)) return LFM_ERR_INVALID;
+  if ((d->lda | d->ldb | d->ldc | d->strideA | d->strideB | d->strideC) & 1) return LFM_ERR_INVALID;
+  LfmGemm g;
+  g.transA = d->transA; g.transB = d->transB; g.M = d->M; g.N = d->N; g.K = d->K;
+  g.A = d->A; g.lda = d->lda; g.B = d->B; g.ldb = d->ldb; g.C = d->C; g.ldc = d->ldc;
+  g.alpha = d->alpha; g.beta = d->beta; g.lower_only = d->lower_only; g.kmode = d->kmode;
+  g.batch = d->batch; g.strideA = d->strideA; g.strideB = d->strideB; g.strideC = d->strideC;
+  g.tile = d->tile; g.tri_skip = d->tri_skip; g.k_split = d->k_split; g.k_lo = d->k_lo; g.k_hi = d->k_hi;
+  return dgemm_run((cudaStream_t)stream, g, variant);
 }

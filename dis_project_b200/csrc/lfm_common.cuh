@@ -71,11 +71,10 @@ static inline LfmTheta lfm_theta_view(const double* theta, int G) {
 
 // ---- dense primitives (dgemm.cu / chol.cu) -------------------------------------------------
 // C[M x N] = alpha * op(A) op(B) + beta * C, row-major, M,N multiples of 128, K multiple of 16.
-// kmode restricts the k-range per output tile (triangular operands):
+// kmode restricts the k-range per output tile (triangular operands; 2 is not a mode):
 enum LfmKMode {
   LFM_K_FULL = 0,
   LFM_K_LE_ROW = 1,   // k <  row_tile_end          (A lower-triangular, op(A) = A)
-  LFM_K_GE_COL = 2,   // k >= col_tile_start        (B lower-triangular, op(B) = B, NN)
   LFM_K_GE_ROW = 3,   // k >= row_tile_start        (op(A) = A^T with A lower-triangular)
   LFM_K_GE_ROWCOL = 4, // k >= max(row, col) start   (A^T A with A lower-triangular)
   LFM_K_LAUUM_LATE = 5 // as 4 for the tiles of the rows >= k_split (beta = 0); tiles of the rows < k_split ACCUMULATE (beta = 1) over

@@ -4,6 +4,7 @@ path.  All calls are stream-ordered on torch's current stream and do not synchro
 """
 from __future__ import annotations
 
+import ctypes
 import math
 from typing import Dict, Optional, Tuple
 
@@ -656,6 +657,42 @@ def debug_dgemm_nt(A: torch.Tensor, B: torch.Tensor) -> torch.Tensor:
     _lib.check(_lib.lib().lfm_debug_dgemm_nt(_stream(), M, N, K, A.data_ptr(), B.data_ptr(), Cm.data_ptr()),
                "lfm_debug_dgemm_nt")
     return Cm
+
+
+GEMM_KMODES = {"full": 0, "le_row": 1, "ge_row": 3, "ge_rowcol": 4, "lauum_late": 5}
+
+
+def debug_dgemm(A: torch.Tensor, B: torch.Tensor, C: torch.Tensor, M: int, N: int, K: int, *, lda: int, ldb: int,
+                ldc: int, transA: int = 0, transB: int = 0, offA: int = 0, offB: int = 0, offC: int = 0,
+                alpha: float = 1.0, beta: float = 0.0, lower_only: bool = False, kmode: int = 0, batch: int = 1,
+                strideA: int = 0, strideB: int = 0, strideC: int = 0, tile: int = 0, tri_skip: int = 0,
+                k_split: int = 0, k_lo: int = 0, k_hi: int = 1 << 62) -> int:
+    """One launch of the dense path's DMMA GEMM (lfm_debug_dgemm, include/lfm_b200.h) over 1-D float64 CUDA buffers.
+    Operands start at element offsets offA / offB / offC of their buffers; pass the same buffer and offset for C and A
+    to multiply in place.  Returns the code of the instantiation that ran (TA TBN WM WN GM as decimal digits); a
+    descriptor the library refuses raises _lib.LfmError with its status.  Raises ValueError, before calling the
+    library, if any element an operand could be read or written at lies outside its buffer."""
+    nb = batch if batch > 1 else 1
+    ops_ = (("A", A, offA, lda, strideA, (K, M) if transA else (M, K)),
+            ("B", B, offB, ldb, strideB, (N, K) if transB else (K, N)),
+            ("C", C, offC, ldc, strideC, (M, N)))
+    for name, buf, off, ld, stride, (rows, cols) in ops_:
+        if not (isinstance(buf, torch.Tensor) and buf.is_cuda and buf.dtype == F64 and buf.ndim == 1
+                and buf.is_contiguous()):
+            raise ValueError(f"{name} must be a contiguous 1-D float64 CUDA tensor")
+        if min(off, ld, stride) < 0:
+            raise ValueError(f"{name}: negative offset, leading dimension or stride")
+        if rows > 0 and cols > 0 and off + (nb - 1) * stride + (rows - 1) * ld + cols - 1 >= buf.numel():
+            raise ValueError(f"{name}: a {rows} x {cols} operand (ld {ld}, {nb} problems, stride {stride}) at offset "
+                             f"{off} reaches past the buffer's {buf.numel()} elements")
+    d = _lib.GemmDesc(transA=int(transA), transB=int(transB), M=M, N=N, K=K,
+                      A=A.data_ptr() + 8 * offA, lda=lda, B=B.data_ptr() + 8 * offB, ldb=ldb,
+                      C=C.data_ptr() + 8 * offC, ldc=ldc, alpha=alpha, beta=beta, lower_only=int(lower_only),
+                      kmode=kmode, batch=batch, strideA=strideA, strideB=strideB, strideC=strideC, tile=tile,
+                      tri_skip=tri_skip, k_split=k_split, k_lo=k_lo, k_hi=k_hi)
+    variant = ctypes.c_int(0)
+    _lib.check(_lib.lib().lfm_debug_dgemm(_stream(), ctypes.byref(d), ctypes.byref(variant)), "lfm_debug_dgemm")
+    return variant.value
 
 
 def debug_potrf_potri(A: torch.Tensor, want_inverse: bool = True):

@@ -397,6 +397,28 @@ int lfm_batched_fit_het_host(lfm_handle* h, int64_t B, int64_t N, int G, const d
 /* Plain C = A B^T fp64 GEMM through the library's own DMMA kernel (M,N % 128 == 0, K % 16 == 0). */
 int lfm_debug_dgemm_nt(lfm_stream_t stream, int64_t M, int64_t N, int64_t K, const double* A,
                        const double* B, double* C);
+/* Every launch the dense path's DMMA GEMM can make: C = alpha op(A) op(B) + beta C, row-major, the fields of the
+ * library's internal launch descriptor (csrc/lfm_common.cuh, LfmGemm).  transA = 1: A stored K x M; transB = 1: B stored
+ * N x K.  kmode restricts each output tile's k-range: 0 full, 1 k < row tile end, 3 k >= row tile start, 4 k >= max(row,
+ * column) tile start, 5 as 4 for the tile rows >= k_split and k in [k_split, K) accumulating (beta = 1) above them.  The
+ * range is then clipped to [k_lo, k_hi) (multiples of 16); with beta = 1 and alpha = +-1, a tile whose range is empty is
+ * left untouched.  lower_only skips the tiles above the diagonal and, with tri_skip, those of the first tri_skip rows.
+ * batch > 1 runs problem y at A + y strideA, B + y strideB, C + y strideC.  tile: 0 heuristic, 1 16 x 128, 2 128 x 128,
+ * 3 64 x 64 tiles.  LFM_ERR_INVALID before any launch for a base pointer that is not 16-byte aligned or an odd leading
+ * dimension or stride.  *variant receives the instantiation that ran, TA TBN WM WN GM as decimal digits (0 if none). */
+typedef struct lfm_gemm_desc {
+  int transA, transB;
+  int64_t M, N, K;
+  const double* A; int64_t lda;
+  const double* B; int64_t ldb;
+  double* C; int64_t ldc;
+  double alpha, beta;
+  int lower_only, kmode, batch;
+  int64_t strideA, strideB, strideC;
+  int tile, tri_skip;
+  int64_t k_split, k_lo, k_hi;
+} lfm_gemm_desc;
+int lfm_debug_dgemm(lfm_stream_t stream, const lfm_gemm_desc* desc, int* variant);
 /* In-place dense lower Cholesky / inverse of an n x n row-major matrix (n % 128 == 0): after the
  * call A holds L (lower), and if Sinv != NULL it receives Sigma^-1 (lower triangle valid).
  * W is an n x n scratch matrix. */
