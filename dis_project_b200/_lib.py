@@ -137,6 +137,7 @@ SIGNATURES = {
     "lfm_debug_dgemm_nt": (_int, [_ptr, _i64, _i64, _i64, _ptr, _ptr, _ptr]),
     "lfm_debug_dgemm": (_int, [_ptr, _ptr, C.POINTER(_int)]),
     "lfm_debug_potrf_potri": (_int, [_ptr, _i64, _ptr, _ptr, _ptr, _ptr]),
+    "lfm_debug_potrf_potri_eval": (_int, [_ptr, _i64, _ptr, _ptr, _ptr, _int, C.POINTER(_int), _ptr]),
     "lfm_debug_syrk": (_int, [_ptr, _i64, _i64, _ptr, _i64, _ptr, _i64]),
     "lfm_debug_syrk_stamps": (_int, [_ptr, _i64, _i64, _ptr, _i64, _ptr, _i64, _ptr]),
 }

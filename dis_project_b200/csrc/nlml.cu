@@ -506,3 +506,23 @@ extern "C" int lfm_debug_potrf_potri(lfm_stream_t stream, int64_t n, double* A, 
   }
   return LFM_OK;
 }
+// The factorisation and Sigma^-1 exactly as nlml_grad_impl runs them on Sigma (nlml_factor with grad = true, then lauum).
+extern "C" int lfm_debug_potrf_potri_eval(lfm_stream_t stream, int64_t n, double* A, double* W, double* ldiag,
+                                          int chain_ready, int* early_done, int* info) {
+  if (n <= 0 || n % LFM_NB || !A || !W || !ldiag || !info) return LFM_ERR_INVALID;
+  cudaStream_t st = (cudaStream_t)stream;
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 16) return LFM_ERR_CUDA;
+  if (!g_eval_side[dev].init()) return LFM_ERR_CUDA;
+  int early = 0;
+  if (chain_ready && lfm_potrf_trtri_is_one_sweep(n)) {
+    LFM_CUDA_OK(cudaMemsetAsync(info, 0, sizeof(int), st));
+    LFM_CUDA_OK(cudaEventRecord(g_eval_side[dev].cols, st));
+    LFM_TRY(lfm_potrf_trtri_diag(st, n, A, n, W, n, info, ldiag, &early, g_eval_side[dev].cols));
+  } else {
+    LFM_TRY(lfm_potrf_trtri_diag(st, n, A, n, W, n, info, ldiag, &early));
+  }
+  LFM_TRY(early ? lfm_lauum_late(st, n, W, n, A, n) : lfm_lauum(st, n, W, n, A, n));
+  if (early_done) *early_done = early;
+  return LFM_OK;
+}

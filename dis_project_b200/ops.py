@@ -695,14 +695,38 @@ def debug_dgemm(A: torch.Tensor, B: torch.Tensor, C: torch.Tensor, M: int, N: in
     return variant.value
 
 
-def debug_potrf_potri(A: torch.Tensor, want_inverse: bool = True):
-    """In-place Cholesky (+ inverse) of a dense SPD matrix; returns (L, Sinv_lower or None, info)."""
+def _scratch_like(A: torch.Tensor, W: Optional[torch.Tensor]) -> torch.Tensor:
+    if W is None:
+        return torch.zeros_like(A)
+    if not (W.is_cuda and W.dtype == F64 and W.shape == A.shape and W.is_contiguous()):
+        raise ValueError(f"W must be a contiguous float64 CUDA tensor of shape {tuple(A.shape)}")
+    return W
+
+
+def debug_potrf_potri(A: torch.Tensor, want_inverse: bool = True, W: Optional[torch.Tensor] = None):
+    """In-place Cholesky (+ inverse) of a dense SPD matrix; returns (L, Sinv_lower or None, info).  `W` (n x n, may be
+    None) is the scratch the library works in: after the call its lower triangle holds W = L^-1 when want_inverse."""
     A = _dev(A)
     n = A.shape[0]
-    W = torch.zeros_like(A)
+    W = _scratch_like(A, W)
     Sinv = torch.zeros_like(A) if want_inverse else None
     info = torch.zeros(1, dtype=torch.int32, device=A.device)
     _lib.check(_lib.lib().lfm_debug_potrf_potri(_stream(), n, A.data_ptr(), W.data_ptr(),
                                                 Sinv.data_ptr() if want_inverse else None, info.data_ptr()),
                "lfm_debug_potrf_potri")
     return A, Sinv, info
+
+
+def debug_factor_inverse_eval(A: torch.Tensor, chain_ready: bool = True, W: Optional[torch.Tensor] = None):
+    """The factorisation and Sigma^-1 in the sequence the NLML gradient runs them (lfm_debug_potrf_potri_eval), in place:
+    returns (Sinv_lower (= A), W = L^-1 (lower), diag(L), early_done, info)."""
+    A = _dev(A)
+    n = A.shape[0]
+    W = _scratch_like(A, W)
+    ldiag = torch.empty(n, dtype=F64, device=A.device)
+    info = torch.zeros(1, dtype=torch.int32, device=A.device)
+    early = ctypes.c_int(0)
+    _lib.check(_lib.lib().lfm_debug_potrf_potri_eval(_stream(), n, A.data_ptr(), W.data_ptr(), ldiag.data_ptr(),
+                                                     int(bool(chain_ready)), ctypes.byref(early), info.data_ptr()),
+               "lfm_debug_potrf_potri_eval")
+    return A, W, ldiag, bool(early.value), info

@@ -18,7 +18,9 @@
  *   - return value: LFM_OK or a negative lfm_status.  Numerical failure (Sigma not positive
  *     definite) is reported asynchronously through the device word `info` (0 = ok, k>0 = 1-based
  *     failing pivot), exactly like LAPACK; the outputs are then NaN, as in the reference
- *     (JAX's Cholesky returns NaN instead of raising).
+ *     (JAX's Cholesky returns NaN instead of raising).  One deviation: the dense factorisation also
+ *     fails at a positive pivot below DBL_MIN (2^-1022), which LAPACK would factor (its reciprocal
+ *     square root flushes subnormals to zero).
  */
 #ifndef LFM_B200_H
 #define LFM_B200_H
@@ -423,6 +425,14 @@ int lfm_debug_dgemm(lfm_stream_t stream, const lfm_gemm_desc* desc, int* variant
  * call A holds L (lower), and if Sinv != NULL it receives Sigma^-1 (lower triangle valid).
  * W is an n x n scratch matrix. */
 int lfm_debug_potrf_potri(lfm_stream_t stream, int64_t n, double* A, double* W, double* Sinv, int* info);
+/* The same factorisation and inverse in the sequence the NLML gradient runs: W = L^-1 (lower), diag(L) into ldiag
+ * (n doubles), Sigma^-1 = W^T W started early where the sweep does so, and after the call A holds Sigma^-1 (lower
+ * triangle valid).  chain_ready != 0: info is zeroed and an event recorded on `stream`, and the factorisation's chain
+ * starts behind that event, as behind the first two block columns of Sigma (one-sweep sizes: n / 128 a power of two,
+ * 4 <= n / 128 <= 32; ignored otherwise).  *early_done (host int, may be NULL) receives 1 when Sigma^-1 was finished by
+ * the late half of the product (lfm_lauum_late) and 0 when by one full product. */
+int lfm_debug_potrf_potri_eval(lfm_stream_t stream, int64_t n, double* A, double* W, double* ldiag, int chain_ready,
+                               int* early_done, int* info);
 /* C (lower tiles, m x m) -= P P^T, P m x K: the trailing update of the blocked Cholesky (roofline helper). */
 int lfm_debug_syrk(lfm_stream_t stream, int64_t m, int64_t K, const double* P, int64_t ldp, double* C, int64_t ldc);
 /* The same launch with 8 debug words per CTA in `stamps` (tiles of the launch x 8 int64): [0] SM id, clock64 at [1] entry,

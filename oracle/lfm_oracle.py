@@ -44,6 +44,8 @@ from scipy.special import erf, erfc
 from scipy.linalg import cho_solve, cholesky, solve_triangular
 from scipy.linalg.lapack import dpotrf, dpotri
 
+from . import ld_linalg
+
 SQRT_PI = math.sqrt(math.pi)
 L_LOW, L_HIGH = 0.5, 3.5  # model.py:111
 
@@ -333,12 +335,15 @@ def _h_partials(p: Params, a, b, u, v):
 
 
 def nlml_and_grad(p: Params, x: np.ndarray, y: np.ndarray, *, chunk: int = 256, threads: int | None = None,
-                  variances=None):
+                  variances=None, linalg: str = "fp64"):
     """Closed-form NLML and gradient w.r.t. the CONSTRAINED theta=[d,s,b,l,sigma].
 
     K_bar = 1/2 (S^-1 - a a^T); dNLML/dtheta = sum_ij K_bar_ij dK_ij/dtheta (+ mean terms).
     Training rows only (all flags 1).  Row-chunked (so N=32768 fits in RAM) and the chunks are
     spread over `threads` host threads (numpy ufuncs and LAPACK release the GIL).
+    linalg="ld": the Cholesky, the solve, the log-determinant and S^-1 run in extended precision
+    (oracle.ld_linalg, n <= ~1024) and are rounded to fp64 before the same contraction -- the reference
+    where cond(S) makes LAPACK's fp64 answer itself inaccurate.
     """
     import os
     from concurrent.futures import ThreadPoolExecutor
@@ -367,13 +372,25 @@ def nlml_and_grad(p: Params, x: np.ndarray, y: np.ndarray, *, chunk: int = 256, 
             S[np.diag_indices(n)] += np.asarray(variances, dtype=np.float64).reshape(-1)   # formulas are unchanged
         mu = mean_function(p, x)
         z = y - mu
-        c, info = dpotrf(S, lower=1, overwrite_a=1, clean=0)
-        if info != 0:
-            raise np.linalg.LinAlgError(f"Sigma not positive definite at pivot {info}")
-        logdet = 2.0 * np.sum(np.log(np.diag(c)))
-        alpha = cho_solve((c, True), z)
+        if linalg == "ld":
+            Lx, info = ld_linalg.cholesky(S)
+            if info != 0:
+                raise np.linalg.LinAlgError(f"Sigma not positive definite at pivot {info}")
+            logdet = float(ld_linalg.logdet(Lx))
+            Wx = ld_linalg.tri_inv(Lx)
+            alpha = (Wx.T @ (Wx @ z.astype(ld_linalg.LD))).astype(np.float64)
+            Sinv = ld_linalg.wtw(Wx).astype(np.float64)
+            del Lx, Wx
+        elif linalg == "fp64":
+            c, info = dpotrf(S, lower=1, overwrite_a=1, clean=0)
+            if info != 0:
+                raise np.linalg.LinAlgError(f"Sigma not positive definite at pivot {info}")
+            logdet = 2.0 * np.sum(np.log(np.diag(c)))
+            alpha = cho_solve((c, True), z)
+            Sinv, info = dpotri(c, lower=1, overwrite_c=1)  # valid in the lower triangle
+        else:
+            raise ValueError(f"linalg must be 'fp64' or 'ld', got {linalg!r}")
         val = 0.5 * (n * math.log(2.0 * math.pi) + logdet + z @ alpha)
-        Sinv, info = dpotri(c, lower=1, overwrite_c=1)  # valid in the lower triangle
         mult0 = p.l * SQRT_PI * 0.5
 
         def contract(b):

@@ -310,3 +310,103 @@ def test_latent_posterior_against_mpmath_end_to_end():
         vv = 1 + 2 * mp.mpf(p.jitter) - (k.T * Kinv * k)[0]
         assert abs(float(mp.mpf(float(m[q])) - mean)) <= 1e-11 * max(1.0, abs(float(mean)))
         assert abs(float(mp.mpf(float(v[q])) - vv)) <= 1e-11 * max(1.0, abs(float(vv)))
+
+
+# ---- the extended-precision linear algebra the dense factorisation is tested against (oracle/ld_linalg.py) ----------
+def _mp_cholesky(S):
+    """Textbook Cholesky in mpmath (40 digits) with LAPACK's info."""
+    n = len(S)
+    A = [[mp.mpf(float(S[i][j])) for j in range(n)] for i in range(n)]
+    L = [[mp.mpf(0)] * n for _ in range(n)]
+    for j in range(n):
+        d = A[j][j] - mp.fsum(L[j][k] ** 2 for k in range(j))
+        if not d > 0:
+            return L, j + 1
+        L[j][j] = mp.sqrt(d)
+        for i in range(j + 1, n):
+            L[i][j] = (A[i][j] - mp.fsum(L[i][k] * L[j][k] for k in range(j))) / L[j][j]
+    return L, 0
+
+
+def _mp_ld(M):
+    """mpmath matrix -> longdouble array, through decimal strings (no fp64 rounding on the way)."""
+    from oracle import ld_linalg as ld
+    return np.array([[ld.LD(mp.nstr(M[i, j], 30)) for j in range(M.cols)] for i in range(M.rows)])
+
+
+@pytest.mark.parametrize("n", [1, 2, 7, 24])
+def test_ld_linalg_matches_mpmath(n):
+    """Cholesky, triangular inverse, W^T W, log-determinant, solves and the residual helpers of oracle/ld_linalg.py
+    against a 40-digit mpmath evaluation, on an ill-conditioned (cond 1e10) and a graded matrix (rows 2^+-40).  Each
+    longdouble result must be at least 100x closer to the 40-digit value than the fp64 LAPACK / numpy result of the same
+    quantity (or within 1e-17 of its scale): what makes it a reference for fp64 kernels."""
+    from scipy.linalg import lapack, solve_triangular
+    from oracle import ld_linalg as ld
+
+    assert ld.EPS_LD < 1e-18, "np.longdouble is not the 80-bit extended format on this host"
+    rng = np.random.default_rng(n)
+    Q, _ = np.linalg.qr(rng.standard_normal((n, n)))
+    lam = np.logspace(0, -10, n)
+    d = 2.0 ** rng.integers(-40, 40, n)
+    for S in ((Q * lam) @ Q.T, d[:, None] * (np.eye(n) + 0.1 * np.ones((n, n))) * d[None, :]):
+        S = 0.5 * (S + S.T)
+        with mp.workdps(40):
+            Lm, info_m = _mp_cholesky(S)
+            assert info_m == 0
+            Wm = mp.matrix(Lm) ** -1
+            b = rng.standard_normal(n)
+            bm = mp.matrix([mp.mpf(float(v)) for v in b])
+            refs = {"L": _mp_ld(mp.matrix(Lm)), "W": _mp_ld(Wm), "Sinv": _mp_ld(Wm.T * Wm), "x": _mp_ld(Wm * bm),
+                    "xt": _mp_ld(Wm.T * bm)}
+            logdet_ref = ld.LD(mp.nstr(2 * mp.fsum(mp.log(Lm[i][i]) for i in range(n)), 30))
+
+        L, info = ld.cholesky(S, nb=5)   # a block size that does not divide n: every branch of the blocking
+        assert info == 0
+        W = ld.tri_inv(L, nb=5)
+        c, _ = lapack.dpotrf(S, lower=1, clean=1)
+        Wf, _ = lapack.dtrtri(c, lower=1)
+        Sf, _ = lapack.dpotri(c, lower=1)
+        Sf = np.tril(Sf) + np.tril(Sf, -1).T
+        got = {"L": L, "W": W, "Sinv": ld.wtw(W, nb=5), "x": ld.tri_solve(L, b)[:, None],
+               "xt": ld.tri_solve(L, b, trans=True)[:, None]}
+        fp64 = {"L": c, "W": Wf, "Sinv": Sf, "x": solve_triangular(c, b, lower=True)[:, None],
+                "xt": solve_triangular(c, b, lower=True, trans=1)[:, None]}
+        for k, ref in refs.items():
+            rs = np.abs(ref).max(axis=1, keepdims=True)   # per row: graded rows differ by 2^80
+            rs[rs == 0] = 1
+            e_ld = float(np.max(np.abs(got[k] - ref) / rs))
+            e_64 = float(np.max(np.abs(fp64[k].astype(ld.LD) - ref) / rs))
+            assert e_ld <= max(1e-17, 1e-2 * e_64), (k, e_ld, e_64)
+        e_64 = abs(ld.LD(2 * np.sum(np.log(np.diag(c)))) - logdet_ref)
+        assert abs(ld.logdet(L) - logdet_ref) <= max(1e-17 * abs(float(logdet_ref)), 1e-2 * e_64)
+        # residual helpers: the longdouble factor rounded to fp64 has residuals at the fp64 level
+        Lf = np.tril(np.asarray(L, dtype=np.float64))
+        assert ld.componentwise_backward_error(Lf, S, rows=5) < (n + 1) * 2.0 ** -53
+        assert ld.normwise_backward_error(Lf, S, rows=5) < (n + 1) * 2.0 ** -53
+        v = rng.standard_normal((n, 2))
+        assert ld.chol_probe_residual(Lf, S, v, rows=5) < (n + 1) * 2.0 ** -53
+    if n > 1:
+        # exact residuals: L = I against S = I + E e_n e_n^T
+        E = 2.0 ** -30
+        Se = np.eye(n)
+        Se[-1, -1] += E
+        assert ld.componentwise_backward_error(np.eye(n), Se) == E
+        assert ld.normwise_backward_error(np.eye(n), Se) == E / (1 + E)
+        v = np.zeros((n, 1))
+        v[-1] = 1.0
+        assert ld.chol_probe_residual(np.eye(n), Se, v) == E / (1 + E)
+        assert ld.sinv_probe_residual(np.eye(n), Se, v) == E
+    # LAPACK's info: 1-based failing pivot (against mpmath), rows before it final
+    for p in range(n):
+        A = rng.standard_normal((n, n))
+        S = A @ A.T + n * np.eye(n)
+        Lc, info = ld.cholesky(S, nb=5)
+        S[p, p] -= 1.5 * float(Lc[p, p]) ** 2
+        with mp.workdps(40):
+            info_m = _mp_cholesky(S)[1]
+        L, info = ld.cholesky(S, nb=5)
+        assert info == info_m == p + 1
+        assert np.array_equal(L[:p], Lc[:p])
+    Sn = np.eye(n)
+    Sn[n - 1, 0] = np.nan
+    assert ld.cholesky(Sn)[1] == n
