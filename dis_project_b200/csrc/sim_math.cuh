@@ -220,11 +220,13 @@ __device__ __forceinline__ void lfm_kxx_grad_tab(const LfmGrid& g, const LfmPoin
 
 // k_xx between gene point pi = (t, j) and gene point pj = (t', k)  (model.py:197-235):
 //   S_j S_k (sqrt(pi) l / 2) [ h(k, j, t', t) + h(j, k, t, t') ]
+// H1 + H2 is rounded as written (__dadd_rn): contracted into fma(E0, ., H1) it would depend on which point is the row,
+// and k_xx(X*, X*) -- the prior covariance of the gene posterior -- would not be exactly symmetric.
 __device__ __forceinline__ double lfm_kxx(const LfmPoint& pi, const LfmPoint& pj, double l, double inv_l) {
   double H1, H2, u0, u1, u2;
   lfm_h<false>(pj, pi, l, inv_l, H1, u0, u1, u2);  // h(k, j, t', t): a = col gene, b = row gene
   lfm_h<false>(pi, pj, l, inv_l, H2, u0, u1, u2);  // h(j, k, t, t'): a = row gene, b = col gene
-  return pi.s * pj.s * (LFM_SQRT_PI * 0.5 * l) * (H1 + H2);
+  return pi.s * pj.s * (LFM_SQRT_PI * 0.5 * l) * __dadd_rn(H1, H2);
 }
 
 // k_xx and the partials of it with respect to D of the ROW gene, D of the COLUMN gene and l.

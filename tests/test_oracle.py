@@ -153,6 +153,60 @@ def test_gradients_two_derivations():
         assert abs(v1 - o.nlml(o.Params.unpack(o.constrain(u), 1e-4), x, y)) < 1e-11 * abs(v1)
 
 
+def test_gradient_magnitudes_against_dense_derivatives():
+    """nlml_and_grad(magnitudes=True): M_k against the same sums taken over the dense derivative matrices dK/dtheta_k
+    (torch autograd of the kernel, entry by entry) and dmu/dtheta_k; M_k >= |grad_k|; the value and the gradient are
+    the default call's, bit for bit.  Replicates put equal genes at different times, so entries whose row and column
+    are the same gene (one term for the two decay paths) are covered."""
+    import torch
+    for (G, T, R, seed) in ((3, 5, 2, 0), (4, 6, 1, 1)):
+        x, y, var, _ = o.synthetic_problem(G, T, R, seed=seed)
+        p = rand_params(G, seed + 30)
+        p.sigma = 0.8
+        v0, g0 = o.nlml_and_grad(p, x, y, chunk=7)
+        v, g, M = o.nlml_and_grad(p, x, y, chunk=7, magnitudes=True)
+        assert v == v0 and np.array_equal(g, g0)
+        n, P = x.shape[0], 3 * G + 2
+        t = torch.as_tensor(x[:, 0])
+        gi = torch.as_tensor(x[:, 1].astype(np.int64))
+
+        def kern(th):
+            d, s, l = th[:G], th[G:2 * G], th[3 * G]
+
+            def hh(j, k, t1, t2):
+                g_ = d[k] * l / 2
+                return torch.exp(g_ ** 2) / (d[j] + d[k]) * (
+                    torch.exp(-d[k] * (t2 - t1)) * (torch.erf((t2 - t1) / l - g_) + torch.erf(t1 / l + g_))
+                    - torch.exp(-(d[k] * t2 + d[j] * t1)) * (torch.erf(t2 / l - g_) + torch.erf(g_)))
+            j, k, tt, tp = gi[:, None], gi[None, :], t[:, None], t[None, :]
+            return s[j] * s[k] * l * np.sqrt(np.pi) / 2 * (hh(k, j, tp, tt) + hh(j, k, tt, tp))
+
+        def mean(th):
+            return torch.repeat_interleave(th[2 * G:3 * G] / th[:G], n // G)
+
+        th = torch.as_tensor(p.pack())
+        dK = torch.autograd.functional.jacobian(kern, th).numpy()      # (n, n, P)
+        dmu = torch.autograd.functional.jacobian(mean, th).numpy()     # (n, P)
+        S = o.sigma_matrix(p, x)
+        Sinv = np.linalg.inv(S)
+        alpha = np.linalg.solve(S, y - o.mean_function(p, x))
+        Kbar = 0.5 * (Sinv - np.outer(alpha, alpha))
+        ref = np.abs(Kbar[:, :, None] * dK).sum(axis=(0, 1)) + np.abs(alpha[:, None] * dmu).sum(axis=0)
+        ref[P - 1] = p.sigma * (np.abs(np.diag(Sinv)).sum() + alpha @ alpha)
+        gref = (Kbar[:, :, None] * dK).sum(axis=(0, 1)) - alpha @ dmu
+        gref[P - 1] = 2 * p.sigma * np.trace(Kbar)
+        # the closed-form partials and autograd round each entry's derivative differently: 1.2e-12 of M_k measured
+        assert np.max(np.abs(g - gref) / ref) < 1e-10           # the brute force computes the same gradient
+        assert np.max(np.abs(M - ref) / ref) < 1e-10, (M, ref)
+        assert np.all(M >= np.abs(g))
+        assert np.min(M / np.abs(g)) < 10.0                      # a scale of the component, not of the whole gradient
+        # unconstrained: the chain rule scales each term by the bijector's derivative
+        u = o.unconstrain(p.pack())
+        vu, gu = o.nlml_and_grad_unc(u, x, y, p.jitter)
+        _, gc, Mc = o.nlml_and_grad(o.Params.unpack(o.constrain(u), p.jitter), x, y, magnitudes=True)
+        assert np.array_equal(gu, gc * o.constrain_jac(u)) and np.all(Mc * np.abs(o.constrain_jac(u)) >= np.abs(gu))
+
+
 def test_heteroscedastic_objective_two_derivations():
     """sigma_matrix(variances=...): the GPyTorch twin's training convention (measurement variances on the diagonal,
     src/gpytorch_alfi/model_alfi.py:294-299).  Closed-form gradient against torch autograd of the literal expressions;
