@@ -231,7 +231,8 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
         }
         __syncthreads();
         const double p = piv;
-        if (tid == 0 && !(p > 0.0) && fail == 0) fail = k + 1;
+        // pivots below DBL_MIN fail too, as in the warp and team kernels, whose ftz reciprocals cannot take them
+        if (tid == 0 && !(p >= 0x1p-1022) && fail == 0) fail = k + 1;
         if (row >= k && row < U && half == 0) {
           const double dk = sqrt(p);
           S[row * ld + k] = (row == k) ? dk : v / dk;
@@ -427,9 +428,9 @@ __global__ void __launch_bounds__(BT, (BT == 128) ? 4 : 2) lfm_batched_kernel(Ba
       a.theta_out[bidx * P + tid] = t;
     }
   }
-  if (tid == 0 && a.info) {
+  if (tid == 0 && a.info) {   // a later chunk keeps the first failure (its NaN iterate fails again, at another pivot)
     if (a.first_step == 0 || eval_only) a.info[bidx] = fail;
-    else if (fail) a.info[bidx] = fail;
+    else if (fail && a.info[bidx] == 0) a.info[bidx] = fail;
   }
   if (tid == 0 && a.best_key && !eval_only && a.hist && a.steps > 0) {
     const double v = a.hist[bidx * a.ld_hist + a.first_step + a.steps - 1];

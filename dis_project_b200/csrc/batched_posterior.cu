@@ -190,7 +190,7 @@ __global__ void __launch_bounds__(BPOST_BT) lfm_batched_posterior_kernel(BPostAr
     }
     __syncthreads();
     const double pk = piv;
-    if (tid == 0 && !(pk > 0.0) && fail == 0) fail = k + 1;
+    if (tid == 0 && !(pk >= 0x1p-1022) && fail == 0) fail = k + 1;   // below DBL_MIN fails: the rule of every batched kernel
     if (tid >= k && tid < U) {
       const double dk = sqrt(pk);
       S[tid * ld + k] = (tid == k) ? dk : v / dk;

@@ -28,7 +28,8 @@ __device__ __forceinline__ void wpair_decode(int p, int& r, int& c) {
   while (r * (r + 1) / 2 > p) --r;
   c = p - r * (r + 1) / 2;
 }
-// 1/sqrt(x) for x > 0 normal: MUFU.RSQ64H seed + one third-order step (branch free)
+// 1/sqrt(x) for x >= DBL_MIN: MUFU.RSQ64H seed + one third-order step (branch free).  The ftz seed flushes a subnormal
+// x to zero and the step turns the infinite seed into NaN: the pivot tests therefore fail every pivot below DBL_MIN.
 __device__ __forceinline__ double w_rsqrt(double x) {
   double y0;
   asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y0) : "d"(x));
@@ -94,7 +95,8 @@ template <int NW> __device__ __forceinline__ void tsum2(double& v0, double& v1, 
 #pragma unroll
   for (int w = 1; w < NW; ++w) { v0 += r[w]; v1 += r[NW + w]; }
 }
-// 1/x for x > 0 normal: MUFU.RCP64H seed + two Newton steps (branch free; on the pivot chain of the sweep)
+// 1/x for x >= DBL_MIN: MUFU.RCP64H seed + two Newton steps (branch free; on the pivot chain of the sweep, whose pivot
+// test fails every pivot below DBL_MIN, which the ftz seed would flush to zero)
 __device__ __forceinline__ double w_rcp(double x) {
   double y0;
   asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y0) : "d"(x));
@@ -891,7 +893,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       double akk = __shfl_sync(0xffffffffu, am[0], 0);
 #pragma unroll
       for (int k = 0; k < 32; ++k) {
-        if (!(akk > 0.0) && fail == 0) fail = ex + k + 1;
+        if (!(akk >= 0x1p-1022) && fail == 0) fail = ex + k + 1;
         const double rk = w_rsqrt(akk);
         const double lik = (lane == k) ? akk * rk : am[k] * rk;
         double akk_next = 0.0;
@@ -978,7 +980,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
 #pragma unroll
         for (int k = 0; k < WEX; ++k) {
           const double piv = s11[k][k];
-          if (k < ex && !(piv > 0.0) && fail == 0) fail = k + 1;
+          if (k < ex && !(piv >= 0x1p-1022) && fail == 0) fail = k + 1;
           const double rkk = w_rsqrt(piv);
           rd[k] = rkk;
           if (k < ex) rprod *= rkk;
@@ -1115,7 +1117,7 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
             }
             asm volatile("bar.sync 1, %0;" ::"n"(SWEEP_THREADS) : "memory");
             const double d = ring[par * GJN + k];
-            if (!(d > 0.0) && fail == 0) fail = k + 1;
+            if (!(d >= 0x1p-1022) && fail == 0) fail = k + 1;
             if (tid == k) mypiv = d;
             if (active) {
               const double pinv = w_rcp(d);
@@ -1410,9 +1412,9 @@ __global__ void __launch_bounds__(32 * NW, NW == 1 ? 1 : (NW <= 4 ? 4 : 2)) lfm_
       }
     }
   }
-  if (tid == 0 && a.info) {
+  if (tid == 0 && a.info) {   // a later chunk keeps the first failure (its NaN iterate fails again, at another pivot)
     if (first_step == 0 || eval_only) a.info[bidx] = fail;
-    else if (fail) a.info[bidx] = fail;
+    else if (fail && __ldcg(a.info + bidx) == 0) a.info[bidx] = fail;
   }
   // (queue mode: the launch covers the whole fit, so "after the launch's last step" is the task that reaches total_steps)
   if (tid == 0 && a.best_key && !eval_only && a.hist && task_steps > 0 && (!a.queue || first_step + task_steps >= a.total_steps)) {

@@ -163,6 +163,16 @@ int lfm_gene_posterior(lfm_stream_t stream, int64_t N, int G, const double* X, c
 
 /* ---- batched multi-start path (many independent small LFMs per GPU) -------------------------- */
 
+/* `info` of the batched NLML, fit and posterior entry points, per LFM: 0 = ok, k > 0 = the 1-based failing pivot of the
+ * compressed matrix M = diag(cbar) + R K_u (below), whose rows are the unique rows of X in order of first occurrence.
+ * A pivot fails when it is not >= DBL_MIN (2^-1022): NaN, zero, negative, and -- the one deviation from LAPACK, as in the
+ * dense factorisation -- positive subnormal pivots, which the warp and team kernels' ftz reciprocals cannot take.  The
+ * failing pivot is LAPACK's dpotrf index on M, except in the one-warp-per-LFM kernel at 33 <= U <= 36: it factorises
+ * the trailing U - ex rows M22 first (ex = U - 32) and then the Schur complement S11 of the ex leading rows, and reports
+ * pivot k of M22 as ex + k + 1 and pivot k of S11 as k + 1.  That numbering is kept rather than reordered: every caller
+ * only tests info != 0, and LAPACK's order would need another row-to-lane mapping in the hot kernel.  A fit split over
+ * several calls keeps the info of its first failure.  The outputs of a failed LFM are NaN. */
+
 /* Rows of the duplicate-row-compressed problem for a HOST copy of X: the number of distinct rows when every distinct
  * (time, gene, flag) row occurs the same number of times R > 1 (the p53 layout repeats each row once per replicate),
  * else N -- the batched kernels compress only uniform multiplicities, and this mirrors their rule.  Passing it as

@@ -486,11 +486,16 @@ def nlml_and_grad(p: Params, x: np.ndarray, y: np.ndarray, *, chunk: int = 256, 
     return float(val), grad, np.concatenate([md, ms, mb, [ml, msig]])
 
 
-def nlml_and_grad_unc(theta_unc: np.ndarray, x, y, jitter: float, variances=None):
-    """value_and_grad of JaxTrainer.loss w.r.t. the UNCONSTRAINED leaves (trainer.py:86-131)."""
+def nlml_and_grad_unc(theta_unc: np.ndarray, x, y, jitter: float, variances=None, *, linalg: str = "fp64",
+                      magnitudes: bool = False):
+    """value_and_grad of JaxTrainer.loss w.r.t. the UNCONSTRAINED leaves (trainer.py:86-131).  `linalg` and
+    `magnitudes` as nlml_and_grad; the magnitudes are chained as M_k |d theta_k / d u_k|."""
     theta = constrain(theta_unc)
-    val, g = nlml_and_grad(Params.unpack(theta, jitter), x, y, variances=variances)
-    return val, g * constrain_jac(theta_unc)
+    out = nlml_and_grad(Params.unpack(theta, jitter), x, y, variances=variances, linalg=linalg, magnitudes=magnitudes)
+    jac = constrain_jac(theta_unc)
+    if magnitudes:
+        return out[0], out[1] * jac, out[2] * np.abs(jac)
+    return out[0], out[1] * jac
 
 
 # --------------------------------------------------------------------------- #

@@ -95,7 +95,7 @@ def compressed_het(p, x, y, var):
     gl = np.sum(w * (dH1_dl + dH2_dl)) + np.sum(W * Ku) / p.l
     asum = alpha.reshape(G, N // G).sum(axis=1)
     grad = np.concatenate([gd + asum * p.b / p.d**2, gs, -asum / p.d, [gl, p.sigma * (trS - alpha @ alpha)]])
-    return val, grad, dict(Pt=Pt, beta=beta, W=W, sens=sens, Ku=Ku, alpha=alpha, trS=trS)
+    return val, grad, dict(Pt=Pt, beta=beta, W=W, sens=sens, Ku=Ku, alpha=alpha, trS=trS, M=M, q=q, cbar=cbar, R=R)
 
 
 @pytest.mark.parametrize("design", ["R1", "R3", "non_uniform", "zero_variances"])
