@@ -53,19 +53,10 @@ SIGNATURES = {
     "lfm_mean_function": (_int, [_ptr, _i64, _ptr, _int, _ptr, _ptr]),
     "lfm_constrain": (_int, [_ptr, _i64, _int, _ptr, _ptr]),
     "lfm_unconstrain": (_int, [_ptr, _i64, _int, _ptr, _ptr]),
-    "lfm_nlml_workspace_bytes": (_sz, [_i64, _int]),
-    "lfm_nlml": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _dbl, _ptr, _sz, _ptr, _ptr]),
-    "lfm_nlml_grad": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _dbl, _ptr, _sz, _ptr, _ptr]),
-    "lfm_nlml_grad_unc": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _dbl, _ptr, _sz, _ptr, _ptr]),
     "lfm_count_distinct_times": (_i64, [_i64, _ptr]),
-    "lfm_nlml_grad_plan_create": (_int, [C.POINTER(C.c_void_p), _i64, _int, _ptr, _ptr, _ptr, _dbl, _i64, _int, _ptr, _sz,
-                                         _ptr, _ptr]),
     "lfm_plan_launch": (_int, [_ptr, _ptr]),
     "lfm_plan_destroy": (_int, [_ptr]),
     "lfm_nlml_workspace_bytes_tg": (_sz, [_i64, _int, _i64]),
-    "lfm_nlml_tg": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _sz, _ptr, _ptr]),
-    "lfm_nlml_grad_tg": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _sz, _ptr, _ptr]),
-    "lfm_nlml_grad_unc_tg": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _sz, _ptr, _ptr]),
     "lfm_nlml_het_tg": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _sz, _ptr, _ptr]),
     "lfm_nlml_grad_het_tg": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _sz, _ptr, _ptr]),
     "lfm_nlml_grad_unc_het_tg": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _sz, _ptr, _ptr]),
@@ -79,22 +70,8 @@ SIGNATURES = {
     "lfm_gene_posterior": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _ptr, _sz,
                                   _ptr, _ptr, _ptr, _ptr]),
     "lfm_count_unique_rows": (_int, [_i64, _ptr]),
-    "lfm_batched_nlml_grad_unc": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _dbl, _int, _ptr, _ptr, _ptr]),
-    "lfm_batched_fit": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
-                               _int, _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr]),
-    "lfm_batched_nlml_grad_unc_tg": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _dbl, _int, _int, _ptr, _ptr, _ptr]),
-    "lfm_batched_fit_tg": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
-                                  _int, _int, _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr, _ptr, _ptr]),
-    "lfm_batched_nlml_grad_unc_multi": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _dbl, _int, _int, _ptr, _ptr,
-                                               _ptr]),
-    "lfm_batched_fit_multi": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
-                                     _int, _int, _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr, _ptr, _ptr]),
-    "lfm_batched_fit_trace": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
-                                     _int, _int, _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _ptr]),
     "lfm_batched_fit_init": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _ptr, _i64, _ptr, _ptr, _i64]),
     "lfm_batched_queue_bytes": (_sz, [_i64, _int, _int]),
-    "lfm_batched_fit_queue": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
-                                     _int, _int, _int, _int, _int, _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _ptr, _int, _ptr, _sz]),
     "lfm_batched_nlml_grad_unc_het": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _dbl, _int, _int,
                                              _ptr, _ptr, _ptr]),
     "lfm_batched_fit_het": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl,
@@ -121,8 +98,6 @@ SIGNATURES = {
     "lfm_nlml_grad_host": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _dbl, _int, _ptr, _ptr]),
     "lfm_latent_posterior_host": (_int, [_ptr, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _i64, _ptr, _ptr,
                                          _ptr, _ptr]),
-    "lfm_batched_fit_host": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
-                                    _int, _int, _int, _ptr, _ptr, _ptr]),
     "lfm_batched_fit_het_host": (_int, [_ptr, _i64, _i64, _int, _ptr, _ptr, _ptr, _ptr, _dbl, _dbl, _dbl, _dbl, _dbl,
                                         _int, _int, _int, _ptr, _ptr, _ptr]),
     "lfm_debug_leaf_profile": (_int, [_ptr, _ptr, _ptr, _ptr, _ptr]),

@@ -500,47 +500,7 @@ extern "C" int lfm_batched_nlml_grad_unc_het(lfm_stream_t stream, int64_t B, int
   if (N > 128) return LFM_ERR_UNSUPPORTED;
   return batched_launch((cudaStream_t)stream, a, time_grid_hint);
 }
-extern "C" int lfm_batched_nlml_grad_unc_multi(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
-                                               const double* y, int64_t y_stride, const double* theta_unc, double jitter,
-                                               int unique_rows_hint, int time_grid_hint, double* out_val,
-                                               double* out_grad, int* info) {
-  return lfm_batched_nlml_grad_unc_het(stream, B, N, G, X, y, y_stride, nullptr, 0, theta_unc, jitter, unique_rows_hint,
-                                       time_grid_hint, out_val, out_grad, info);
-}
-extern "C" int lfm_batched_nlml_grad_unc_tg(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
-                                            const double* y, const double* theta_unc, double jitter,
-                                            int unique_rows_hint, int time_grid_hint, double* out_val,
-                                            double* out_grad, int* info) {
-  return lfm_batched_nlml_grad_unc_multi(stream, B, N, G, X, y, 0, theta_unc, jitter, unique_rows_hint, time_grid_hint,
-                                         out_val, out_grad, info);
-}
-extern "C" int lfm_batched_nlml_grad_unc(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
-                                         const double* y, const double* theta_unc, double jitter,
-                                         int unique_rows_hint, double* out_val, double* out_grad, int* info) {
-  return lfm_batched_nlml_grad_unc_tg(stream, B, N, G, X, y, theta_unc, jitter, unique_rows_hint, 0, out_val, out_grad,
-                                      info);
-}
 
-extern "C" int lfm_batched_fit_tg(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                                  double* theta_unc_io, double* adam_state, double jitter, double lr, double b1,
-                                  double b2, double eps, int first_step, int steps, int total_steps, int fix_params,
-                                  int steps_per_epoch, int unique_rows_hint, int time_grid_hint, double* out_hist,
-                                  int64_t ld_hist, double* out_theta, int* info, long long* best_key,
-                                  void* structure_cache) {
-  return lfm_batched_fit_multi(stream, B, N, G, X, y, 0, theta_unc_io, adam_state, jitter, lr, b1, b2, eps, first_step,
-                               steps, total_steps, fix_params, steps_per_epoch, unique_rows_hint, time_grid_hint,
-                               out_hist, ld_hist, out_theta, info, best_key, structure_cache);
-}
-extern "C" int lfm_batched_fit_multi(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                                     int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter,
-                                     double lr, double b1, double b2, double eps, int first_step, int steps,
-                                     int total_steps, int fix_params, int steps_per_epoch, int unique_rows_hint,
-                                     int time_grid_hint, double* out_hist, int64_t ld_hist, double* out_theta,
-                                     int* info, long long* best_key, void* structure_cache) {
-  return lfm_batched_fit_trace(stream, B, N, G, X, y, y_stride, theta_unc_io, adam_state, jitter, lr, b1, b2, eps,
-                               first_step, steps, total_steps, fix_params, steps_per_epoch, unique_rows_hint,
-                               time_grid_hint, out_hist, ld_hist, out_theta, info, best_key, nullptr, structure_cache);
-}
 // Whole fit in ONE launch with persistent workers and a device-side task queue (batched_warp.cu): see the header.
 extern "C" size_t lfm_batched_queue_bytes(int64_t B, int total_steps, int chunk_steps) {
   if (B <= 0 || total_steps <= 0 || chunk_steps <= 0) return 0;
@@ -574,30 +534,6 @@ extern "C" int lfm_batched_fit_het(lfm_stream_t stream, int64_t B, int64_t N, in
   if (queue_ws) { a.queue = (int*)queue_ws; a.queue_chunk = chunk_steps; }
   a.var = variances; a.var_stride = variances ? var_stride : 0;
   return batched_launch((cudaStream_t)stream, a, time_grid_hint);
-}
-extern "C" int lfm_batched_fit_queue(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                                     int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter,
-                                     double lr, double b1, double b2, double eps, int total_steps, int fix_params,
-                                     int steps_per_epoch, int unique_rows_hint, int time_grid_hint, double* out_hist,
-                                     int64_t ld_hist, double* out_theta, int* info, long long* best_key,
-                                     long long* step_keys, void* structure_cache, int chunk_steps, void* queue_ws,
-                                     size_t queue_bytes) {
-  if (total_steps < 0) return LFM_ERR_INVALID;
-  return lfm_batched_fit_het(stream, B, N, G, X, y, y_stride, nullptr, 0, theta_unc_io, adam_state, jitter, lr, b1, b2,
-                             eps, 0, total_steps, total_steps, fix_params, steps_per_epoch, unique_rows_hint,
-                             time_grid_hint, out_hist, ld_hist, out_theta, info, best_key, step_keys, structure_cache,
-                             chunk_steps, queue_ws, queue_bytes);
-}
-extern "C" int lfm_batched_fit_trace(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                                     int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter,
-                                     double lr, double b1, double b2, double eps, int first_step, int steps,
-                                     int total_steps, int fix_params, int steps_per_epoch, int unique_rows_hint,
-                                     int time_grid_hint, double* out_hist, int64_t ld_hist, double* out_theta,
-                                     int* info, long long* best_key, long long* step_keys, void* structure_cache) {
-  return lfm_batched_fit_het(stream, B, N, G, X, y, y_stride, nullptr, 0, theta_unc_io, adam_state, jitter, lr, b1, b2,
-                             eps, first_step, steps, total_steps, fix_params, steps_per_epoch, unique_rows_hint,
-                             time_grid_hint, out_hist, ld_hist, out_theta, info, best_key, step_keys, structure_cache, 0,
-                             nullptr, 0);
 }
 // Debug: one launch of `steps` >= 2 steps with clock64 stamps at the phase boundaries of the SECOND step of LFM 0
 // (warp-per-LFM kernel only): A B C D E[load] E[routine] E[W^T W] E[Schur] E[store] F I J K end.
@@ -665,16 +601,6 @@ extern "C" size_t lfm_batched_structure_bytes(int64_t N, int G, int unique_rows_
   int MU = unique_rows_hint;
   if (MU <= 0 || MU > N) MU = (int)N;
   return lfm_batched_warp_structure_bytes((int)N, G, MU, time_grid_hint);
-}
-
-extern "C" int lfm_batched_fit(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                               double* theta_unc_io, double* adam_state, double jitter, double lr, double b1,
-                               double b2, double eps, int first_step, int steps, int total_steps, int fix_params,
-                               int steps_per_epoch, int unique_rows_hint, double* out_hist, int64_t ld_hist,
-                               double* out_theta, int* info) {
-  return lfm_batched_fit_tg(stream, B, N, G, X, y, theta_unc_io, adam_state, jitter, lr, b1, b2, eps, first_step, steps,
-                            total_steps, fix_params, steps_per_epoch, unique_rows_hint, 0, out_hist, ld_hist, out_theta,
-                            info, nullptr, nullptr);
 }
 
 // Number of rows of the duplicate-row-compressed problem for a HOST copy of X: the `unique_rows_hint` that

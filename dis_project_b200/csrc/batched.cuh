@@ -21,7 +21,7 @@ struct BatchedArgs {
   int max_unique;
   long long* stamps;   // debug (lfm_debug_batched_stamps): clock64 at the phase boundaries of the first step of LFM 0
   void* struct_cache;  // NULL or lfm_batched_structure_bytes() device bytes kept by the caller between the launches of a fit
-  int* queue;           // NULL or lfm_batched_queue_bytes() device bytes, initialised by lfm_batched_fit_queue: persistent workers + task queue
+  int* queue;           // NULL or lfm_batched_queue_bytes() device bytes, initialised by lfm_batched_fit_het: persistent workers + task queue
   int queue_chunk;      // steps per task in queue mode
   long long* step_keys; // NULL or total_steps device words: word s receives atomicMin of lfm_loss_key(loss at step s) over the batch
   long long* best_key; // NULL or one device word: atomicMin of lfm_loss_key(loss after the launch's last step) over the batch     // shared-memory matrix is sized for this many unique rows (N when unknown)

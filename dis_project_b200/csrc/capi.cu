@@ -107,12 +107,6 @@ extern "C" int lfm_nlml_grad_plan_create_het(lfm_plan** out_plan, int64_t N, int
   *out_plan = p;
   return LFM_OK;
 }
-extern "C" int lfm_nlml_grad_plan_create(lfm_plan** out_plan, int64_t N, int G, const double* X, const double* y,
-                                         const double* theta, double jitter, int64_t time_grid, int unconstrained,
-                                         void* ws, size_t ws_bytes, double* out, int* info) {
-  return lfm_nlml_grad_plan_create_het(out_plan, N, G, X, y, nullptr, theta, jitter, time_grid, unconstrained, ws,
-                                       ws_bytes, out, info);
-}
 extern "C" int lfm_plan_launch(lfm_plan* p, lfm_stream_t stream) {
   if (!p || !p->exec) return LFM_ERR_INVALID;
   LFM_CUDA_OK(cudaGraphLaunch(p->exec, (cudaStream_t)stream));
@@ -188,7 +182,7 @@ extern "C" int lfm_handle_destroy(lfm_handle* h) {
 
 static size_t r2(size_t n) { return (n + 1) & ~(size_t)1; }
 
-// every training row must carry flag 1 (include/lfm_b200.h, lfm_nlml): checked where a host copy is at hand
+// every training row must carry flag 1 (include/lfm_b200.h, section (b,c)): checked where a host copy is at hand
 static bool training_flags_ok(int64_t N, const double* X) {
   for (int64_t i = 0; i < N; ++i)
     if (X[3 * i + 2] != 1.0) return false;
@@ -343,11 +337,4 @@ extern "C" int lfm_batched_fit_het_host(lfm_handle* h, int64_t B, int64_t N, int
   }
   if (B > 4096) cudaFree(dinfo);
   return st;
-}
-extern "C" int lfm_batched_fit_host(lfm_handle* h, int64_t B, int64_t N, int G, const double* X, const double* y,
-                                    const double* theta0, double jitter, double lr, double b1, double b2,
-                                    double eps, int steps, int fix_params, int steps_per_epoch, double* out_theta,
-                                    double* out_hist, int* info) {
-  return lfm_batched_fit_het_host(h, B, N, G, X, y, nullptr, theta0, jitter, lr, b1, b2, eps, steps, fix_params,
-                                  steps_per_epoch, out_theta, out_hist, info);
 }

@@ -105,11 +105,11 @@ ffi::Error BatchedFit(cudaStream_t stream, F64 X, F64 y, F64 theta_unc_in, F64 a
   }
   // y is (N,) -- every LFM fits the same observations -- or (B, N): one row per LFM
   const int64_t y_stride = y.dimensions().size() == 2 ? N : 0;
-  return status(lfm_batched_fit_multi(stream, B, N, (int)G, X.typed_data(), y.typed_data(), y_stride,
-                                      theta_unc->typed_data(), adam->typed_data(), jitter, lr, b1, b2, eps, 0,
-                                      (int)steps, (int)steps, (int)fix_params, (int)steps_per_epoch, (int)unique_rows,
-                                      (int)time_grid, hist->typed_data(), steps, theta->typed_data(), info->typed_data(),
-                                      nullptr, nullptr));
+  return status(lfm_batched_fit_het(stream, B, N, (int)G, X.typed_data(), y.typed_data(), y_stride, nullptr, 0,
+                                    theta_unc->typed_data(), adam->typed_data(), jitter, lr, b1, b2, eps, 0, (int)steps,
+                                    (int)steps, (int)fix_params, (int)steps_per_epoch, (int)unique_rows, (int)time_grid,
+                                    hist->typed_data(), steps, theta->typed_data(), info->typed_data(), nullptr,
+                                    nullptr, nullptr, 0, nullptr, 0));
 }
 
 }  // namespace

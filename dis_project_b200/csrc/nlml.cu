@@ -276,7 +276,6 @@ extern "C" size_t lfm_nlml_workspace_bytes_tg(int64_t N, int G, int64_t time_gri
   if (N <= 0 || G <= 0) return 0;
   return nlml_ws_layout(N, G, time_grid, nullptr).total_doubles * sizeof(double);
 }
-extern "C" size_t lfm_nlml_workspace_bytes(int64_t N, int G) { return lfm_nlml_workspace_bytes_tg(N, G, 0); }
 
 static int check_common(int64_t N, int G, const void* X, const void* y, const void* theta, int64_t time_grid, void* ws,
                         size_t ws_bytes, void* out, void* info) {
@@ -326,15 +325,6 @@ extern "C" int lfm_nlml_het_tg(lfm_stream_t stream, int64_t N, int G, const doub
   LFM_LAUNCHED(1);
   LFM_CUDA_OK(cudaGetLastError());
   return LFM_OK;
-}
-extern "C" int lfm_nlml_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                           const double* theta, double jitter, int64_t time_grid, void* ws, size_t ws_bytes,
-                           double* out, int* info) {
-  return lfm_nlml_het_tg(stream, N, G, X, y, nullptr, theta, jitter, time_grid, ws, ws_bytes, out, info);
-}
-extern "C" int lfm_nlml(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                        const double* theta, double jitter, void* ws, size_t ws_bytes, double* out, int* info) {
-  return lfm_nlml_tg(stream, N, G, X, y, theta, jitter, 0, ws, ws_bytes, out, info);
 }
 
 // Side stream of an evaluation: w = W z, alpha = W^T w and the NLML reduction only read W, z and the diagonal of L,
@@ -400,22 +390,7 @@ extern "C" int lfm_nlml_grad_het_tg(lfm_stream_t stream, int64_t N, int G, const
   const NlmlWs s = nlml_ws_layout(N, G, time_grid, ws);
   return nlml_grad_impl((cudaStream_t)stream, N, G, X, y, variances, theta, jitter, s, out, info);
 }
-extern "C" int lfm_nlml_grad_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                                const double* theta, double jitter, int64_t time_grid, void* ws, size_t ws_bytes,
-                                double* out, int* info) {
-  return lfm_nlml_grad_het_tg(stream, N, G, X, y, nullptr, theta, jitter, time_grid, ws, ws_bytes, out, info);
-}
-extern "C" int lfm_nlml_grad(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                             const double* theta, double jitter, void* ws, size_t ws_bytes, double* out,
-                             int* info) {
-  return lfm_nlml_grad_tg(stream, N, G, X, y, theta, jitter, 0, ws, ws_bytes, out, info);
-}
 
-extern "C" int lfm_nlml_grad_unc_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                                    const double* theta_unc, double jitter, int64_t time_grid, void* ws,
-                                    size_t ws_bytes, double* out, int* info) {
-  return lfm_nlml_grad_unc_het_tg(stream, N, G, X, y, nullptr, theta_unc, jitter, time_grid, ws, ws_bytes, out, info);
-}
 extern "C" int lfm_nlml_grad_unc_het_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
                                         const double* variances, const double* theta_unc, double jitter,
                                         int64_t time_grid, void* ws, size_t ws_bytes, double* out, int* info) {
@@ -431,11 +406,6 @@ extern "C" int lfm_nlml_grad_unc_het_tg(lfm_stream_t stream, int64_t N, int G, c
   LFM_LAUNCHED(1);
   LFM_CUDA_OK(cudaGetLastError());
   return LFM_OK;
-}
-extern "C" int lfm_nlml_grad_unc(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                                 const double* theta_unc, double jitter, void* ws, size_t ws_bytes,
-                                 double* out, int* info) {
-  return lfm_nlml_grad_unc_tg(stream, N, G, X, y, theta_unc, jitter, 0, ws, ws_bytes, out, info);
 }
 
 extern "C" int lfm_constrain(lfm_stream_t stream, int64_t B, int G, const double* theta_unc, double* theta) {

@@ -41,7 +41,7 @@ def _rows3(X: torch.Tensor, name: str) -> torch.Tensor:
 def _check_training_flags(X) -> None:
     """The training covariance Sigma is built from k_xx only (every training row of the reference has flag 1,
     dataset.py:388; objectives.py:70 would blend the other branches in for flag-0 rows).  A host copy of X is checked
-    here; a device-resident X is the caller's responsibility (include/lfm_b200.h, lfm_nlml)."""
+    here; a device-resident X is the caller's responsibility (include/lfm_b200.h, section (b,c))."""
     if isinstance(X, torch.Tensor):
         if X.is_cuda or X.ndim != 2 or X.shape[1] != 3:
             return
@@ -404,16 +404,11 @@ def batched_nlml_grad_unc(X, y, theta_unc, jitter: float, G: int, time_grid: Opt
     info = torch.zeros(B, dtype=torch.int32, device=X.device)
     if B == 0:
         return val, grad, info
-    if v is not None:
-        _lib.check(_lib.lib().lfm_batched_nlml_grad_unc_het(_stream(), B, N, G, X.data_ptr(), y.data_ptr(), y_stride,
-                                                            v.data_ptr(), v_stride, u.data_ptr(), float(jitter), hint, tg,
-                                                            val.data_ptr(), grad.data_ptr(), info.data_ptr()),
-                   "lfm_batched_nlml_grad_unc_het")
-        return val, grad, info
-    _lib.check(_lib.lib().lfm_batched_nlml_grad_unc_multi(_stream(), B, N, G, X.data_ptr(), y.data_ptr(), y_stride,
-                                                          u.data_ptr(), float(jitter), hint, tg, val.data_ptr(),
-                                                          grad.data_ptr(), info.data_ptr()),
-               "lfm_batched_nlml_grad_unc_multi")
+    _lib.check(_lib.lib().lfm_batched_nlml_grad_unc_het(_stream(), B, N, G, X.data_ptr(), y.data_ptr(), y_stride,
+                                                        v.data_ptr() if v is not None else None, v_stride, u.data_ptr(),
+                                                        float(jitter), hint, tg, val.data_ptr(), grad.data_ptr(),
+                                                        info.data_ptr()),
+               "lfm_batched_nlml_grad_unc_het")
     return val, grad, info
 
 

@@ -44,7 +44,7 @@ typedef enum lfm_status {
   LFM_ERR_COMM = -6         /* NCCL is not loadable on this host, or an NCCL call failed          */
 } lfm_status;
 
-#define LFM_ABI_VERSION 2
+#define LFM_ABI_VERSION 3
 
 int lfm_abi_version(void);
 const char* lfm_status_string(int status);
@@ -77,63 +77,42 @@ int lfm_mean_function(lfm_stream_t stream, int64_t N, const double* X, int G, co
 int lfm_constrain(lfm_stream_t stream, int64_t B, int G, const double* theta_unc, double* theta);
 int lfm_unconstrain(lfm_stream_t stream, int64_t B, int G, const double* theta, double* theta_unc);
 
-/* ---- (b,c) objective and its gradient ------------------------------------------------------- */
-
-size_t lfm_nlml_workspace_bytes(int64_t N, int G);
-
-/* CustomConjMLL(negative=True)(model, Dataset(X, y)) (src/objectives.py:21-78):
- * Sigma = K + jitter I + sigma^2 I; out[0] = 1/2 [N log 2pi + log det Sigma + z^T Sigma^-1 z].
+/* ---- (b,c) objective and its gradient -------------------------------------------------------
+ * Sigma = K + diag(variances) + jitter I + sigma^2 I.  `variances` is N device doubles or NULL.  NULL is the
+ * reference's objective, CustomConjMLL(negative=True) (src/objectives.py:21-78).  Variances put the measurement
+ * variances of dataset_3d (src/dataset.py:396-397) inside the training covariance, the convention of the reference's
+ * GPyTorch twin when it trains (src/gpytorch_alfi/model_alfi.py:294-299: K_xx += 1e-4 I; K_xx += self.variance).  The
+ * gradient formulas do not change (d Sigma / d theta has no variance term); only the diagonal tiles of the Sigma build
+ * read `variances`.
+ *
  * TRAINING ROWS MUST ALL CARRY FLAG 1: Sigma is built from k_xx alone (every training row of the reference has flag
  * 1, src/dataset.py:388); for a flag-0 row objectives.py:70 would blend k_xf / k_ff in, which this path (and the
  * posteriors' training covariance, and the batched fits) does not do.  The *_host entry points and the Python layer
- * reject such X (LFM_ERR_UNSUPPORTED / ValueError); device-pointer callers are trusted. */
-int lfm_nlml(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-             const double* theta, double jitter, void* ws, size_t ws_bytes, double* out, int* info);
-
-/* jax.value_and_grad(JaxTrainer.loss) (src/trainer.py:86-103,126) in CONSTRAINED coordinates:
- * out[0] = NLML, out[1..P] = dNLML/dtheta.  dK/dtheta blocks are contracted with
- * K_bar = 1/2 (Sigma^-1 - alpha alpha^T) on the fly and never materialised. */
-int lfm_nlml_grad(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                  const double* theta, double jitter, void* ws, size_t ws_bytes, double* out, int* info);
-
-/* Same, differentiated w.r.t. the UNCONSTRAINED leaves -- the exact quantity the optimiser in
- * src/trainer.py:126-128 consumes.  out[0] = NLML, out[1..P] = gradient. */
-int lfm_nlml_grad_unc(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                      const double* theta_unc, double jitter, void* ws, size_t ws_bytes, double* out,
-                      int* info);
-
-/* ---- time-grid variants ----------------------------------------------------------------------
- * `time_grid` is an upper bound on the number of DISTINCT times among the rows of X (0 = unknown;
- * lfm_count_distinct_times gives it from a host copy).  The reference's layout observes every gene on
- * the same few time points (src/dataset.py:380-391), and the exp/erf factors of h (src/model.py:315-365)
- * depend on (gene, t, t') only: when the bound is small the library finds the distinct times on the
- * device, tabulates those factors once per evaluation (G T^2 entries instead of N^2) and builds Sigma
- * and the dK/dtheta contraction from the tables.  The tables hold the very values the direct path
- * computes; results agree to rounding.  If X has more distinct times than the bound, the kernels
- * detect it on the device and evaluate directly.  The plain entry points above are time_grid = 0. */
+ * reject such X (LFM_ERR_UNSUPPORTED / ValueError); device-pointer callers are trusted.
+ *
+ * `time_grid` is an upper bound on the number of DISTINCT times among the rows of X (0 = unknown: every entry is
+ * evaluated directly; lfm_count_distinct_times gives it from a host copy).  The reference's layout observes every gene
+ * on the same few time points (src/dataset.py:380-391), and the exp/erf factors of h (src/model.py:315-365) depend on
+ * (gene, t, t') only: when the bound is small the library finds the distinct times on the device, tabulates those
+ * factors once per evaluation (G T^2 entries instead of N^2) and builds Sigma and the dK/dtheta contraction from the
+ * tables.  The tables hold the very values the direct path computes; results agree to rounding.  If X has more
+ * distinct times than the bound, the kernels detect it on the device and evaluate directly.  The workspace
+ * (lfm_nlml_workspace_bytes_tg with the same time_grid) holds the tables when they are worthwhile. */
 int64_t lfm_count_distinct_times(int64_t N, const double* X_host);
 size_t lfm_nlml_workspace_bytes_tg(int64_t N, int G, int64_t time_grid);
-int lfm_nlml_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y, const double* theta,
-                double jitter, int64_t time_grid, void* ws, size_t ws_bytes, double* out, int* info);
-int lfm_nlml_grad_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                     const double* theta, double jitter, int64_t time_grid, void* ws, size_t ws_bytes,
-                     double* out, int* info);
-int lfm_nlml_grad_unc_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
-                         const double* theta_unc, double jitter, int64_t time_grid, void* ws, size_t ws_bytes,
-                         double* out, int* info);
 
-/* ---- heteroscedastic objective ----------------------------------------------------------------
- * Sigma = K + diag(variances) + jitter I + sigma^2 I: the measurement variances of dataset_3d
- * (src/dataset.py:396-397) inside the training covariance, the convention of the reference's GPyTorch twin when it
- * trains (src/gpytorch_alfi/model_alfi.py:294-299: K_xx += 1e-4 I; K_xx += self.variance).  `variances` is N doubles
- * (device) or NULL, in which case these ARE the entry points above.  The gradient formulas do not change
- * (d Sigma / d theta has no variance term); only the diagonal tiles of the Sigma build read `variances`. */
+/* out[0] = NLML = 1/2 [N log 2pi + log det Sigma + z^T Sigma^-1 z]. */
 int lfm_nlml_het_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y, const double* variances,
                     const double* theta, double jitter, int64_t time_grid, void* ws, size_t ws_bytes, double* out,
                     int* info);
+/* jax.value_and_grad(JaxTrainer.loss) (src/trainer.py:86-103,126) in CONSTRAINED coordinates: out[0] = NLML,
+ * out[1..P] = dNLML/dtheta.  dK/dtheta blocks are contracted with K_bar = 1/2 (Sigma^-1 - alpha alpha^T) on the fly
+ * and never materialised. */
 int lfm_nlml_grad_het_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
                          const double* variances, const double* theta, double jitter, int64_t time_grid, void* ws,
                          size_t ws_bytes, double* out, int* info);
+/* The same, differentiated w.r.t. the UNCONSTRAINED leaves theta_unc -- the exact quantity the optimiser in
+ * src/trainer.py:126-128 consumes.  out[0] = NLML, out[1..P] = gradient. */
 int lfm_nlml_grad_unc_het_tg(lfm_stream_t stream, int64_t N, int G, const double* X, const double* y,
                              const double* variances, const double* theta_unc, double jitter, int64_t time_grid,
                              void* ws, size_t ws_bytes, double* out, int* info);
@@ -180,95 +159,20 @@ int lfm_gene_posterior(lfm_stream_t stream, int64_t N, int G, const double* X, c
  * A hint smaller than what the kernel finds makes it refuse with info = -1. */
 int lfm_count_unique_rows(int64_t N, const double* X_host);
 
-/* B independent value_and_grad evaluations sharing (X, y): theta_unc is B x P, out_val B,
- * out_grad B x P, info B ints.  N <= 128. */
-int lfm_batched_nlml_grad_unc(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
-                              const double* y, const double* theta_unc, double jitter,
-                              int unique_rows_hint, double* out_val, double* out_grad, int* info);
-
-/* B independent JaxTrainer.fit loops (src/trainer.py:162-228) with optax.adam(lr) restated
- * (b1,b2,eps as given; src/main.py:45) and the "fix p21" hook of trainer.py:133-160,205-210,218-220.
- * theta_unc_io is B x P UNCONSTRAINED (in: start / current iterate, out: iterate after the last step
- * of this call).  The fit may be split into chunks of steps [first_step, first_step + steps) of a
- * total_steps-long fit (with a collective in between); adam_state (B x 2P doubles: m then v) carries
- * the moments between calls and may be NULL only when the whole fit is one call.  out_hist
- * (B x ld_hist) receives the loss at every step at column first_step + s.  When the call reaches
- * total_steps, out_theta (B x P, may be NULL) receives constrain(theta_unc) with the constrained-space
- * hook of trainer.py:218-220 applied. */
-int lfm_batched_fit(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                    double* theta_unc_io, double* adam_state, double jitter, double lr, double b1,
-                    double b2, double eps, int first_step, int steps, int total_steps, int fix_params,
-                    int steps_per_epoch, int unique_rows_hint, double* out_hist, int64_t ld_hist,
-                    double* out_theta, int* info);
-
-/* Device state of B fits in ONE launch: theta_unc = unconstrain(theta0) (src/trainer.py:75), adam_state (B x 2P, may be
- * NULL) = 0, hist (n_hist doubles, may be NULL) = NaN, info (B ints, may be NULL) = 0, keys (n_keys int64 words for
- * best_key / step_keys, may be NULL) = INT64_MAX. */
-int lfm_batched_fit_init(lfm_stream_t stream, int64_t B, int G, const double* theta0, double* theta_unc,
-                         double* adam_state, double* hist, int64_t n_hist, int* info, long long* keys, int64_t n_keys);
-
-/* Time-grid variants of the two batched entry points: `time_grid_hint` is an upper bound on the number of
- * DISTINCT times among the rows of X (lfm_count_distinct_times; 0 = unknown).  With both hints set and
- * the problem inside the limits of the one-warp-per-LFM kernel (unique rows <= 36, G T^2 <= 2048), every
- * LFM is fitted by a single warp with the exp/erf pair terms tabulated once per step in shared memory;
- * otherwise the one-CTA-per-LFM kernel runs.  A hint smaller than the true count gives info = -2. */
-int lfm_batched_nlml_grad_unc_tg(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
-                                 const double* y, const double* theta_unc, double jitter, int unique_rows_hint,
-                                 int time_grid_hint, double* out_val, double* out_grad, int* info);
-int lfm_batched_fit_tg(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                       double* theta_unc_io, double* adam_state, double jitter, double lr, double b1, double b2,
-                       double eps, int first_step, int steps, int total_steps, int fix_params,
-                       int steps_per_epoch, int unique_rows_hint, int time_grid_hint, double* out_hist,
-                       int64_t ld_hist, double* out_theta, int* info, long long* best_key, void* structure_cache);
-/* Per-LFM observations: LFM b fits y + b * y_stride (y_stride >= N; 0 = every LFM fits the same y, which is what the
- * entry points above do).  X -- and with it the duplicate-row / time-grid structure -- stays shared, so this is the
- * batch over replicas, gene subsets of equal size and candidate transcription factors of north_star: same design
- * points, different expression data, independent hyper-parameters.  Everything else as lfm_batched_fit_tg /
- * lfm_batched_nlml_grad_unc_tg. */
-int lfm_batched_fit_multi(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                          int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter, double lr,
-                          double b1, double b2, double eps, int first_step, int steps, int total_steps,
-                          int fix_params, int steps_per_epoch, int unique_rows_hint, int time_grid_hint,
-                          double* out_hist, int64_t ld_hist, double* out_theta, int* info, long long* best_key,
-                          void* structure_cache);
-int lfm_batched_nlml_grad_unc_multi(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X,
-                                    const double* y, int64_t y_stride, const double* theta_unc, double jitter,
-                                    int unique_rows_hint, int time_grid_hint, double* out_val, double* out_grad,
-                                    int* info);
-/* lfm_batched_fit_multi plus `step_keys` (may be NULL): total_steps device words, initialised to INT64_MAX by the caller;
- * word s receives atomicMin over the batch of the order-preserving image of every LFM's loss at optimiser step s (see
- * best_key below).  The best objective of EVERY step of a sharded fit is then ONE integer MIN all-reduce of that vector
- * after the launch, however many steps the launch ran -- the per-step reduction of north_star without a launch boundary
- * per step. */
-int lfm_batched_fit_trace(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                          int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter, double lr,
-                          double b1, double b2, double eps, int first_step, int steps, int total_steps,
-                          int fix_params, int steps_per_epoch, int unique_rows_hint, int time_grid_hint,
-                          double* out_hist, int64_t ld_hist, double* out_theta, int* info, long long* best_key,
-                          long long* step_keys, void* structure_cache);
-/* The WHOLE fit (steps 0 .. total_steps) in one launch, with `queue_ws` (lfm_batched_queue_bytes() device bytes, may be
- * NULL = plain launch): the CTAs become persistent workers that take "the next chunk_steps steps of LFM b" tasks from a
- * device-side queue, so an LFM moves to whichever resident slot is free after every chunk.  The library uses the queue
- * when a static one-CTA-per-LFM assignment would be unbalanced (more LFMs than SMs, fewer than resident team slots, not
- * a whole number per SM -- e.g. the 512-LFM shard of 4096 restarts over 8 GPUs: 4 teams on 68 SMs and 3 on 80 for the
- * whole fit otherwise) and ignores it elsewhere; results do not depend on it beyond the rounding of Adam's running bias
- * products at chunk boundaries.  adam_state is required with a queue (the moments travel between workers through it);
- * the CTA-per-LFM fallback kernel ignores the queue.  LFM_BATCHED_QUEUE = 0 | 1 in the environment forces it off / on. */
-size_t lfm_batched_queue_bytes(int64_t B, int total_steps, int chunk_steps);
-int lfm_batched_fit_queue(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
-                          int64_t y_stride, double* theta_unc_io, double* adam_state, double jitter, double lr,
-                          double b1, double b2, double eps, int total_steps, int fix_params, int steps_per_epoch,
-                          int unique_rows_hint, int time_grid_hint, double* out_hist, int64_t ld_hist,
-                          double* out_theta, int* info, long long* best_key, long long* step_keys,
-                          void* structure_cache, int chunk_steps, void* queue_ws, size_t queue_bytes);
-/* structure_cache (may be NULL): lfm_batched_structure_bytes() device bytes the caller keeps between the calls of ONE
- * chunked fit.  The call with first_step == 0 stores the structure of X (duplicate rows, distinct times and time
- * differences, pair table) there; calls with first_step > 0 load it instead of repeating the O(N^2) scans. */
-size_t lfm_batched_structure_bytes(int64_t N, int G, int unique_rows_hint, int time_grid_hint);
-/* ---- batched fits with measurement variances: the heteroscedastic objective of lfm_nlml_grad_unc_het_tg ------------
- * Sigma = K + diag(v) + (jitter + sigma^2) I, i.e. noise c_i = v_i + jitter + sigma^2 per point.  `variances` is N
+/* Arguments of the batched evaluations and fits.  The B LFMs share X (N <= 128 rows), and with it the duplicate-row /
+ * time-grid structure.  LFM b fits y + b * y_stride (y_stride >= N), or with y_stride = 0 every LFM fits the same y.
+ * A stride makes the batch one over replicas, gene subsets of equal size and candidate transcription factors of
+ * north_star: same design points, different expression data, independent hyper-parameters.
+ *
+ * `time_grid_hint` is an upper bound on the number of DISTINCT times among the rows of X (lfm_count_distinct_times;
+ * 0 = unknown).  With both hints set and the problem inside the limits of the one-warp-per-LFM kernel (unique rows
+ * <= 36, G T^2 <= 2048), every LFM is fitted by a single warp with the exp/erf pair terms tabulated once per step in
+ * shared memory; otherwise the one-CTA-per-LFM kernel runs.  A hint smaller than the true count gives info = -2.
+ *
+ * `variances` is NULL (the reference's objective) or selects the heteroscedastic objective of lfm_nlml_grad_unc_het_tg:
+ * Sigma = K + diag(v) + (jitter + sigma^2) I, i.e. noise c_i = v_i + jitter + sigma^2 per point.  `variances` is then N
  * device doubles shared by every LFM (var_stride 0) or one row per LFM at variances + b * var_stride (var_stride >= N),
- * as y / y_stride; NULL means exactly lfm_batched_nlml_grad_unc_multi / lfm_batched_fit_trace / _fit_queue.
+ * as y / y_stride.
  * The duplicate-row compression stays exact with a noise per point (same rule for U and R as above): per unique row u
  *   omega_u = sum_{i in u} 1/c_i, omega2_u = sum_{i in u} 1/c_i^2, cbar_u = R / omega_u, q_u = cbar_u sum_{i in u} z_i/c_i,
  *   M = diag(cbar) + R K_u,  beta = M^-1 q = P^T alpha,  K_u beta = (q - cbar o beta) / R,
@@ -280,12 +184,54 @@ size_t lfm_batched_structure_bytes(int64_t N, int G, int unique_rows_hint, int t
  *   dNLML/dsigma = sigma (tr Sigma^-1 - alpha^T alpha);
  * with v = 0 every line is the homoscedastic one.  Every c_i must be > 0: otherwise (or with NaN variances) info = 1 and
  * the loss / gradient are NaN, as for a failed factorisation. */
+
+/* B independent value_and_grad evaluations w.r.t. the UNCONSTRAINED leaves (src/trainer.py:126): theta_unc is B x P,
+ * out_val B, out_grad B x P, info B ints. */
 int lfm_batched_nlml_grad_unc_het(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
                                   int64_t y_stride, const double* variances, int64_t var_stride,
                                   const double* theta_unc, double jitter, int unique_rows_hint, int time_grid_hint,
                                   double* out_val, double* out_grad, int* info);
-/* lfm_batched_fit_trace with variances; with `queue_ws` non-NULL it is lfm_batched_fit_queue instead (then first_step must
- * be 0 and steps == total_steps: the queue runs the whole fit). */
+
+/* Device state of B fits in ONE launch: theta_unc = unconstrain(theta0) (src/trainer.py:75), adam_state (B x 2P, may be
+ * NULL) = 0, hist (n_hist doubles, may be NULL) = NaN, info (B ints, may be NULL) = 0, keys (n_keys int64 words for
+ * best_key / step_keys, may be NULL) = INT64_MAX. */
+int lfm_batched_fit_init(lfm_stream_t stream, int64_t B, int G, const double* theta0, double* theta_unc,
+                         double* adam_state, double* hist, int64_t n_hist, int* info, long long* keys, int64_t n_keys);
+
+/* B independent JaxTrainer.fit loops (src/trainer.py:162-228) with optax.adam(lr) restated (b1,b2,eps as given;
+ * src/main.py:45) and the "fix p21" hook of trainer.py:133-160,205-210,218-220.  theta_unc_io is B x P UNCONSTRAINED
+ * (in: start / current iterate, out: iterate after the last step of this call).  The fit may be split into chunks of
+ * steps [first_step, first_step + steps) of a total_steps-long fit (with a collective in between); adam_state (B x 2P
+ * doubles: m then v) carries the moments between calls and may be NULL only when the whole fit is one call.  out_hist
+ * (B x ld_hist) receives the loss at every step at column first_step + s.  When the call reaches total_steps, out_theta
+ * (B x P, may be NULL) receives constrain(theta_unc) with the constrained-space hook of trainer.py:218-220 applied.
+ *
+ * best_key (may be NULL): one device word that receives atomicMin over the batch of the order-preserving integer
+ * image of each LFM's loss after the last step of this call (finite losses only; initialise it to INT64_MAX).
+ * key(v) = bits(v) for v >= 0, bits(v) ^ 0x7fff...f otherwise -- monotone in v, so the global best objective of a
+ * chunk of steps is ONE integer MIN all-reduce of that word across ranks (north_star: "one NCCL allreduce of
+ * best-objective ... state per step").
+ *
+ * step_keys (may be NULL): total_steps device words, initialised to INT64_MAX by the caller; word s receives atomicMin
+ * over the batch of the key of every LFM's loss at optimiser step s.  The best objective of EVERY step of a sharded fit
+ * is then ONE integer MIN all-reduce of that vector after the launch, however many steps the launch ran -- the per-step
+ * reduction of north_star without a launch boundary per step.
+ *
+ * structure_cache (may be NULL): lfm_batched_structure_bytes() device bytes the caller keeps between the calls of ONE
+ * chunked fit.  The call with first_step == 0 stores the structure of X (duplicate rows, distinct times and time
+ * differences, pair table) there; calls with first_step > 0 load it instead of repeating the O(N^2) scans.
+ *
+ * queue_ws (may be NULL = plain launch, chunk_steps and queue_bytes unused): lfm_batched_queue_bytes() device bytes.  The
+ * call then runs the WHOLE fit in one launch (first_step must be 0 and steps == total_steps): the CTAs become persistent
+ * workers that take "the next chunk_steps steps of LFM b" tasks from a device-side queue, so an LFM moves to whichever
+ * resident slot is free after every chunk.  The library uses the queue when a static one-CTA-per-LFM assignment would be
+ * unbalanced (more LFMs than SMs, fewer than resident team slots, not a whole number per SM -- e.g. the 512-LFM shard of
+ * 4096 restarts over 8 GPUs: 4 teams on 68 SMs and 3 on 80 for the whole fit otherwise) and ignores it elsewhere;
+ * results do not depend on it beyond the rounding of Adam's running bias products at chunk boundaries.  adam_state is
+ * required with a queue (the moments travel between workers through it); the CTA-per-LFM fallback kernel ignores the
+ * queue.  LFM_BATCHED_QUEUE = 0 | 1 in the environment forces it off / on. */
+size_t lfm_batched_structure_bytes(int64_t N, int G, int unique_rows_hint, int time_grid_hint);
+size_t lfm_batched_queue_bytes(int64_t B, int total_steps, int chunk_steps);
 int lfm_batched_fit_het(lfm_stream_t stream, int64_t B, int64_t N, int G, const double* X, const double* y,
                         int64_t y_stride, const double* variances, int64_t var_stride, double* theta_unc_io,
                         double* adam_state, double jitter, double lr, double b1, double b2, double eps, int first_step,
@@ -322,18 +268,12 @@ int lfm_batched_gene_posterior(lfm_stream_t stream, int64_t B, int64_t N, int G,
                                double jitter, int64_t Tstar, const double* Xstar, int unique_rows_hint, void* ws,
                                size_t ws_bytes, double* out_mean, double* out_cov, double* out_var, int* info);
 
-/* best_key (may be NULL): one device word that receives atomicMin over the batch of the order-preserving integer
- * image of each LFM's loss after the last step of this call (finite losses only; initialise it to INT64_MAX).
- * key(v) = bits(v) for v >= 0, bits(v) ^ 0x7fff...f otherwise -- monotone in v, so the global best objective of a
- * chunk of steps is ONE integer MIN all-reduce of that word across ranks (north_star: "one NCCL allreduce of
- * best-objective ... state per step"). */
-
 /* Warps per LFM the batched entry points use for a batch of B LFMs of this shape on the current device: 1 (one warp per
  * LFM, register-resident Cholesky; a full GPU), 4 (a team of four warps per LFM, symmetric sweep in register tiles;
  * shards that leave SMs idle, e.g. 4096 restarts over 8 GPUs), or 0 when the shape runs the CTA-per-LFM kernel.
- * LFM_BATCHED_TEAM = 1 | 4 | 8 in the environment overrides the choice (measurements).  The answer is for the entry
- * points without variances: the _het ones keep N + 2U more doubles per LFM in shared memory and choose from their own
- * occupancy. */
+ * LFM_BATCHED_TEAM = 1 | 4 | 8 in the environment overrides the choice (measurements).  The answer is for calls with
+ * variances = NULL: with variances the kernels keep N + 2U more doubles per LFM in shared memory and choose from their
+ * own occupancy. */
 int lfm_batched_team_size(int64_t B, int64_t N, int G, int unique_rows_hint, int time_grid_hint);
 
 /* Winner of a shard after a fit: out_packed (P + 2 doubles) = [loss, id, theta(P)] of the LFM with the smallest FINITE
@@ -364,16 +304,13 @@ int lfm_comm_destroy(lfm_comm* c);
  * binds).  They allocate device scratch on first use per (N,G) and cache it in a handle. -------- */
 
 /* ---- evaluation plans -------------------------------------------------------------------------
- * One lfm_nlml_grad[_unc]_tg evaluation over FIXED device buffers, captured once as a CUDA graph (the ~140
- * launches and ~70 cross-stream event edges of an N = 4000 evaluation replay with ~1 us between dependent
- * kernels).  A fit loop writes the next theta into the bound `theta` buffer and launches the plan again
- * (src/trainer.py:201-216 evaluates the same (X, y) at every step).  create runs the evaluation once eagerly
- * (validation, lazy initialisation) and synchronises; launch is stream-ordered and never synchronises. */
+ * One lfm_nlml_grad_het_tg evaluation (lfm_nlml_grad_unc_het_tg when `unconstrained` != 0) over FIXED device buffers
+ * (`variances`, or NULL, bound like X and y), captured once as a CUDA graph (the ~140 launches and ~70 cross-stream
+ * event edges of an N = 4000 evaluation replay with ~1 us between dependent kernels).  A fit loop writes the next theta
+ * into the bound `theta` buffer and launches the plan again (src/trainer.py:201-216 evaluates the same (X, y) at every
+ * step).  create runs the evaluation once eagerly (validation, lazy initialisation) and synchronises; launch is
+ * stream-ordered and never synchronises. */
 typedef struct lfm_plan lfm_plan;
-int lfm_nlml_grad_plan_create(lfm_plan** out_plan, int64_t N, int G, const double* X, const double* y,
-                              const double* theta, double jitter, int64_t time_grid, int unconstrained, void* ws,
-                              size_t ws_bytes, double* out, int* info);
-/* same with the heteroscedastic objective: `variances` (N device doubles, bound like X and y) or NULL */
 int lfm_nlml_grad_plan_create_het(lfm_plan** out_plan, int64_t N, int G, const double* X, const double* y,
                                   const double* variances, const double* theta, double jitter, int64_t time_grid,
                                   int unconstrained, void* ws, size_t ws_bytes, double* out, int* info);
@@ -393,12 +330,9 @@ int lfm_latent_posterior_host(lfm_handle* h, int64_t N, int G, const double* X, 
                               const double* variances, const double* theta, double jitter,
                               int64_t Tstar, const double* Xstar, double* out_mean, double* out_var,
                               int* info);
-int lfm_batched_fit_host(lfm_handle* h, int64_t B, int64_t N, int G, const double* X, const double* y,
-                         const double* theta0, double jitter, double lr, double b1, double b2,
-                         double eps, int steps, int fix_params, int steps_per_epoch, double* out_theta,
-                         double* out_hist, int* info);
-/* lfm_batched_fit_host with measurement variances (N host doubles, staged in the same single host->device copy as X, y
- * and theta0; the objective of lfm_batched_fit_het) or NULL (= lfm_batched_fit_host). */
+/* B whole fits of lfm_batched_fit_het from host buffers: theta0 (B x P CONSTRAINED start points), out_theta (B x P
+ * constrained result), out_hist (B x steps, may be NULL), info (B ints, may be NULL).  `variances` is N host doubles,
+ * staged in the same single host->device copy as X, y and theta0, or NULL. */
 int lfm_batched_fit_het_host(lfm_handle* h, int64_t B, int64_t N, int G, const double* X, const double* y,
                              const double* variances, const double* theta0, double jitter, double lr, double b1,
                              double b2, double eps, int steps, int fix_params, int steps_per_epoch, double* out_theta,

@@ -377,14 +377,16 @@ def test_batched_het_matches_the_gpytorch_twin(cuda, name):
 
 @pytest.mark.gpu
 def test_batched_fit_het_host_equals_device_path(cuda):
-    """lfm_batched_fit_het_host (host buffers, one H2D copy) equals the device entry point; NULL variances equals
-    lfm_batched_fit_host."""
+    """lfm_batched_fit_het_host (host buffers, one H2D copy) equals the device entry point, with variances and with NULL
+    variances (the homoscedastic fit); a second NULL-variance call on the same handle repeats the fit bit for bit."""
     from dis_project_b200 import _lib, ops
     G, T, R, B, steps = 5, 7, 3, 4, 25
     x, y, var = het_problem(G, T, R, 171)
     TH = start_points(G, B, 172)
     st = ops.BatchedFitState(TH, G, steps)
     ops.batched_fit_steps(st, x, y, 1e-4, steps, variances=var)
+    st0 = ops.BatchedFitState(TH, G, steps)
+    ops.batched_fit_steps(st0, x, y, 1e-4, steps)
     lib = _lib.lib()
     h = C.c_void_p()
     assert lib.lfm_handle_create(C.byref(h)) == 0
@@ -400,9 +402,10 @@ def test_batched_fit_het_host_equals_device_path(cuda):
         if v is not None:
             assert relerr(hist, st.hist.cpu().numpy()) < 1e-12 and relerr(th, st.theta.cpu().numpy()) < 1e-12
         else:
+            assert relerr(hist, st0.hist.cpu().numpy()) < 1e-12 and relerr(th, st0.theta.cpu().numpy()) < 1e-12
             th2, hist2 = np.empty((B, P)), np.empty((B, steps))
-            assert lib.lfm_batched_fit_host(h, B, x.shape[0], G, x.ctypes.data, y.ctypes.data, TH_c.ctypes.data, 1e-4,
-                                            0.01, 0.9, 0.999, 1e-8, steps, 1, 1000, th2.ctypes.data, hist2.ctypes.data,
-                                            info.ctypes.data) == 0
+            assert lib.lfm_batched_fit_het_host(h, B, x.shape[0], G, x.ctypes.data, y.ctypes.data, None,
+                                                TH_c.ctypes.data, 1e-4, 0.01, 0.9, 0.999, 1e-8, steps, 1, 1000,
+                                                th2.ctypes.data, hist2.ctypes.data, info.ctypes.data) == 0
             assert np.array_equal(hist, hist2) and np.array_equal(th, th2)
     assert lib.lfm_handle_destroy(h) == 0

@@ -130,16 +130,16 @@ def test_host_buffer_capi(cuda):
     B = 4
     TH = np.ascontiguousarray(np.tile(th, (B, 1))); TH[1:, :5] *= np.array([[1.1], [0.9], [1.3]])
     oth = np.empty((B, 17)); hist = np.empty((B, 30)); infos = (C.c_int * B)()
-    assert lib.lfm_batched_fit_host(h, B, 105, 5, x.ctypes.data, y.ctypes.data, TH.ctypes.data, 1e-4, 0.01, 0.9, 0.999,
-                                    1e-8, 30, 1, 1000, oth.ctypes.data, hist.ctypes.data, infos) == 0
+    assert lib.lfm_batched_fit_het_host(h, B, 105, 5, x.ctypes.data, y.ctypes.data, None, TH.ctypes.data, 1e-4, 0.01,
+                                        0.9, 0.999, 1e-8, 30, 1, 1000, oth.ctypes.data, hist.ctypes.data, infos) == 0
     for b in range(B):
         t_ref, h_ref = o.fit(TH[b], x, y, 1e-4, num_iters=30)
         assert relerr(hist[b], h_ref) < 1e-9 and relerr(oth[b], t_ref) < 1e-8
     # error behaviour: invalid arguments are rejected with a status, not a crash
     assert lib.lfm_nlml_grad_host(h, 104, 5, x.ctypes.data, y.ctypes.data, th.ctypes.data, 1e-4, 0, out.ctypes.data,
                                   C.byref(info)) == -1
-    assert lib.lfm_batched_fit_host(h, 1, 640, 5, x.ctypes.data, y.ctypes.data, TH.ctypes.data, 1e-4, 0.01, 0.9, 0.999,
-                                    1e-8, 1, 1, 1000, oth.ctypes.data, hist.ctypes.data, infos) == -3
+    assert lib.lfm_batched_fit_het_host(h, 1, 640, 5, x.ctypes.data, y.ctypes.data, None, TH.ctypes.data, 1e-4, 0.01,
+                                        0.9, 0.999, 1e-8, 1, 1, 1000, oth.ctypes.data, hist.ctypes.data, infos) == -3
     assert lib.lfm_handle_destroy(h) == 0
 
 

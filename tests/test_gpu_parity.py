@@ -448,7 +448,7 @@ def test_bijector_kernels(cuda):
 
 @pytest.mark.parametrize("team,B", [(4, 20), (1, 9), (4, 333)])
 def test_batched_queue_mode_matches_chunked_launches(cuda, team, B, monkeypatch):
-    """lfm_batched_fit_queue: persistent workers + device-side task queue (an LFM changes SM after every chunk).  Forced
+    """lfm_batched_fit_het with a queue workspace: persistent workers + device-side task queue (an LFM changes SM after every chunk).  Forced
     on here (LFM_BATCHED_QUEUE=1; the library otherwise only uses it where the static assignment is unbalanced): the fit
     must equal the same fit run as separate launches of the same chunk length, bit for bit -- same arithmetic, only the
     placement differs -- including per-LFM observations and the per-step best-objective keys."""

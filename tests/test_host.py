@@ -26,10 +26,10 @@ def test_capi_library_exports_every_declared_symbol():
         assert hasattr(lib, name), f"{name} declared in include/lfm_b200.h but not exported"
         assert name in _lib.SIGNATURES, f"{name} has no ctypes signature in dis_project_b200/_lib.py"
     l = _lib.lib()
-    assert l.lfm_abi_version() == 2
+    assert l.lfm_abi_version() == 3
     assert l.lfm_status_string(-5).decode().startswith("no sm_100")
-    assert l.lfm_nlml_workspace_bytes(4000, 50) >= 2 * 4096 * 4096 * 8
-    assert l.lfm_nlml_workspace_bytes(0, 5) == 0
+    assert l.lfm_nlml_workspace_bytes_tg(4000, 50, 0) >= 2 * 4096 * 4096 * 8
+    assert l.lfm_nlml_workspace_bytes_tg(0, 5, 0) == 0
 
 
 def test_product_path_has_no_cpu_fallback_and_never_imports_the_oracle():
@@ -248,8 +248,8 @@ def test_count_distinct_times():
     x2 = np.ascontiguousarray(np.concatenate([x, x + [[0.5, 0, 0]]]))
     assert lib.lfm_count_distinct_times(70, x2.ctypes.data) == 14
     assert lib.lfm_count_distinct_times(0, None) == 0
-    assert lib.lfm_nlml_workspace_bytes_tg(4000, 50, 80) > lib.lfm_nlml_workspace_bytes(4000, 50)
-    assert lib.lfm_nlml_workspace_bytes_tg(120, 4, 120) == lib.lfm_nlml_workspace_bytes(120, 4)  # tables not worthwhile
+    assert lib.lfm_nlml_workspace_bytes_tg(4000, 50, 80) > lib.lfm_nlml_workspace_bytes_tg(4000, 50, 0)
+    assert lib.lfm_nlml_workspace_bytes_tg(120, 4, 120) == lib.lfm_nlml_workspace_bytes_tg(120, 4, 0)  # tables not worthwhile
 
 
 def test_count_distinct_times_many_values_and_unique_rows_rule():

@@ -1,5 +1,5 @@
 """Kernel time of a 150-step p53 fit of B LFMs on one GPU: separate launches of 10 steps (static one-CTA-per-LFM
-assignment) against ONE launch with persistent workers + task queue (lfm_batched_fit_queue), team of four warps per LFM."""
+assignment) against ONE launch with persistent workers + task queue (lfm_batched_fit_het with queue_ws), team of four warps per LFM."""
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
